@@ -2,6 +2,7 @@
 """bench.py -- 31-mer count_kmer throughput (queries/s) on B200, per the driver contract.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload default|cfg2|cfg3|cfg5|tiny]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (pack/seed + backward-search kernels) over one batch of synthetic k-mer
 queries.  Headline workload = BASELINE.json configs[2]: 10 M synthetic 150-bp reads with 1 % errors (1.51 Gsymbol
@@ -19,6 +20,11 @@ Nested `other_workloads`: configs[1] (151 Msymbol BWT, N = 1 only) and configs[4
 125 M-query share at N = 1, the full 10^9 queries over 8 replicas at N = 8).
 
 One JSON line on stdout (rank 0).  Everything else goes to stderr.
+
+--dump-outputs DIR: rank 0 writes, per workload, the counts the last timed step returned for its queries
+(DIR/<workload>_counts.npy, float64) and their positions in the batch (DIR/<workload>_query_index.npy); a batch larger
+than DUMP_SAMPLE queries is sampled at fixed, seeded positions.  The inputs are seeded too, so two builds run with the
+same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -63,6 +69,8 @@ PAIR_SYMS = 96
 QUAD_SECTOR_BYTES = 32  # layout.h: one 32-byte sector per 224 positions and 4-symbol code, four steps per sector (quad path)
 QUAD_SYMS = 224
 LINE_BYTES = 128      # what one L2 miss costs HBM whatever the request size (profiles/r1_gather_dram_bytes.csv)
+DUMP_SAMPLE = 1 << 20  # --dump-outputs: queries kept per workload, 16 B each (count + index): 48 MB for the default run
+DUMP_SEED = 0x5EED00D0
 
 
 def log(*a):
@@ -227,6 +235,17 @@ def encode_u64(q, k: int):
     return out
 
 
+def dump_outputs(out_dir: str, key: str, counts, offset: int) -> None:
+    """--dump-outputs: `counts` (u64, one per query of the batch slice starting at query `offset`) as float64, exact
+    below 2^53, with the batch position of every entry kept; at most DUMP_SAMPLE entries, at seeded positions"""
+    import numpy as np
+    n = counts.shape[0]
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_SAMPLE, replace=False)) if n > DUMP_SAMPLE else np.arange(n)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{key}_counts.npy"), counts[idx].astype(np.float64))
+    np.save(os.path.join(out_dir, f"{key}_query_index.npy"), (idx + offset).astype(np.float64))
+
+
 def cpu_reference_leg(orc, q_host, k, threads, target_s, label):
     """Times the oracle's count_kmer loop on a bounded prefix of the batch."""
     n = q_host.shape[0]
@@ -320,7 +339,7 @@ def e2e_legs(args, cfg, handle, lib, M, q_dev_list, k, reads_sample, n_devices, 
     import torch
 
     n = sum(int(q.shape[0]) for q in q_dev_list)
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     legs = {}
     vp = ctypes.c_void_p
 
@@ -479,6 +498,8 @@ def measure_ours(args, cfg, ctx, primary: bool):
     value = n_job * args.steps / (total_ms / 1e3)
     checksum = int(d_out.sum().item())
     got = d_out.cpu().numpy().view(np.uint64)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, cfg["key"], got, lo)
 
     # ---- the same step with the k-mers resident as 2-bit-per-symbol integers (8 B per query instead of k): what a
     #      k-mer counter that keeps packed k-mers on the device would call (msbwt_seed_kmers_u64_device + search) ----
@@ -891,7 +912,13 @@ def main():
     ap.add_argument("--workload", choices=sorted(WORKLOADS) + ["default"],
                     default=os.environ.get("MSBWT_BENCH_WORKLOAD", "default"),
                     help="default = configs[2] as the bench line; configs[1] (N = 1) and configs[4] (N = 1 and 8) nested beside it")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the counts of the last timed step of every workload to DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "ours":
         args.warmup = max(args.warmup, 3)
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,12 +1,11 @@
-"""Regenerates the committed golden fixtures.  Run from the repo root in the BUILD
-container (it may read /root/reference; nothing at test time does):
+"""Regenerates the committed golden fixtures.  Run from the repo root:
 
     python tests/golden/make_golden.py
 
 two_string.npy    -- byte-identical to the reference fixture test_data/two_string.npy
                      (strings ACGT, TGCA; payload [13,9,10,8,11,9,13,10,11,8]); produced
-                     with the oracle's own naive_bwt -> convert_to_vec -> save_bwt_numpy
-                     and compared with the reference file when it is mounted.
+                     with the oracle's own naive_bwt -> convert_to_vec -> save_bwt_numpy.
+                     tests/test_oracle_kat.py pins its SHA-256.
 reads30x_k31.npz  -- 3000 synthetic 100-bp reads (30x, 1% substitutions, one read with N),
                      their msbwt RLE stream, 3000 31-mers + 3000 12-mers (half read-sampled,
                      half random) and the counts the pinned CPU oracle gives for them.
@@ -31,10 +30,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 def main():
     p = os.path.join(HERE, "two_string.npy")
     O.save_bwt_numpy(O.convert_to_vec(naive.naive_bwt(["ACGT", "TGCA"])), p)
-    ref = "/root/reference/test_data/two_string.npy"
-    if os.path.exists(ref):
-        assert open(ref, "rb").read() == open(p, "rb").read(), "fixture differs from the reference's"
-        print("two_string.npy == reference fixture")
 
     reads = synth.np_make_reads(3000, 100, 30.0, 0.01, seed=20261018)
     reads[11, 50:52] = 4

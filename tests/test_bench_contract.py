@@ -76,6 +76,36 @@ def test_bench_helpers_on_cpu():
     assert bench.HEADLINE == "cfg3" and bench.WORKLOADS["cfg3"]["scaling"] == "strong"
 
 
+def test_steps_below_one_are_refused():
+    res = run_bench("--impl", "reference", "--workload", "tiny", "--steps", "0")
+    assert res.returncode != 0 and "--steps must be at least 1" in res.stderr
+
+
+def test_dump_outputs_writes_a_fixed_sample_of_the_counts(tmp_path):
+    """--dump-outputs: float64 counts with their batch positions; a large batch is sampled at the same positions every
+    run, and the default run's three workloads stay within 64 MB"""
+    import numpy as np
+
+    import bench
+    small = np.arange(1000, dtype=np.uint64) * np.uint64(3)
+    bench.dump_outputs(str(tmp_path / "a"), "tiny", small, 0)
+    c, i = np.load(tmp_path / "a" / "tiny_counts.npy"), np.load(tmp_path / "a" / "tiny_query_index.npy")
+    assert c.dtype == np.float64 and i.dtype == np.float64
+    assert (i == np.arange(1000)).all() and (c == 3 * np.arange(1000)).all()
+
+    n = 3 * bench.DUMP_SAMPLE + 5
+    big = np.arange(n, dtype=np.uint64) + np.uint64(2**40)
+    for run in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / run), "cfg3", big, 7)
+    c, i = np.load(tmp_path / "b" / "cfg3_counts.npy"), np.load(tmp_path / "b" / "cfg3_query_index.npy")
+    assert c.shape == i.shape == (bench.DUMP_SAMPLE,)
+    assert (np.diff(i) > 0).all() and i[0] >= 7 and i[-1] < n + 7
+    assert (c == i - 7 + 2**40).all()
+    assert (np.load(tmp_path / "c" / "cfg3_query_index.npy") == i).all()
+    per_workload = sum(os.path.getsize(tmp_path / "b" / f) for f in os.listdir(tmp_path / "b"))
+    assert 3 * per_workload <= 64 << 20
+
+
 def test_clock_sampler_keeps_the_samples_inside_the_timed_region(tmp_path):
     """bench.py's `clocks` object: nvidia-smi lines carry their own time stamps; only those inside the timed region count
     (the region is ~40 ms on the headline workload), with explicit fallbacks when none falls inside"""

@@ -1,6 +1,6 @@
 """Parity tests proper: the CUDA path, called through the C ABI (include/msbwt_gpu.h via
 the RleBWT mirror), against the CPU oracle on the same inputs -- bit-exact (u64 counts /
-positions).  The cases follow the reference's own tests (file:line under /root/reference)."""
+positions).  The cases follow the reference's own tests (file:line in the reference, rust-msbwt)."""
 import itertools
 
 import numpy as np

@@ -1,8 +1,8 @@
 """Pins the CPU oracle against every known-answer test the reference holds for the
 count_kmer / constrain_range path (SURVEY.md section 4 / 8c).  Citations are
-file:line under /root/reference/.  CPU only."""
+file:line in the reference (rust-msbwt).  CPU only."""
+import hashlib
 import itertools
-import os
 
 import numpy as np
 import pytest
@@ -166,11 +166,14 @@ def test_two_string_fixture(two_string_npy):
     assert nonzero == [4, 6, 4, 2, 0, 0, 0, 0]
 
 
-def test_reference_fixture_is_identical_when_reference_is_mounted(two_string_npy):
-    ref = "/root/reference/test_data/two_string.npy"
-    if not os.path.exists(ref):
-        pytest.skip("reference not mounted (GPU box)")
-    assert open(ref, "rb").read() == open(two_string_npy, "rb").read()
+def test_reference_fixture_copy_is_reproduced_by_the_oracle(two_string_npy, tmp_path):
+    """tests/golden/two_string.npy is a byte-identical copy of the reference's test_data/two_string.npy; its hash pins
+    the copy, and the oracle's writer must reproduce it from the fixture's two strings"""
+    raw = open(two_string_npy, "rb").read()
+    assert hashlib.sha256(raw).hexdigest() == "1849b221e871bcc1a137955db7c1659d4c140d727be18321ce64d917863991de"
+    p = str(tmp_path / "two_string.npy")
+    O.save_bwt_numpy(O.convert_to_vec(naive.naive_bwt(["ACGT", "TGCA"])), p)
+    assert open(p, "rb").read() == raw
 
 
 # ---- load_numpy_file error classes (rle_bwt.rs:84-147) ----
