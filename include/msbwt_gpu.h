@@ -339,6 +339,22 @@ int msbwt_build_rle_bwt(const uint8_t *reads, uint64_t n_reads, uint32_t read_le
  * equal suffixes by the lexicographic rank of their whole reads.  *total = sum of (length + 1). */
 int msbwt_build_rle_bwt_ragged(const uint8_t *syms, const uint64_t *offsets, uint64_t n_reads, int device,
                                uint8_t **rle, uint64_t *rle_len, uint64_t *total);
+/* Merge two multi-string BWTs (pairwise_bwt_merge, src/bwt_util.rs:108-141): Holt and McMillan's interleave, run on
+ * `device`.  `rle_a` / `rle_b` are host RLE byte streams, as msbwt_index_create_from_rle takes them (either may be
+ * empty).  The result is the stable interleave of both inputs' rows by their infinite forward symbol sequences (rows
+ * that tie keep A's before B's), in the canonical RLE encoding msbwt_build_rle_bwt emits.  For BWTs built from reads
+ * it is the BWT of the union of the two read sets, byte for byte what msbwt_build_rle_bwt(_ragged) makes from all the
+ * reads at once, and merge(A, B) == merge(B, A).  *rle is a buffer of *rle_len bytes owned by the caller (release it
+ * with msbwt_buffer_free); *total = N_A + N_B; *iterations (may be NULL) = interleave passes run, the last of which
+ * changed nothing (at most 2 L + 2 for reads of at most L symbols; 0 when both inputs are empty).
+ * Device memory: about 0.82 byte per merged symbol while iterating (the two inputs' one-step block images, 0.56; two
+ * interleave bit-vectors, 0.25), then 1 byte per merged symbol for the merged symbols plus the encoder's run table
+ * (17 bytes per run) and the RLE bytes.  While an input is loaded, the loader's scan buffers come on top for a moment
+ * (up to 26 bytes per RLE byte of that input, plus 0.56 byte per symbol).
+ * EINVAL: a NULL output pointer, or a NULL input with a length above 0.  EFORMAT: an input holds a symbol >= 6 or a
+ * run of 2^60 symbols or more, or N_A + N_B >= 2^62.  ENOMEM / ECUDA: nothing is leaked and *rle is NULL. */
+int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const uint8_t *rle_b, uint64_t len_b, int device,
+                         uint8_t **rle, uint64_t *rle_len, uint64_t *total, uint32_t *iterations /* may be NULL */);
 void msbwt_buffer_free(uint8_t *p);
 
 /* ---- the data format either side of the path: src/bwt_converter.rs ----

@@ -12,6 +12,7 @@ from .rle_bwt import (  # noqa: F401
     BWTRange,
     build_rle_bwt,
     build_rle_bwt_ragged,
+    merge_rle_bwts,
     MsbwtError,
     RleBWT,
     convert_itos,

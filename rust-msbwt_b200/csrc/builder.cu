@@ -145,16 +145,6 @@ __global__ void stamp_checkpoints_kernel(const uint64_t *__restrict__ before, ui
     aux[b * 2 + 1] = rel[4];
 }
 
-struct Scratch {
-    std::vector<void *> ptrs;
-    ~Scratch() { for (void *p : ptrs) cudaFree(p); }
-    template <class T> cudaError_t alloc(T **p, size_t count) {
-        cudaError_t e = cudaMalloc((void **)p, (count ? count : 1) * sizeof(T));
-        if (e == cudaSuccess) ptrs.push_back(*p);
-        return e;
-    }
-};
-
 #define B_TRY(expr)                                                                        \
     do {                                                                                   \
         cudaError_t e_ = (expr);                                                           \
@@ -170,7 +160,7 @@ int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift,
     if (len && !h_rle) { why = "rle is NULL"; return MSBWT_EINVAL; }
     if (sb_shift == 0) sb_shift = kDefaultSuperShift;
     if (sb_shift > (uint32_t)kDefaultSuperShift) { why = "superblock_shift > 25 would overflow the u32 block counters"; return MSBWT_EINVAL; }
-    Scratch tmp;
+    DeviceScratch tmp;
     uint8_t *d_rle = nullptr;
     uint64_t *d_before = nullptr, *d_run_byte = nullptr, *d_nruns = nullptr, *d_run_pos = nullptr;
     uint8_t *d_run_sym = nullptr;

@@ -15,6 +15,7 @@
 //   3. suffix: ids (rank of the read) * (L+1) + offset start in tie-break order; LSD over the suffix's
 //              21-symbol key words, extracted from the packed read by a funnel shift.
 //   4. emit  : BWT[i] = the symbol before suffix i ('$' for offset 0); run heads -> run table -> RLE bytes.
+//              (the last three steps are encode_rle_on_device, which the merge of bwt_merge.cu shares)
 // Reads of different lengths (create_from_fastx takes any, src/dynamic_bwt.rs:453-473) use the same padded layout
 // -- max length + 1 symbols per read, zeros after the '$' -- and simply list only the suffixes that exist (offsets
 // 0..len of every read): a shorter suffix ends in '$' = 0 followed by zeros, which is exactly how naive_bwt's
@@ -199,20 +200,6 @@ __global__ void emit_rle_kernel(const uint8_t *__restrict__ bwt, const uint64_t 
     while (len) { *out++ = (uint8_t)(sym | ((len & 31u) << 3)); len >>= 5; }
 }
 
-struct Scratch {
-    std::vector<void *> ptrs;
-    ~Scratch() { for (void *p : ptrs) cudaFree(p); }
-    template <class T> cudaError_t alloc(T **p, size_t count) {
-        cudaError_t e = cudaMalloc((void **)p, (count ? count : 1) * sizeof(T));
-        if (e == cudaSuccess) ptrs.push_back(*p);
-        return e;
-    }
-    void release(void *p) {
-        auto it = std::find(ptrs.begin(), ptrs.end(), p);
-        if (it != ptrs.end()) { cudaFree(p); ptrs.erase(it); }
-    }
-};
-
 #define W_TRY(expr)                                                                        \
     do {                                                                                   \
         cudaError_t e_ = (expr);                                                           \
@@ -239,7 +226,7 @@ int sort_pass(cub::DoubleBuffer<uint64_t> &keys, cub::DoubleBuffer<IdT> &ids, ui
 // nullptr: every read has l1 suffixes
 template <class IdT>
 int suffix_sort_and_emit(const uint64_t *d_sorted, uint64_t n_reads, uint64_t n, uint32_t l1, uint32_t stride_words, uint32_t key_words,
-                         const uint64_t *d_starts, const uint64_t *d_counts, uint8_t *d_bwt, Scratch &tmp, std::string &why,
+                         const uint64_t *d_starts, const uint64_t *d_counts, uint8_t *d_bwt, DeviceScratch &tmp, std::string &why,
                          int *launches) {
     uint64_t *k0 = nullptr, *k1 = nullptr;
     IdT *v0 = nullptr, *v1 = nullptr;
@@ -271,6 +258,84 @@ int suffix_sort_and_emit(const uint64_t *d_sorted, uint64_t n_reads, uint64_t n,
 
 }  // namespace
 
+// d_bwt: n symbol bytes on the current device -> *d_rle_out, a cudaMalloc'd buffer of *rle_len msbwt RLE bytes
+// (src/bwt_converter.rs:52-56; the caller frees it).  Shared by the builder above and the merge (bwt_merge.cu), so
+// both emit the same canonical encoding.
+int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, uint64_t *rle_len, std::string &why,
+                         int *launches) {
+    *d_rle_out = nullptr;
+    *rle_len = 0;
+    if (!n) return MSBWT_OK;
+    DeviceScratch tmp;
+    // run heads -> run table (select in chunks of 2^30 positions) -> digits -> RLE bytes
+    const uint64_t kChunk = 1ull << 30;
+    uint64_t *d_count = nullptr;
+    W_TRY(tmp.alloc(&d_count, 1));
+    void *d_temp = nullptr;
+    size_t temp_bytes = 0, need = 0;
+    using HeadIt = cub::TransformInputIterator<bool, RunHead, cub::CountingInputIterator<uint64_t>>;
+    using CountIt = cub::TransformInputIterator<uint64_t, RunHead, cub::CountingInputIterator<uint64_t>>;
+    {
+        cub::CountingInputIterator<uint64_t> idx(0);
+        HeadIt heads(idx, RunHead{d_bwt});
+        CountIt ones(idx, RunHead{d_bwt});
+        W_TRY(cub::DeviceReduce::Sum(nullptr, need, ones, d_count, (int64_t)std::min(kChunk, n)));
+        temp_bytes = need;
+        W_TRY(cub::DeviceSelect::Flagged(nullptr, need, idx, heads, (uint64_t *)nullptr, d_count, (int64_t)std::min(kChunk, n)));
+        temp_bytes = std::max(temp_bytes, need);
+    }
+    W_TRY(tmp.alloc((uint8_t **)&d_temp, temp_bytes));
+    uint64_t n_runs = 0;
+    std::vector<uint64_t> chunk_runs;
+    for (uint64_t b = 0; b < n; b += kChunk) {
+        cub::CountingInputIterator<uint64_t> idx(b);
+        CountIt ones(idx, RunHead{d_bwt});
+        size_t tb = temp_bytes;
+        W_TRY(cub::DeviceReduce::Sum(d_temp, tb, ones, d_count, (int64_t)std::min(kChunk, n - b)));
+        uint64_t c = 0;
+        W_TRY(cudaMemcpy(&c, d_count, sizeof(c), cudaMemcpyDeviceToHost));
+        chunk_runs.push_back(c);
+        n_runs += c;
+    }
+    uint64_t *d_starts = nullptr, *d_byte_offsets = nullptr;
+    uint8_t *d_ndigits = nullptr;
+    W_TRY(tmp.alloc(&d_starts, n_runs));
+    uint64_t done = 0;
+    for (uint64_t b = 0, ci = 0; b < n; b += kChunk, ci++) {
+        cub::CountingInputIterator<uint64_t> idx(b);
+        HeadIt heads(idx, RunHead{d_bwt});
+        size_t tb = temp_bytes;
+        W_TRY(cub::DeviceSelect::Flagged(d_temp, tb, idx, heads, d_starts + done, d_count, (int64_t)std::min(kChunk, n - b)));
+        done += chunk_runs[ci];
+    }
+    W_TRY(tmp.alloc(&d_ndigits, n_runs));
+    W_TRY(tmp.alloc(&d_byte_offsets, n_runs + 1));
+    run_digits_kernel<<<(unsigned)((n_runs + 255) / 256), 256>>>(d_starts, n_runs, n, d_ndigits);
+    W_TRY(cudaGetLastError());
+    {
+        cub::TransformInputIterator<uint64_t, WidenDigits, const uint8_t *> in(d_ndigits, WidenDigits{});
+        void *d_temp2 = nullptr;
+        size_t tb = 0;
+        W_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tb, in, d_byte_offsets, (int64_t)n_runs));
+        W_TRY(tmp.alloc((uint8_t **)&d_temp2, tb));
+        W_TRY(cub::DeviceScan::ExclusiveSum(d_temp2, tb, in, d_byte_offsets, (int64_t)n_runs));
+    }
+    uint64_t last_off = 0;
+    uint8_t last_nd = 0;
+    W_TRY(cudaMemcpy(&last_off, d_byte_offsets + (n_runs - 1), sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    W_TRY(cudaMemcpy(&last_nd, d_ndigits + (n_runs - 1), 1, cudaMemcpyDeviceToHost));
+    const uint64_t bytes = last_off + last_nd;
+    uint8_t *d_rle = nullptr;
+    W_TRY(cudaMalloc((void **)&d_rle, bytes));
+    emit_rle_kernel<<<(unsigned)((n_runs + 255) / 256), 256>>>(d_bwt, d_starts, d_byte_offsets, n_runs, n, d_rle);
+    if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) { cudaFree(d_rle); W_TRY(e); }
+    if (cudaError_t e = cudaDeviceSynchronize(); e != cudaSuccess) { cudaFree(d_rle); W_TRY(e); }
+    if (launches) *launches += 4;
+    *d_rle_out = d_rle;
+    *rle_len = bytes;
+    return MSBWT_OK;
+}
+
 // d_reads: symbol bytes (1..5) on the current device -- n_reads * read_len of them (d_offsets == nullptr: reads of one
 // length), or read r at d_reads[d_offsets[r] .. d_offsets[r + 1]) with read_len = the longest read (d_offsets: n_reads + 1
 // offsets on the device).  On success *d_rle_out is a cudaMalloc'd buffer of *rle_len RLE bytes (the caller frees it)
@@ -288,7 +353,7 @@ int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, u
     uint64_t n = n_reads * l1;  // (reads of different lengths: the suffixes that exist, counted below)
     const uint32_t words = (l1 + kKeySyms - 1) / kKeySyms;  // key words per read ('$' included)
     const uint32_t stride_words = words + 1;                // + one zero word for the funnel shift
-    Scratch tmp;
+    DeviceScratch tmp;
     uint64_t *d_packed = nullptr, *d_sorted = nullptr, *d_suffix_counts = nullptr, *d_suffix_starts = nullptr;
     uint32_t *d_bad = nullptr;
     uint8_t *d_bwt = nullptr;
@@ -360,72 +425,8 @@ int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, u
     if (rc != MSBWT_OK) return rc;
     tmp.release(d_sorted);
 
-    // 4b. run table -> RLE bytes (select in chunks of 2^30 positions)
-    const uint64_t kChunk = 1ull << 30;
-    uint64_t *d_count = nullptr;
-    W_TRY(tmp.alloc(&d_count, 1));
-    void *d_temp = nullptr;
-    size_t temp_bytes = 0, need = 0;
-    using HeadIt = cub::TransformInputIterator<bool, RunHead, cub::CountingInputIterator<uint64_t>>;
-    using CountIt = cub::TransformInputIterator<uint64_t, RunHead, cub::CountingInputIterator<uint64_t>>;
-    {
-        cub::CountingInputIterator<uint64_t> idx(0);
-        HeadIt heads(idx, RunHead{d_bwt});
-        CountIt ones(idx, RunHead{d_bwt});
-        W_TRY(cub::DeviceReduce::Sum(nullptr, need, ones, d_count, (int64_t)std::min(kChunk, n)));
-        temp_bytes = need;
-        W_TRY(cub::DeviceSelect::Flagged(nullptr, need, idx, heads, (uint64_t *)nullptr, d_count, (int64_t)std::min(kChunk, n)));
-        temp_bytes = std::max(temp_bytes, need);
-    }
-    W_TRY(tmp.alloc((uint8_t **)&d_temp, temp_bytes));
-    uint64_t n_runs = 0;
-    std::vector<uint64_t> chunk_runs;
-    for (uint64_t b = 0; b < n; b += kChunk) {
-        cub::CountingInputIterator<uint64_t> idx(b);
-        CountIt ones(idx, RunHead{d_bwt});
-        size_t tb = temp_bytes;
-        W_TRY(cub::DeviceReduce::Sum(d_temp, tb, ones, d_count, (int64_t)std::min(kChunk, n - b)));
-        uint64_t c = 0;
-        W_TRY(cudaMemcpy(&c, d_count, sizeof(c), cudaMemcpyDeviceToHost));
-        chunk_runs.push_back(c);
-        n_runs += c;
-    }
-    uint64_t *d_starts = nullptr, *d_byte_offsets = nullptr;
-    uint8_t *d_ndigits = nullptr;
-    W_TRY(tmp.alloc(&d_starts, n_runs));
-    uint64_t done = 0;
-    for (uint64_t b = 0, ci = 0; b < n; b += kChunk, ci++) {
-        cub::CountingInputIterator<uint64_t> idx(b);
-        HeadIt heads(idx, RunHead{d_bwt});
-        size_t tb = temp_bytes;
-        W_TRY(cub::DeviceSelect::Flagged(d_temp, tb, idx, heads, d_starts + done, d_count, (int64_t)std::min(kChunk, n - b)));
-        done += chunk_runs[ci];
-    }
-    W_TRY(tmp.alloc(&d_ndigits, n_runs));
-    W_TRY(tmp.alloc(&d_byte_offsets, n_runs + 1));
-    run_digits_kernel<<<(unsigned)((n_runs + 255) / 256), 256>>>(d_starts, n_runs, n, d_ndigits);
-    W_TRY(cudaGetLastError());
-    {
-        cub::TransformInputIterator<uint64_t, WidenDigits, const uint8_t *> in(d_ndigits, WidenDigits{});
-        void *d_temp2 = nullptr;
-        size_t tb = 0;
-        W_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tb, in, d_byte_offsets, (int64_t)n_runs));
-        W_TRY(tmp.alloc((uint8_t **)&d_temp2, tb));
-        W_TRY(cub::DeviceScan::ExclusiveSum(d_temp2, tb, in, d_byte_offsets, (int64_t)n_runs));
-    }
-    uint64_t last_off = 0;
-    uint8_t last_nd = 0;
-    W_TRY(cudaMemcpy(&last_off, d_byte_offsets + (n_runs - 1), sizeof(uint64_t), cudaMemcpyDeviceToHost));
-    W_TRY(cudaMemcpy(&last_nd, d_ndigits + (n_runs - 1), 1, cudaMemcpyDeviceToHost));
-    const uint64_t bytes = last_off + last_nd;
-    uint8_t *d_rle = nullptr;
-    W_TRY(cudaMalloc((void **)&d_rle, bytes));
-    emit_rle_kernel<<<(unsigned)((n_runs + 255) / 256), 256>>>(d_bwt, d_starts, d_byte_offsets, n_runs, n, d_rle);
-    if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) { cudaFree(d_rle); W_TRY(e); }
-    if (cudaError_t e = cudaDeviceSynchronize(); e != cudaSuccess) { cudaFree(d_rle); W_TRY(e); }
-    if (launches) *launches += 4;
-    *d_rle_out = d_rle;
-    *rle_len = bytes;
+    // 4b. run table -> RLE bytes
+    if (int rc2 = encode_rle_on_device(d_bwt, n, d_rle_out, rle_len, why, launches); rc2 != MSBWT_OK) return rc2;
     *total = n;
     return MSBWT_OK;
 }

@@ -1146,6 +1146,43 @@ extern "C" int msbwt_build_rle_bwt_ragged(const uint8_t *syms, const uint64_t *o
     return build_rle_bwt_common(syms + offsets[0], rebased.data(), n_reads, (uint32_t)longest, n_syms, 0, device, rle, rle_len, total);
 }
 
+extern "C" int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const uint8_t *rle_b, uint64_t len_b, int device,
+                                    uint8_t **rle, uint64_t *rle_len, uint64_t *total, uint32_t *iterations) {
+    g_last_error.clear();
+    if (!rle || !rle_len || !total) return fail(MSBWT_EINVAL, "NULL output pointer");
+    *rle = nullptr;
+    *rle_len = 0;
+    *total = 0;
+    if (iterations) *iterations = 0;
+    if ((len_a && !rle_a) || (len_b && !rle_b)) return fail(MSBWT_EINVAL, "NULL input with a length above 0");
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(MSBWT_ENODEV, "no usable CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= count) return fail(MSBWT_ENODEV, "device ordinal out of range");
+    DeviceGuard guard(device);
+    uint8_t *d_rle = nullptr;
+    uint64_t len = 0, n = 0;
+    uint32_t passes = 0;
+    std::string why;
+    int launches = 0;
+    int rc = merge_rle_bwts_on_device(rle_a, len_a, rle_b, len_b, &d_rle, &len, &n, &passes, why, &launches);
+    g_launches += (uint64_t)launches;
+    struct DevPtr { void *p; ~DevPtr() { if (p) cudaFree(p); } } d_rle_owner{d_rle};
+    if (rc != MSBWT_OK) return fail(rc, why);
+    uint8_t *host = (uint8_t *)malloc(len ? len : 1);
+    if (!host) return fail(MSBWT_ENOMEM, "host buffer for the RLE bytes");
+    if (len) {
+        if (cudaError_t e = cudaMemcpy(host, d_rle, len, cudaMemcpyDeviceToHost); e != cudaSuccess) {
+            free(host);
+            return fail(MSBWT_ECUDA, std::string("copying the RLE bytes: ") + cudaGetErrorString(e));
+        }
+    }
+    *rle = host;
+    *rle_len = len;
+    *total = n;
+    if (iterations) *iterations = passes;
+    return MSBWT_OK;
+}
+
 extern "C" void msbwt_buffer_free(uint8_t *p) { free(p); }
 
 // ================================================================ measurement aid

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstdint>
 #include <string>
 #include <vector>
@@ -10,6 +11,28 @@
 #include "layout.h"
 
 namespace msbwt {
+
+// cudaMalloc'd scratch buffers of one build step: whatever is still listed is freed when it goes out of scope
+struct DeviceScratch {
+    std::vector<void *> ptrs;
+    DeviceScratch() = default;
+    DeviceScratch(const DeviceScratch &) = delete;
+    DeviceScratch &operator=(const DeviceScratch &) = delete;
+    ~DeviceScratch() { release_all(); }
+    template <class T> cudaError_t alloc(T **p, size_t count) {
+        cudaError_t e = cudaMalloc((void **)p, (count ? count : 1) * sizeof(T));
+        if (e == cudaSuccess) ptrs.push_back(*p);
+        return e;
+    }
+    void release(void *p) {
+        auto it = std::find(ptrs.begin(), ptrs.end(), p);
+        if (it != ptrs.end()) { cudaFree(p); ptrs.erase(it); }
+    }
+    void release_all() {
+        for (void *p : ptrs) cudaFree(p);
+        ptrs.clear();
+    }
+};
 
 constexpr int kCountThreads = 256;
 constexpr uint64_t kMaxPerLaunch = 1ull << 30;  // queries per pack/count launch (u32 indices inside the kernels)
@@ -124,6 +147,15 @@ void free_fin_image(FinImage &img);
 // of read_len symbols each; otherwise read r = d_reads[d_offsets[r] .. d_offsets[r + 1]) and read_len = the longest ----
 int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, uint64_t n_reads, uint32_t read_len,
                             uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, std::string &why, int *launches);
+// n symbol bytes (device) -> their msbwt RLE bytes (a cudaMalloc'd device buffer the caller frees); step 4b of the builder
+int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, uint64_t *rle_len, std::string &why,
+                         int *launches);
+
+// ---- bwt_merge.cu: two RLE byte streams (host) -> RLE bytes of their Holt-McMillan merge (device buffer the caller
+// frees); *iterations = interleave passes run, the last of which changed nothing ----
+int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8_t *h_rle_b, uint64_t len_b,
+                             uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, uint32_t *iterations,
+                             std::string &why, int *launches);
 
 // return an msbwt_status; on failure `why` explains
 int validate_rle(const uint8_t *rle, uint64_t len, std::string &why);

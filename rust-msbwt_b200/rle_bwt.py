@@ -153,6 +153,7 @@ def load_library():
         "msbwt_debug_copy_image": (i32, [vp, i32, C.POINTER(u64), C.POINTER(u32), vp, vp, vp]),
         "msbwt_build_rle_bwt": (i32, [vp, u64, u32, i32, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]),
         "msbwt_build_rle_bwt_ragged": (i32, [vp, vp, u64, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]),
+        "msbwt_merge_rle_bwts": (i32, [vp, u64, vp, u64, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(u32)]),
         "msbwt_buffer_free": (None, [vp]),
         "msbwt_convert_to_rle": (i32, [vp, u64, C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_save_rle_npy": (i32, [vp, u64, C.c_char_p]),
@@ -182,7 +183,7 @@ EXPORTED_SYMBOLS = (
     "msbwt_count_kmers_fixed", "msbwt_constrain_ranges", "msbwt_count_kmers_fixed_device",
     "msbwt_constrain_ranges_device", "msbwt_packed_bytes", "msbwt_pack_kmers_device",
     "msbwt_count_kmers_packed_device", "msbwt_launch_count", "msbwt_gather_bench", "msbwt_l2_fetch_granularity", "msbwt_debug_build_image", "msbwt_debug_copy_image",
-    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
+    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_merge_rle_bwts", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
     "msbwt_save_runs_npy",
     "msbwt_host_free", "msbwt_last_error", "msbwt_abi_version",
 )
@@ -610,6 +611,23 @@ def build_rle_bwt_ragged(reads, device: int = 0) -> tuple[np.ndarray, int]:
     finally:
         L.msbwt_buffer_free(out)
     return rle, int(total.value)
+
+
+def merge_rle_bwts(rle_a, rle_b, device: int = 0) -> tuple[np.ndarray, int, int]:
+    """Merge two multi-string BWTs (msbwt RLE bytes) on the GPU: Holt and McMillan's interleave, as the reference's
+    pairwise_bwt_merge (src/bwt_util.rs:108-141).  For BWTs built from reads the result is the BWT of the union of the
+    read sets, byte for byte what build_rle_bwt(_ragged) makes from all the reads.  Returns (rle bytes, total symbols,
+    interleave passes run -- the last of which changed nothing)."""
+    L = load_library()
+    a, b = _u8(rle_a).reshape(-1), _u8(rle_b).reshape(-1)
+    out, nbytes, total, iters = C.c_void_p(0), C.c_uint64(0), C.c_uint64(0), C.c_uint32(0)
+    _check(L.msbwt_merge_rle_bwts(_p(a) if a.size else None, a.size, _p(b) if b.size else None, b.size, device, C.byref(out),
+                                  C.byref(nbytes), C.byref(total), C.byref(iters)), "merge_rle_bwts")
+    try:
+        rle = np.ctypeslib.as_array(C.cast(out, C.POINTER(C.c_uint8)), shape=(nbytes.value,)).copy() if nbytes.value else np.zeros(0, np.uint8)
+    finally:
+        L.msbwt_buffer_free(out)
+    return rle, int(total.value), int(iters.value)
 
 
 def convert_to_vec(text) -> np.ndarray:
