@@ -356,6 +356,32 @@ int msbwt_build_rle_bwt_ragged(const uint8_t *syms, const uint64_t *offsets, uin
 int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const uint8_t *rle_b, uint64_t len_b, int device,
                          uint8_t **rle, uint64_t *rle_len, uint64_t *total, uint32_t *iterations /* may be NULL */);
 void msbwt_buffer_free(uint8_t *p);
+/* The k-mer spectrum of the index, and optionally its k-mers.  S = every string X of k symbols over {A,C,G,T}
+ * (1 <= k <= 32) with count_kmer(X) >= min_count (>= 1), count_kmer being BWT::count_kmer (src/msbwt_core.rs:125-161),
+ * i.e. what msbwt_count_kmers_u64 returns for X; for a BWT built from reads, the occurrences of X inside the reads (X
+ * never spans a read boundary or an N).  *n_kmers = |S|.  hist: nbins u64 (may be NULL when nbins == 0);
+ * hist[c] = #{X in S : count = c} for c < nbins - 1 and hist[nbins - 1] = #{X in S : count >= nbins - 1}, so entries
+ * below min_count and hist[0] are 0.  kmers / counts: both NULL (histogram only) or both non-NULL, in which case *kmers
+ * and *counts become buffers of *n_kmers u64 owned by the caller (release each with msbwt_buffer_free; NULL when
+ * *n_kmers == 0): S in msbwt_count_kmers_u64's encoding (A,C,G,T = 0..3, first symbol in the most significant of the
+ * 2k bits, upper bits zero) in co-lexicographic order -- ascending by the last symbol, then the one before it, and so
+ * on -- with their counts.  Two calls return identical arrays.
+ * The walk is a depth-first backward search from [0, N) that extends every surviving range by A, C, G and T and drops
+ * ranges narrower than min_count, over slices of at most B = 2^20 ranges per depth.  It reads only the one-step
+ * blocks, so it works the same whatever images the index carries, and runs on the handle's first replica on a stream
+ * and scratch of its own (it may run concurrently with queries on the same handle).
+ * Device memory: at most (k - 1) * 4B stored ranges of 8 bytes (16 with 64-bit positions), plus 8 bytes each for the
+ * packed k-mer when the list is requested, one slice's 4B children before compaction, 4B flag bytes, 2^22 staged
+ * (k-mer, count) pairs of 16 bytes when the list is requested, nbins * 8 bytes and CUB's scratch: independent of N and
+ * of |S| (and no buffer is larger than N / min_count entries).  At k = 31 with 32-bit positions: 1.0 GB for the
+ * histogram, 2.1 GB with the list.  Host memory for the list grows with |S| (16 bytes per k-mer, and up to twice that
+ * while a buffer grows).
+ * EINVAL (nothing written): k == 0 or k > 32, min_count == 0, n_kmers NULL, hist NULL with nbins > 0, nbins == 1 or
+ * nbins > 2^20, exactly one of kmers / counts NULL.  An index with no ACGT k-mer of length k (or min_count > N) gives
+ * *n_kmers = 0 and an all-zero hist.  ENOMEM / ECUDA: nothing is leaked, nothing is left running on the device and
+ * *kmers / *counts are NULL. */
+int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist, uint32_t nbins,
+                        uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers);
 
 /* ---- the data format either side of the path: src/bwt_converter.rs ----
  * convert_to_vec (:26-80): a text BWT over `$ACGNT` (newlines are skipped and do not end a run) -> msbwt RLE bytes

@@ -139,6 +139,26 @@ class RleBWT {
         check(msbwt_count_read_kmers(h_, reads.data(), read_len, n, k, both_strands ? 2 : 1, out.data()));
         return out;
     }
+    // the k-mer spectrum (hist: nbins entries, the last one = count >= nbins - 1) and, with want_list, the k-mers with
+    // count >= min_count and their counts in co-lexicographic order (k <= 32; msbwt_count_kmers_u64's encoding)
+    struct KmerSpectrum {
+        std::vector<uint64_t> hist, kmers, counts;
+        uint64_t n_kmers = 0;
+    };
+    KmerSpectrum kmer_spectrum(uint32_t k, uint64_t min_count = 1, uint32_t nbins = 10001, bool want_list = false) const {
+        KmerSpectrum out;
+        out.hist.assign(nbins, 0);
+        uint64_t *km = nullptr, *cn = nullptr;
+        check(msbwt_kmer_spectrum(h_, k, min_count, nbins ? out.hist.data() : nullptr, nbins, want_list ? &km : nullptr,
+                                  want_list ? &cn : nullptr, &out.n_kmers));
+        if (km) {
+            out.kmers.assign(km, km + out.n_kmers);
+            out.counts.assign(cn, cn + out.n_kmers);
+        }
+        msbwt_buffer_free(reinterpret_cast<uint8_t *>(km));
+        msbwt_buffer_free(reinterpret_cast<uint8_t *>(cn));
+        return out;
+    }
     const msbwt_index *handle() const { return h_; }
 
   private:

@@ -1183,6 +1183,30 @@ extern "C" int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const 
     return MSBWT_OK;
 }
 
+extern "C" int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist, uint32_t nbins,
+                                   uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
+    g_last_error.clear();
+    if (!idx || idx->reps.empty()) return fail(MSBWT_EINVAL, "bad handle");
+    if (!k || k > 32) return fail(MSBWT_EINVAL, "kmer_spectrum: k must be in 1..32");
+    if (!min_count) return fail(MSBWT_EINVAL, "kmer_spectrum: min_count must be at least 1");
+    if (!n_kmers) return fail(MSBWT_EINVAL, "kmer_spectrum: NULL n_kmers");
+    if (nbins && !hist) return fail(MSBWT_EINVAL, "kmer_spectrum: NULL hist with nbins > 0");
+    if (nbins == 1 || nbins > (1u << 20)) return fail(MSBWT_EINVAL, "kmer_spectrum: nbins must be 0 or in 2..2^20");
+    if (!kmers != !counts) return fail(MSBWT_EINVAL, "kmer_spectrum: kmers and counts must be both NULL or both set");
+    *n_kmers = 0;
+    if (kmers) *kmers = *counts = nullptr;
+    // replica 0's images are read-only after create; the call has its own stream and scratch, so it takes no lock and
+    // runs beside the query entry points
+    const Replica &rep = *idx->reps[0];
+    DeviceGuard guard(rep.device);
+    std::string why;
+    int launches = 0;
+    const int rc = kmer_spectrum_on_device(rep.device, rep.view, k, min_count, hist, nbins, kmers, counts, n_kmers, why,
+                                           &launches);
+    g_launches += (uint64_t)launches;
+    return rc == MSBWT_OK ? rc : fail(rc, why);
+}
+
 extern "C" void msbwt_buffer_free(uint8_t *p) { free(p); }
 
 // ================================================================ measurement aid

@@ -157,6 +157,13 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
                              uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, uint32_t *iterations,
                              std::string &why, int *launches);
 
+// ---- spectrum.cu: the k-mer spectrum of an index (one replica, on the current device): hist[nbins] (nbins may be 0)
+// and *n_kmers; when `kmers` is not null, also the k-mers with count >= min_count and their counts in co-lexicographic
+// order (*kmers, *counts: malloc'd host arrays the caller frees, null when there are none).  1 <= k <= 32, min_count >= 1.
+int kmer_spectrum_on_device(int device, const IndexView &ix, uint32_t k, uint64_t min_count, uint64_t *hist,
+                            uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers, std::string &why,
+                            int *launches);
+
 // return an msbwt_status; on failure `why` explains
 int validate_rle(const uint8_t *rle, uint64_t len, std::string &why);
 int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, HostImage &img, std::string &why);
