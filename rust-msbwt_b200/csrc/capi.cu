@@ -86,9 +86,50 @@ int finish_replica(msbwt_index *idx, size_t slot, std::unique_ptr<Replica> rep, 
     rep->view.nblocks = nblocks;
     rep->view.n_super = n_super;
     rep->view.sb_shift = sb_shift;
-    if (slot == 0) idx->bytes_per_replica = nblocks * kBlockBytes + nblocks * 2 * sizeof(uint32_t) + (uint64_t)n_super * 8 * sizeof(uint64_t);
     idx->reps[slot] = std::move(rep);
     return MSBWT_OK;
+}
+
+// The optional-image fields of the view, from what the replica owns: an image that was never built or has been freed
+// reads as null / 0.  Called after every build stage that adds or frees an image.
+void refresh_view(Replica &rep) {
+    IndexView &v = rep.view;
+    v.table = rep.d_table;
+    v.table2 = rep.d_table_lower[0];
+    v.table3 = rep.d_table_lower[1];
+    v.table4 = rep.d_table_lower[2];
+    v.table_s = rep.table_s;
+    v.pair = rep.pair.lines;
+    v.c2base = rep.pair.c2base;
+    v.npair = rep.pair.npair;
+    v.n_super2 = rep.pair.n_super2;
+    v.quad = rep.quad.sectors;
+    v.c4base = rep.quad.c4base;
+    v.nsec4 = rep.quad.nsec4;
+    v.n_super4 = rep.quad.n_super4;
+    v.sb_shift4 = rep.quad.sb_shift4;
+    v.oct = rep.oct.lines;
+    v.nbuck8 = rep.oct.nbuck8;
+    v.oct_shift = (uint32_t)rep.oct.shift;
+    v.fin = rep.fin.lines;
+    v.fin_shift = (uint32_t)rep.fin.shift;
+    v.fin_lb = (uint32_t)rep.fin.lb;
+}
+
+// Device memory of the images one replica holds (msbwt_index_bytes)
+uint64_t replica_bytes(const Replica &rep) {
+    const IndexView &v = rep.view;
+    uint64_t b = v.nblocks * kBlockBytes + v.nblocks * 2 * sizeof(uint32_t) + (uint64_t)v.n_super * 8 * sizeof(uint64_t);
+    b += rep.pair.npair * kPairBytes + (rep.pair.c2base ? (uint64_t)rep.pair.n_super2 * 16 * sizeof(uint64_t) : 0);
+    b += (uint64_t)kQuadCodes * rep.quad.nsec4 * kQuadSectorBytes +
+         (rep.quad.c4base ? (uint64_t)rep.quad.n_super4 * kQuadCodes * sizeof(uint64_t) : 0);
+    b += (uint64_t)kOctCodes * rep.oct.nbuck8 * kOctLineBytes;
+    b += rep.fin.nlines * (uint64_t)kFinLineBytes;
+    const uint64_t eb = index_is_wide(v) ? 16 : 8;
+    if (rep.d_table) b += (1ull << (2 * rep.table_s)) * eb;
+    for (int j = 1; j <= 3; j++)
+        if (rep.d_table_lower[j - 1]) b += (1ull << (2 * (rep.table_s - j))) * eb;
+    return b;
 }
 
 // Default load path: the block image is built on each device from the RLE bytes (builder.cu).
@@ -216,10 +257,6 @@ bool pick_pair(int device, uint64_t index_bytes, int requested) {
     return lives_in_hbm(device, index_bytes);
 }
 
-uint64_t pair_image_bytes(const PairImage &p) {
-    return p.npair * kPairBytes + (p.c2base ? (uint64_t)p.n_super2 * 16 * sizeof(uint64_t) : 0);
-}
-
 int build_pair(msbwt_index *idx, Replica &rep, uint8_t **keep_codes = nullptr) {
     DeviceGuard guard(rep.device);
     std::string why;
@@ -227,11 +264,7 @@ int build_pair(msbwt_index *idx, Replica &rep, uint8_t **keep_codes = nullptr) {
     int rc = build_pair_image_on_device(rep.device, rep.view, idx->start, rep.pair, why, &n, keep_codes);
     g_launches += (uint64_t)n;
     if (rc != MSBWT_OK) { free_pair_image(rep.pair); return fail(rc, why); }
-    rep.view.pair = rep.pair.lines;
-    rep.view.c2base = rep.pair.c2base;
-    rep.view.npair = rep.pair.npair;
-    rep.view.n_super2 = rep.pair.n_super2;
-    if (idx->reps[0].get() == &rep) idx->bytes_per_replica += pair_image_bytes(rep.pair);
+    refresh_view(rep);
     return MSBWT_OK;
 }
 
@@ -281,17 +314,38 @@ int env_int(const char *name, int fallback) {
     return e ? atoi(e) : fallback;
 }
 
-void drop_quad(msbwt_index *idx, Replica &rep) {
-    if (!rep.quad.sectors) return;
-    if (idx->reps[0].get() == &rep)
-        idx->bytes_per_replica -= (uint64_t)kQuadCodes * rep.quad.nsec4 * kQuadSectorBytes +
-                                  (rep.quad.c4base ? (uint64_t)rep.quad.n_super4 * kQuadCodes * sizeof(uint64_t) : 0);
-    free_quad_image(rep.quad);
-    rep.view.quad = nullptr;
-    rep.view.c4base = nullptr;
-    rep.view.nsec4 = 0;
-    rep.view.n_super4 = 0;
-    rep.view.sb_shift4 = 0;
+// The environment fills the image knobs the caller left unset (-1, or 0 for the shifts), before any builder reads them
+void fill_from_env(Options &o) {
+    if (o.keep_quad == -1) o.keep_quad = env_int("MSBWT_KEEP_QUAD", -1);
+    if (o.fin == -1) o.fin = env_int("MSBWT_FINAL_INDEX", -1);
+    if (!o.fin_shift) o.fin_shift = env_int("MSBWT_FINAL_BUCKET_SHIFT", 16);
+    if (!o.fin_lb) o.fin_lb = env_int("MSBWT_FINAL_LINES_LOG2", 0);
+    if (!o.oct_shift) o.oct_shift = env_int("MSBWT_OCT_BUCKET_SHIFT", 0);
+}
+
+// Lines per final-step bucket: 2^13, 16 bytes per symbol (0.8 % of the read-sampled 31-mers find their line overflowed
+// and take the oct steps), when that fits 30 % of the device (48 GB at 3.02 Gsymbols), else 2^12, 8 bytes per symbol
+// (6.5 %)
+int fin_lines_log2(const Options &opt, uint64_t N, uint64_t device_bytes) {
+    if (opt.fin_lb) return opt.fin_lb;
+    return fin_image_bytes(N, opt.fin_shift, 13) <= device_bytes / 10 * 3 ? 13 : 12;
+}
+
+// The final-step lines on top of the oct image, from the 20-symbol codes (owned by the builder from here on).  Running out
+// of device memory leaves the index without this image unless the caller required it.
+int build_fin(Replica &rep, const Options &opt, uint64_t *codes20, int flb) {
+    std::string why;
+    int n = 0;
+    int rc = build_fin_lines_on_device(rep.device, rep.view.total, codes20, opt.fin_shift, flb, rep.fin, why, &n);
+    g_launches += (uint64_t)n;
+    if (rc != MSBWT_OK) {
+        free_fin_image(rep.fin);
+        if (rc == MSBWT_ENOMEM && opt.fin != 1) { cudaGetLastError(); return MSBWT_OK; }
+        return fail(rc, why);
+    }
+    refresh_view(rep);
+    build_trace("multi-step images done");
+    return MSBWT_OK;
 }
 
 // The multi-step images of an index that lives in HBM, built on the replica's device in stages so that the peak
@@ -307,40 +361,25 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
     uint8_t *codes2 = nullptr;
     if (int rc = build_pair(idx, rep, &codes2); rc != MSBWT_OK) return rc;
     DeviceGuard guard(rep.device);
-    struct DevPtr { void *p = nullptr; ~DevPtr() { if (p) cudaFree(p); } void reset() { if (p) cudaFree(p); p = nullptr; } };
-    DevPtr codes2_owner, codes10_owner;
-    codes2_owner.p = codes2;
+    DevicePtr<uint8_t> codes2_owner(codes2);
     const bool want_oct = pick_oct(rep.view, opt.oct);
-    const int fin_req = opt.fin != -1 ? opt.fin : env_int("MSBWT_FINAL_INDEX", -1);
-    const bool want_fin = want_oct && fin_req != 0;
+    const bool want_fin = want_oct && opt.fin != 0;
     uint16_t *codes4 = nullptr;
     std::string why;
     int n = 0;
     build_trace("quad image");
     int rc = build_quad_image_on_device(rep.device, rep.view, codes2, rep.quad, why, &n, want_oct ? &codes4 : nullptr);
     g_launches += (uint64_t)n;
-    if (idx->reps[0].get() == &rep) idx->bytes_per_replica -= pair_image_bytes(rep.pair);
     free_pair_image(rep.pair);
-    rep.view.pair = nullptr;
-    rep.view.c2base = nullptr;
-    rep.view.npair = 0;
-    rep.view.n_super2 = 0;
     if (rc != MSBWT_OK) { free_quad_image(rep.quad); if (codes4) cudaFree(codes4); return fail(rc, why); }
-    rep.view.quad = rep.quad.sectors;
-    rep.view.c4base = rep.quad.c4base;
-    rep.view.nsec4 = rep.quad.nsec4;
-    rep.view.n_super4 = rep.quad.n_super4;
-    rep.view.sb_shift4 = rep.quad.sb_shift4;
-    const uint64_t quad_bytes = (uint64_t)kQuadCodes * rep.quad.nsec4 * kQuadSectorBytes +
-                                (rep.quad.c4base ? (uint64_t)rep.quad.n_super4 * kQuadCodes * sizeof(uint64_t) : 0);
-    if (idx->reps[0].get() == &rep) idx->bytes_per_replica += quad_bytes;
+    refresh_view(rep);
     if (!want_oct) return MSBWT_OK;
 
     const uint64_t N = rep.view.total;
     size_t free_b = 0, total_b = 0;
     if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { free_b = 0; total_b = 0; }
-    int keep_quad = opt.keep_quad != -1 ? opt.keep_quad : env_int("MSBWT_KEEP_QUAD", -1);
-    if (keep_quad == -1) keep_quad = quad_bytes + 40 * N <= (uint64_t)total_b / 10 * 7 ? 1 : 0;
+    int keep_quad = opt.keep_quad;
+    if (keep_quad == -1) keep_quad = quad_image_bytes(N) + 40 * N <= (uint64_t)total_b / 10 * 7 ? 1 : 0;
 
     // 10-symbol codes (4 B per position), then 20-symbol codes (8 B per position): both walk LF^4 through the quad image
     uint32_t *codes10 = nullptr;
@@ -349,42 +388,38 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
     rc = build_oct_codes_on_device(rep.device, rep.view, codes4, codes2, &codes10, why, &n);  // frees codes4
     g_launches += (uint64_t)n;
     if (rc != MSBWT_OK) return fail(rc, why);
-    codes10_owner.p = codes10;
+    DevicePtr<uint32_t> codes10_owner(codes10);
     codes2_owner.reset();
+    const int flb = fin_lines_log2(opt, N, total_b);
     uint64_t *codes20 = nullptr;
-    int fshift = opt.fin_shift ? opt.fin_shift : env_int("MSBWT_FINAL_BUCKET_SHIFT", 16);
-    int flb = opt.fin_lb ? opt.fin_lb : env_int("MSBWT_FINAL_LINES_LOG2", 0);
     if (want_fin) {
-        // 16 bytes per symbol (0.8 % of the read-sampled 31-mers find their line overflowed and take the oct steps) when
-        // that fits 30 % of the device (48 GB at 3.02 Gsymbols), else 8 bytes per symbol (6.5 %)
-        if (!flb) flb = fin_image_bytes(N, fshift, 13) <= (uint64_t)total_b / 10 * 3 ? 13 : 12;
         n = 0;
         rc = build_fin_codes_on_device(rep.device, rep.view, codes10, &codes20, why, &n);
         g_launches += (uint64_t)n;
-        if (rc == MSBWT_ENOMEM && fin_req != 1) {  // no room for the codes: the index works without this image
+        if (rc == MSBWT_ENOMEM && opt.fin != 1) {  // no room for the codes: the index works without this image
             cudaGetLastError();
             codes20 = nullptr;
         } else if (rc != MSBWT_OK) {
             return fail(rc, why);
         }
     }
-    struct Codes20 { uint64_t *p; ~Codes20() { if (p) cudaFree(p); } } codes20_owner{codes20};
+    DevicePtr<uint64_t> codes20_owner(codes20);
     if (!keep_quad) {
         build_trace("dropping the quad image");
-        drop_quad(idx, rep);
+        free_quad_image(rep.quad);
+        refresh_view(rep);
     }
 
     // oct lines: what is left after the final-step lines, their sort scratch (about 16 B per position, of which the
     // 12 B per position of the two code arrays are free again by then) and 8 GB for the suffix table and the query
     // pipeline; the builder picks coarser buckets, or builds nothing, beyond that
     if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) free_b = 0;
-    const uint64_t fin_need = codes20 ? fin_image_bytes(N, fshift, flb) + 4 * N : 0;
+    const uint64_t fin_need = codes20 ? fin_image_bytes(N, opt.fin_shift, flb) + 4 * N : 0;
     const uint64_t reserve = fin_need + (opt.oct == 1 ? 0 : (8ull << 30));
     const uint64_t budget = free_b > reserve ? free_b - reserve : 0;
-    int oct_shift = opt.oct_shift ? opt.oct_shift : env_int("MSBWT_OCT_BUCKET_SHIFT", 0);
     n = 0;
     build_trace("oct lines");
-    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, oct_shift, budget, rep.oct, why, &n);
+    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, opt.oct_shift, budget, rep.oct, why, &n);
     g_launches += (uint64_t)n;
     codes10_owner.reset();
     if (rc != MSBWT_OK) { free_oct_image(rep.oct); return fail(rc, why); }
@@ -392,28 +427,8 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
         if (!rep.view.quad) return fail(MSBWT_ENOMEM, "no room for the oct image after the quad image was dropped (MSBWT_KEEP_QUAD=1 keeps it)");
         return MSBWT_OK;
     }
-    rep.view.oct = rep.oct.lines;
-    rep.view.nbuck8 = rep.oct.nbuck8;
-    rep.view.oct_shift = (uint32_t)rep.oct.shift;
-    if (idx->reps[0].get() == &rep) idx->bytes_per_replica += (uint64_t)kOctCodes * rep.oct.nbuck8 * kOctLineBytes;
-
-    if (codes20) {  // final-step lines on top of the oct image
-        n = 0;
-        codes20_owner.p = nullptr;  // owned by the builder from here
-        rc = build_fin_lines_on_device(rep.device, N, codes20, fshift, flb, rep.fin, why, &n);
-        g_launches += (uint64_t)n;
-        if (rc == MSBWT_ENOMEM && fin_req != 1) {  // the index works without this image
-            cudaGetLastError();
-            free_fin_image(rep.fin);
-            rep.fin = FinImage{};
-            return MSBWT_OK;
-        }
-        if (rc != MSBWT_OK) { free_fin_image(rep.fin); return fail(rc, why); }
-        rep.view.fin = rep.fin.lines;
-        rep.view.fin_shift = (uint32_t)rep.fin.shift;
-        rep.view.fin_lb = (uint32_t)rep.fin.lb;
-        if (idx->reps[0].get() == &rep) idx->bytes_per_replica += rep.fin.nlines * (uint64_t)kFinLineBytes;
-    }
+    refresh_view(rep);
+    if (codes20) return build_fin(rep, opt, codes20_owner.release(), flb);
     build_trace("multi-step images done");
     return MSBWT_OK;
 }
@@ -426,12 +441,10 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
 //   10-symbol codes -> oct lines -> 20-symbol codes (10-symbol codes dropped) -> final-step lines.
 // `required` false (automatic choice): running out of device memory leaves the index without these images
 // (*built = false, MSBWT_OK) and the caller falls back to the pair image.
-int build_multi_step_wide(msbwt_index *idx, Replica &rep, const Options &opt, bool required, bool *built) {
+int build_multi_step_wide(Replica &rep, const Options &opt, bool required, bool *built) {
     *built = false;
     DeviceGuard guard(rep.device);
-    struct DevPtr { void *p = nullptr; ~DevPtr() { if (p) cudaFree(p); } void reset() { if (p) cudaFree(p); p = nullptr; } };
     const uint64_t N = rep.view.total;
-    const int fin_req = opt.fin != -1 ? opt.fin : env_int("MSBWT_FINAL_INDEX", -1);
     std::string why;
     int n = 0;
     auto soft = [&](int rc) {  // out of memory on an automatic build: the index works without these images
@@ -439,44 +452,36 @@ int build_multi_step_wide(msbwt_index *idx, Replica &rep, const Options &opt, bo
         return false;
     };
 
-    DevPtr codes10_owner;
     uint32_t *codes10 = nullptr;
     build_trace("10-symbol codes (walk)");
     int rc = build_oct_codes_by_walk(rep.device, rep.view, &codes10, why, &n);
     g_launches += (uint64_t)n;
     if (rc != MSBWT_OK) return soft(rc) ? MSBWT_OK : fail(rc, why);
-    codes10_owner.p = codes10;
+    DevicePtr<uint32_t> codes10_owner(codes10);
 
     size_t free_b = 0, total_b = 0;
     if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { free_b = 0; total_b = 0; }
-    const int fshift = opt.fin_shift ? opt.fin_shift : env_int("MSBWT_FINAL_BUCKET_SHIFT", 16);
-    int flb = opt.fin_lb ? opt.fin_lb : env_int("MSBWT_FINAL_LINES_LOG2", 0);
-    if (!flb) flb = fin_image_bytes(N, fshift, 13) <= (uint64_t)total_b / 10 * 3 ? 13 : 12;
+    const int flb = fin_lines_log2(opt, N, total_b);
     // what the final-step image will need after the oct lines exist: its lines, the 20-symbol codes (8 B per
     // position) and the run records + sort scratch (4 B per position once the codes are gone)
-    const uint64_t fin_need = fin_req != 0 ? fin_image_bytes(N, fshift, flb) + 12 * N : 0;
+    const uint64_t fin_need = opt.fin != 0 ? fin_image_bytes(N, opt.fin_shift, flb) + 12 * N : 0;
     const uint64_t reserve = fin_need + (opt.oct == 1 ? 0 : (8ull << 30));
     const uint64_t budget = free_b > reserve ? free_b - reserve : 0;
-    const int oct_shift = opt.oct_shift ? opt.oct_shift : env_int("MSBWT_OCT_BUCKET_SHIFT", 0);
     n = 0;
     build_trace("oct lines");
-    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, oct_shift, budget, rep.oct, why, &n);
+    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, opt.oct_shift, budget, rep.oct, why, &n);
     g_launches += (uint64_t)n;
     if (rc != MSBWT_OK) {
         free_oct_image(rep.oct);
-        rep.oct = OctImage{};
         return soft(rc) ? MSBWT_OK : fail(rc, why);
     }
     if (!rep.oct.lines) {
         if (required) return fail(MSBWT_ENOMEM, "no room for the oct image of this index");
         return MSBWT_OK;
     }
-    rep.view.oct = rep.oct.lines;
-    rep.view.nbuck8 = rep.oct.nbuck8;
-    rep.view.oct_shift = (uint32_t)rep.oct.shift;
-    if (idx->reps[0].get() == &rep) idx->bytes_per_replica += (uint64_t)kOctCodes * rep.oct.nbuck8 * kOctLineBytes;
+    refresh_view(rep);
     *built = true;
-    if (fin_req == 0) return MSBWT_OK;
+    if (opt.fin == 0) return MSBWT_OK;
 
     uint64_t *codes20 = nullptr;
     n = 0;
@@ -484,24 +489,10 @@ int build_multi_step_wide(msbwt_index *idx, Replica &rep, const Options &opt, bo
     g_launches += (uint64_t)n;
     codes10_owner.reset();
     if (rc != MSBWT_OK) {
-        if (rc == MSBWT_ENOMEM && fin_req != 1) { cudaGetLastError(); return MSBWT_OK; }
+        if (rc == MSBWT_ENOMEM && opt.fin != 1) { cudaGetLastError(); return MSBWT_OK; }
         return fail(rc, why);
     }
-    n = 0;
-    rc = build_fin_lines_on_device(rep.device, N, codes20, fshift, flb, rep.fin, why, &n);  // owns codes20
-    g_launches += (uint64_t)n;
-    if (rc != MSBWT_OK) {
-        free_fin_image(rep.fin);
-        rep.fin = FinImage{};
-        if (rc == MSBWT_ENOMEM && fin_req != 1) { cudaGetLastError(); return MSBWT_OK; }
-        return fail(rc, why);
-    }
-    rep.view.fin = rep.fin.lines;
-    rep.view.fin_shift = (uint32_t)rep.fin.shift;
-    rep.view.fin_lb = (uint32_t)rep.fin.lb;
-    if (idx->reps[0].get() == &rep) idx->bytes_per_replica += rep.fin.nlines * (uint64_t)kFinLineBytes;
-    build_trace("multi-step images done");
-    return MSBWT_OK;
+    return build_fin(rep, opt, codes20, flb);
 }
 
 // Automatic choice for an index with 64-bit positions: it lives in HBM, the caller pinned no other layout, and the
@@ -516,7 +507,7 @@ bool pick_wide_oct(int device, uint64_t index_bytes, uint64_t total, const Optio
     return oct_image_bytes(total, kOctMaxShift) + fin_image_bytes(total, 16, 12) + 12 * total + (8ull << 30) <= free_b;
 }
 
-int build_suffix_table(msbwt_index *idx, Replica &rep, int s) {
+int build_suffix_table(Replica &rep, int s) {
     if (s <= 0) return MSBWT_OK;
     DeviceGuard guard(rep.device);
     const bool wide = index_is_wide(rep.view);
@@ -556,24 +547,14 @@ int build_suffix_table(msbwt_index *idx, Replica &rep, int s) {
     }
     cleanup(false);
     rep.d_table = level[(size_t)s];
-    rep.view.table = rep.d_table;
-    const void **lower[3] = {&rep.view.table2, &rep.view.table3, &rep.view.table4};
-    uint64_t bytes = (1ull << (2 * s)) * eb;
-    for (int b = 1; b <= 3; b++) {
-        const int j = s - b;
-        if (j < lowest_kept) break;
-        rep.d_table_lower[b - 1] = level[(size_t)j];
-        *lower[b - 1] = level[(size_t)j];
-        bytes += (1ull << (2 * j)) * eb;
-    }
-    rep.view.table_s = (uint32_t)s;
-    if (idx->reps[0].get() == &rep) idx->table_s = (uint32_t)s;
-    if (idx->reps[0].get() == &rep) idx->bytes_per_replica += bytes;
+    for (int b = 1; b <= 3 && s - b >= lowest_kept; b++) rep.d_table_lower[b - 1] = level[(size_t)(s - b)];
+    rep.table_s = (uint32_t)s;
+    refresh_view(rep);
     return MSBWT_OK;
 }
 
-msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices, int ndev, const Options &opt,
-                           int *err) {
+msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices, int ndev, Options opt, int *err) {
+    fill_from_env(opt);
     const uint32_t sb_shift = opt.sb_shift;
     const int table_s = opt.table_s;
     g_last_error.clear();
@@ -595,7 +576,7 @@ msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices,
         bool explicit_s = false;
         const int s0 = pick_table_s(idx->total, table_s, &explicit_s);
         const bool wide = index_is_wide(idx->reps[0]->view);
-        const uint64_t one_step_bytes = idx->bytes_per_replica + (s0 > 0 ? (1ull << (2 * s0)) * (wide ? 16 : 8) : 0);
+        const uint64_t one_step_bytes = replica_bytes(*idx->reps[0]) + (s0 > 0 ? (1ull << (2 * s0)) * (wide ? 16 : 8) : 0);
         rc = for_each_replica_slot(idx->reps.size(), [&](size_t slot) -> int {
             auto &rep = idx->reps[slot];
             int s = s0;
@@ -604,7 +585,7 @@ msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices,
             {
                 DeviceGuard guard(rep->device);
                 if (wide && pick_wide_oct(rep->device, one_step_bytes, idx->total, opt)) {
-                    if (int r = build_multi_step_wide(idx.get(), *rep, opt, opt.oct == 1, &wide_oct); r != MSBWT_OK) return r;
+                    if (int r = build_multi_step_wide(*rep, opt, opt.oct == 1, &wide_oct); r != MSBWT_OK) return r;
                 }
                 const char *oct_env = getenv("MSBWT_OCT_INDEX");
                 const bool with_oct = idx->total < (1ull << 32) && !index_is_wide(rep->view) && opt.oct != 0 &&
@@ -627,7 +608,7 @@ msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices,
                     if (rep->view.oct) s = std::min(s, kOctAutoTableS);
                 }
             }
-            if (int r = build_suffix_table(idx.get(), *rep, s); r != MSBWT_OK) return r;
+            if (int r = build_suffix_table(*rep, s); r != MSBWT_OK) return r;
             rep->lanes = pick_lanes(rep->device, one_step_bytes, opt.lanes);
             return MSBWT_OK;
         });
@@ -736,8 +717,8 @@ extern "C" int msbwt_device_count(const msbwt_index *idx) { return idx ? (int)id
 extern "C" int msbwt_device_ordinal(const msbwt_index *idx, int slot) {
     return (idx && slot >= 0 && slot < (int)idx->reps.size()) ? idx->reps[slot]->device : -1;
 }
-extern "C" uint64_t msbwt_index_bytes(const msbwt_index *idx) { return idx ? idx->bytes_per_replica : 0; }
-extern "C" int msbwt_suffix_table_s(const msbwt_index *idx) { return idx ? (int)idx->table_s : 0; }
+extern "C" uint64_t msbwt_index_bytes(const msbwt_index *idx) { return (idx && !idx->reps.empty()) ? replica_bytes(*idx->reps[0]) : 0; }
+extern "C" int msbwt_suffix_table_s(const msbwt_index *idx) { return (idx && !idx->reps.empty()) ? (int)idx->reps[0]->view.table_s : 0; }
 extern "C" int msbwt_kernel_lanes(const msbwt_index *idx) { return (idx && !idx->reps.empty()) ? idx->reps[0]->lanes : 0; }
 extern "C" int msbwt_pair_index(const msbwt_index *idx) { return (idx && !idx->reps.empty() && idx->reps[0]->view.pair) ? 1 : 0; }
 extern "C" int msbwt_quad_index(const msbwt_index *idx) { return (idx && !idx->reps.empty() && idx->reps[0]->view.quad) ? 1 : 0; }
@@ -746,8 +727,8 @@ extern "C" uint64_t msbwt_oct_overflow_lines(const msbwt_index *idx) { return (i
 extern "C" uint64_t msbwt_oct_overflow_occurrences(const msbwt_index *idx) { return (idx && !idx->reps.empty()) ? idx->reps[0]->oct.overflow_occurrences : 0; }
 extern "C" uint64_t msbwt_oct_runs(const msbwt_index *idx) { return (idx && !idx->reps.empty()) ? idx->reps[0]->oct.runs : 0; }
 extern "C" int msbwt_oct_symbols(void) { return kOctSyms; }
-// EXPERIMENTAL final-step image (layout.h): 0 / EINVAL unless the library was compiled with -DMSBWT_FINAL_STEP and
-// the index was created with MSBWT_FINAL_INDEX=1
+// final-step image (layout.h): built by default on top of the oct image; final_index = 0 (or MSBWT_FINAL_INDEX=0) turns
+// it off
 extern "C" int msbwt_final_index(const msbwt_index *idx) {
     return (idx && !idx->reps.empty() && idx->reps[0]->view.fin) ? 1 : 0;
 }
@@ -1065,28 +1046,51 @@ extern "C" int msbwt_constrain_ranges_fanout_device(const msbwt_index *idx, int 
 // ================================================================ construction of the BWT itself
 
 namespace {
+int check_device(int device) {
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(MSBWT_ENODEV, "no usable CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= count) return fail(MSBWT_ENODEV, "device ordinal out of range");
+    return MSBWT_OK;
+}
+
+// `len` RLE bytes on the current device -> *rle, a malloc'd host copy (the caller frees it with msbwt_buffer_free)
+int rle_to_host(const uint8_t *d_rle, uint64_t len, uint8_t **rle) {
+    uint8_t *host = (uint8_t *)malloc(len ? len : 1);
+    if (!host) return fail(MSBWT_ENOMEM, "host buffer for the RLE bytes");
+    if (len) {
+        if (cudaError_t e = cudaMemcpy(host, d_rle, len, cudaMemcpyDeviceToHost); e != cudaSuccess) {
+            free(host);
+            return fail(MSBWT_ECUDA, std::string("copying the RLE bytes: ") + cudaGetErrorString(e));
+        }
+    }
+    *rle = host;
+    return MSBWT_OK;
+}
+
 // reads (and, for reads of different lengths, their n_reads + 1 offsets) on the host or already on `device` ->
 // RLE bytes of their multi-string BWT in a malloc'd host buffer
 int build_rle_bwt_common(const uint8_t *reads, const uint64_t *offsets, uint64_t n_reads, uint32_t read_len, uint64_t n_syms,
                          int on_device, int device, uint8_t **rle, uint64_t *rle_len, uint64_t *total) {
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(MSBWT_ENODEV, "no usable CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= count) return fail(MSBWT_ENODEV, "device ordinal out of range");
+    if (int rc = check_device(device); rc != MSBWT_OK) return rc;
     DeviceGuard guard(device);
-    struct DevPtr { void *p = nullptr; ~DevPtr() { if (p) cudaFree(p); } };
-    DevPtr reads_copy, offsets_copy, d_rle_owner;
+    DevicePtr<uint8_t> reads_copy;
+    DevicePtr<uint64_t> offsets_copy;
     const uint8_t *d_reads = reads;
     const uint64_t *d_offsets = offsets;
     if (!on_device && n_reads) {
         if (n_syms) {
-            CU_TRY(cudaMalloc(&reads_copy.p, n_syms));
-            CU_TRY(cudaMemcpy(reads_copy.p, reads, n_syms, cudaMemcpyHostToDevice));
+            uint8_t *p = nullptr;
+            CU_TRY(cudaMalloc(&p, n_syms));
+            reads_copy.reset(p);
+            CU_TRY(cudaMemcpy(p, reads, n_syms, cudaMemcpyHostToDevice));
         }
-        d_reads = (const uint8_t *)reads_copy.p;
+        d_reads = reads_copy.get();
         if (offsets) {
-            CU_TRY(cudaMalloc(&offsets_copy.p, (n_reads + 1) * sizeof(uint64_t)));
-            CU_TRY(cudaMemcpy(offsets_copy.p, offsets, (n_reads + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice));
-            d_offsets = (const uint64_t *)offsets_copy.p;
+            uint64_t *p = nullptr;
+            CU_TRY(cudaMalloc(&p, (n_reads + 1) * sizeof(uint64_t)));
+            offsets_copy.reset(p);
+            CU_TRY(cudaMemcpy(p, offsets, (n_reads + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice));
+            d_offsets = p;
         }
     }
     uint8_t *d_rle = nullptr;
@@ -1094,18 +1098,9 @@ int build_rle_bwt_common(const uint8_t *reads, const uint64_t *offsets, uint64_t
     int n = 0;
     int rc = build_rle_bwt_on_device(d_reads, d_offsets, n_reads, read_len, &d_rle, rle_len, total, why, &n);
     g_launches += (uint64_t)n;
-    d_rle_owner.p = d_rle;
+    DevicePtr<uint8_t> d_rle_owner(d_rle);
     if (rc != MSBWT_OK) return fail(rc, why);
-    uint8_t *host = (uint8_t *)malloc(*rle_len ? *rle_len : 1);
-    if (!host) return fail(MSBWT_ENOMEM, "host buffer for the RLE bytes");
-    if (*rle_len) {
-        if (cudaError_t e = cudaMemcpy(host, d_rle, *rle_len, cudaMemcpyDeviceToHost); e != cudaSuccess) {
-            free(host);
-            return fail(MSBWT_ECUDA, std::string("copying the RLE bytes: ") + cudaGetErrorString(e));
-        }
-    }
-    *rle = host;
-    return MSBWT_OK;
+    return rle_to_host(d_rle, *rle_len, rle);
 }
 }  // namespace
 
@@ -1155,9 +1150,7 @@ extern "C" int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const 
     *total = 0;
     if (iterations) *iterations = 0;
     if ((len_a && !rle_a) || (len_b && !rle_b)) return fail(MSBWT_EINVAL, "NULL input with a length above 0");
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) return fail(MSBWT_ENODEV, "no usable CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= count) return fail(MSBWT_ENODEV, "device ordinal out of range");
+    if (int rc = check_device(device); rc != MSBWT_OK) return rc;
     DeviceGuard guard(device);
     uint8_t *d_rle = nullptr;
     uint64_t len = 0, n = 0;
@@ -1166,17 +1159,9 @@ extern "C" int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const 
     int launches = 0;
     int rc = merge_rle_bwts_on_device(rle_a, len_a, rle_b, len_b, &d_rle, &len, &n, &passes, why, &launches);
     g_launches += (uint64_t)launches;
-    struct DevPtr { void *p; ~DevPtr() { if (p) cudaFree(p); } } d_rle_owner{d_rle};
+    DevicePtr<uint8_t> d_rle_owner(d_rle);
     if (rc != MSBWT_OK) return fail(rc, why);
-    uint8_t *host = (uint8_t *)malloc(len ? len : 1);
-    if (!host) return fail(MSBWT_ENOMEM, "host buffer for the RLE bytes");
-    if (len) {
-        if (cudaError_t e = cudaMemcpy(host, d_rle, len, cudaMemcpyDeviceToHost); e != cudaSuccess) {
-            free(host);
-            return fail(MSBWT_ECUDA, std::string("copying the RLE bytes: ") + cudaGetErrorString(e));
-        }
-    }
-    *rle = host;
+    if (int r = rle_to_host(d_rle, len, rle); r != MSBWT_OK) return r;
     *rle_len = len;
     *total = n;
     if (iterations) *iterations = passes;

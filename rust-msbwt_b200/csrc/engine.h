@@ -5,12 +5,19 @@
 
 #include <algorithm>
 #include <cstdint>
+#include <memory>
 #include <string>
 #include <vector>
 
 #include "layout.h"
 
 namespace msbwt {
+
+// one cudaMalloc'd buffer, freed when it goes out of scope unless release()d
+struct CudaFree {
+    void operator()(void *p) const { cudaFree(p); }
+};
+template <class T> using DevicePtr = std::unique_ptr<T, CudaFree>;
 
 // cudaMalloc'd scratch buffers of one build step: whatever is still listed is freed when it goes out of scope
 struct DeviceScratch {

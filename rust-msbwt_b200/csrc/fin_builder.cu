@@ -1,6 +1,6 @@
 // fin_builder.cu -- device-side construction of the FINAL-STEP image (layout.h; specification and CPU checker in
-// oracle/final_step.py, DESIGN.md section 7 item 4).  EXPERIMENTAL: compiled only with -DMSBWT_FINAL_STEP, written
-// after round 1's GPU budget was spent and not yet run on a GPU.
+// oracle/final_step.py, DESIGN.md section 7 item 4).  Built by default on top of the oct image; final_index = 0 (or
+// MSBWT_FINAL_INDEX=0) turns it off.
 //
 // The last kFinSyms (20) symbols a BWT::count_kmer (src/msbwt_core.rs:125-161) consumes need no rank, only the number
 // of positions of [l, h) whose 20-symbol code matches, so the image holds no checkpoints and nothing for absent codes:
@@ -243,14 +243,14 @@ int build_fin_codes_by_walk(int device, const IndexView &ix, const uint32_t *d_c
 // Stage 2 (needs nothing but the codes, which it OWNS and frees as soon as the run records exist): the lines
 int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20_in, int shift, int lb, FinImage &img,
                               std::string &why, int *launches) {
-    struct Owned { uint64_t *p; ~Owned() { if (p) cudaFree(p); } } codes20{d_codes20_in};
+    DevicePtr<uint64_t> codes20(d_codes20_in);
     if (!d_codes20_in) { why = "final-step image: no position codes"; return MSBWT_EINVAL; }
     if (shift < 8 || shift > 16 || lb < kFinCodeBits - kFinTagBits || lb > 20) { why = "final-step image: bucket shift 8..16, lines per bucket 2^12..2^20"; return MSBWT_EINVAL; }
     if (((((total >> shift) + 1) << lb) >> (64 - kFinTagBits)) != 0) { why = "final-step image: line index and tag do not fit one 64-bit sort key"; return MSBWT_EINVAL; }
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((total + 255) / 256, (uint64_t)sms * 32));
-    const uint64_t *d_codes20 = codes20.p;
+    const uint64_t *d_codes20 = codes20.get();
 
     Scratch tmp;
     unsigned long long *d_stat = nullptr;  // [0] records, [1] emit cursor, [2] overflowed lines
@@ -278,8 +278,7 @@ int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20_in
         F_TRY(cudaDeviceSynchronize());
         if (launches) (*launches)++;
     }
-    cudaFree(codes20.p);  // the records carry everything from here on
-    codes20.p = nullptr;
+    codes20.reset();  // the records carry everything from here on
     F_TRY(cudaMalloc((void **)&img.lines, nlines * kFinLineBytes));
     F_TRY(cudaMemsetAsync(img.lines, 0, nlines * kFinLineBytes));
     if (n_runs) {
@@ -311,7 +310,7 @@ int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20_in
 
 void free_fin_image(FinImage &img) {
     if (img.lines) cudaFree(img.lines);
-    img.lines = nullptr;
+    img = {};
 }
 
 }  // namespace msbwt

@@ -86,14 +86,16 @@ struct Replica {
     int device = -1;
     uint4 *d_blocks = nullptr;
     uint32_t *d_aux = nullptr;
-    void *d_table = nullptr;
+    void *d_table = nullptr;   // suffix table of depth table_s (0 = none)
     void *d_table_lower[3] = {nullptr, nullptr, nullptr};  // depths table_s - 1 .. table_s - 3, kept so that a
                                                            // multi-step image always finds a depth that leaves a multiple
                                                            // of its stride (pair: one level, quad: three)
+    uint32_t table_s = 0;
     PairImage pair;            // 128-byte pair lines (layout.h), when the index lives in HBM
     QuadImage quad;            // 32-byte quad sectors (layout.h), when the index lives in HBM and the image fits
     OctImage oct;              // 128-byte oct lines (layout.h), next to the quad image when positions are 32-bit
-    FinImage fin;              // EXPERIMENTAL final-step lines (layout.h), only with MSBWT_FINAL_INDEX=1
+    FinImage fin;              // final-step lines (layout.h), built by default on top of the oct image; final_index = 0
+                               // (or MSBWT_FINAL_INDEX=0) turns them off
     int lanes = 1;           // kernel mapping: 1 = thread per query, 2 = lane pair per query (kernels.cu)
     uint64_t *d_cbase = nullptr;
     IndexView view{};
@@ -156,7 +158,5 @@ struct msbwt_index {
     uint64_t total = 0;
     uint64_t counts[msbwt::kAlphabet] = {0, 0, 0, 0, 0, 0};
     uint64_t start[msbwt::kAlphabet] = {0, 0, 0, 0, 0, 0};
-    uint64_t bytes_per_replica = 0;
-    uint32_t table_s = 0;
     std::vector<std::unique_ptr<msbwt::Replica>> reps;
 };

@@ -186,7 +186,7 @@ uint64_t oct_image_bytes(uint64_t total, int shift) {
 // soon as the codes exist; `d_codes2` (the pair builder's keep_codes) is borrowed.
 int build_oct_codes_on_device(int device, const IndexView &ix, uint16_t *d_codes4, const uint8_t *d_codes2,
                               uint32_t **d_codes10, std::string &why, int *launches) {
-    struct Owned { uint16_t *p; ~Owned() { if (p) cudaFree(p); } } codes4{d_codes4};
+    DevicePtr<uint16_t> codes4(d_codes4);
     *d_codes10 = nullptr;
     if (!ix.quad || !d_codes4 || !d_codes2) { why = "oct image: needs the quad image, its codes and the pair codes"; return MSBWT_EINVAL; }
     if (index_is_wide(ix)) { why = "oct image: only for indexes with 32-bit positions (N < 2^32, one superblock)"; return MSBWT_EINVAL; }
@@ -312,7 +312,7 @@ int build_oct_lines_on_device(int device, const IndexView &ix, const uint32_t *d
 
 void free_oct_image(OctImage &img) {
     if (img.lines) cudaFree(img.lines);
-    img.lines = nullptr;
+    img = {};
 }
 
 }  // namespace msbwt

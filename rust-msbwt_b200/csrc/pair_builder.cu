@@ -211,8 +211,7 @@ int build_pair_image_on_device(int device, const IndexView &ix, const uint64_t s
 void free_pair_image(PairImage &img) {
     if (img.lines) cudaFree(img.lines);
     if (img.c2base) cudaFree(img.c2base);
-    img.lines = nullptr;
-    img.c2base = nullptr;
+    img = {};
 }
 
 }  // namespace msbwt

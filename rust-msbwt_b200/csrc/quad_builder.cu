@@ -239,8 +239,7 @@ int build_quad_image_on_device(int device, const IndexView &ix, const uint8_t *d
 void free_quad_image(QuadImage &img) {
     if (img.sectors) cudaFree(img.sectors);
     if (img.c4base) cudaFree(img.c4base);
-    img.sectors = nullptr;
-    img.c4base = nullptr;
+    img = {};
 }
 
 }  // namespace msbwt
