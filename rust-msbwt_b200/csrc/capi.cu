@@ -68,28 +68,6 @@ int for_each_replica_slot(size_t n, F &&body) {
     return MSBWT_OK;
 }
 
-int finish_replica(msbwt_index *idx, size_t slot, std::unique_ptr<Replica> rep, uint64_t total, uint64_t nblocks, uint32_t n_super,
-                   uint32_t sb_shift) {
-    CU_TRY(cudaMalloc((void **)&rep->d_status, kStatusWords * sizeof(uint32_t)));
-    CU_TRY(cudaMemset(rep->d_status, 0, kStatusWords * sizeof(uint32_t)));
-    CU_TRY(cudaHostAlloc((void **)&rep->h_status, kStatusWords * sizeof(uint32_t), cudaHostAllocDefault));
-    memset(rep->h_status, 0, kStatusWords * sizeof(uint32_t));
-    for (auto &ln : rep->lane) {
-        CU_TRY(cudaStreamCreateWithFlags(&ln.stream, cudaStreamNonBlocking));
-        CU_TRY(cudaEventCreateWithFlags(&ln.h2d_done, cudaEventDisableTiming));
-        CU_TRY(cudaEventCreateWithFlags(&ln.d2h_done, cudaEventDisableTiming));
-    }
-    rep->view.blocks = rep->d_blocks;
-    rep->view.cbase = rep->d_cbase;
-    rep->view.aux = rep->d_aux;
-    rep->view.total = total;
-    rep->view.nblocks = nblocks;
-    rep->view.n_super = n_super;
-    rep->view.sb_shift = sb_shift;
-    idx->reps[slot] = std::move(rep);
-    return MSBWT_OK;
-}
-
 // The optional-image fields of the view, from what the replica owns: an image that was never built or has been freed
 // reads as null / 0.  Called after every build stage that adds or frees an image.
 void refresh_view(Replica &rep) {
@@ -132,7 +110,7 @@ uint64_t replica_bytes(const Replica &rep) {
     return b;
 }
 
-// Default load path: the block image is built on each device from the RLE bytes (builder.cu).
+// The block image is built on each device from the RLE bytes (builder.cu).
 int build_replicas_on_device(msbwt_index *idx, const uint8_t *rle, uint64_t len, uint32_t sb_shift, const int *devices,
                              int ndev) {
     std::vector<int> devs;
@@ -153,37 +131,27 @@ int build_replicas_on_device(msbwt_index *idx, const uint8_t *rle, uint64_t len,
             idx->total = img.total;
             for (int s = 0; s < kAlphabet; s++) { idx->counts[s] = img.counts[s]; idx->start[s] = img.start[s]; }
         }
-        return finish_replica(idx, i, std::move(rep), img.total, img.nblocks, img.n_super, img.sb_shift);
+        CU_TRY(cudaMalloc((void **)&rep->d_status, kStatusWords * sizeof(uint32_t)));
+        CU_TRY(cudaMemset(rep->d_status, 0, kStatusWords * sizeof(uint32_t)));
+        CU_TRY(cudaHostAlloc((void **)&rep->h_status, kStatusWords * sizeof(uint32_t), cudaHostAllocDefault));
+        memset(rep->h_status, 0, kStatusWords * sizeof(uint32_t));
+        for (auto &ln : rep->lane) {
+            CU_TRY(cudaStreamCreateWithFlags(&ln.stream, cudaStreamNonBlocking));
+            CU_TRY(cudaEventCreateWithFlags(&ln.h2d_done, cudaEventDisableTiming));
+            CU_TRY(cudaEventCreateWithFlags(&ln.d2h_done, cudaEventDisableTiming));
+        }
+        rep->view.blocks = rep->d_blocks;
+        rep->view.cbase = rep->d_cbase;
+        rep->view.aux = rep->d_aux;
+        rep->view.total = img.total;
+        rep->view.nblocks = img.nblocks;
+        rep->view.n_super = img.n_super;
+        rep->view.sb_shift = img.sb_shift;
+        idx->reps[i] = std::move(rep);
+        return MSBWT_OK;
     });
     if (rc != MSBWT_OK) idx->reps.clear();
     return rc;
-}
-
-// MSBWT_HOST_BUILD=1: build the image with the serial host builder (loader.cu) and copy it up.
-int upload(msbwt_index *idx, const HostImage &img, const int *devices, int ndev) {
-    std::vector<int> devs;
-    if (int rc = resolve_devices(devices, ndev, devs); rc != MSBWT_OK) return rc;
-    idx->total = img.total;
-    for (int s = 0; s < kAlphabet; s++) { idx->counts[s] = img.counts[s]; idx->start[s] = img.start[s]; }
-    const size_t block_bytes = img.blocks.size() * sizeof(uint32_t);
-    const size_t cbase_bytes = img.cbase.size() * sizeof(uint64_t);
-    const size_t aux_bytes = img.aux.size() * sizeof(uint32_t);
-    idx->reps.resize(devs.size());
-    for (size_t slot = 0; slot < devs.size(); slot++) {
-        const int d = devs[slot];
-        DeviceGuard guard(d);
-        auto rep = std::make_unique<Replica>();
-        rep->device = d;
-        CU_TRY(cudaMalloc((void **)&rep->d_blocks, block_bytes));
-        CU_TRY(cudaMalloc((void **)&rep->d_cbase, cbase_bytes));
-        CU_TRY(cudaMalloc((void **)&rep->d_aux, aux_bytes));
-        CU_TRY(cudaMemcpy(rep->d_aux, img.aux.data(), aux_bytes, cudaMemcpyHostToDevice));
-        CU_TRY(cudaMemcpy(rep->d_blocks, img.blocks.data(), block_bytes, cudaMemcpyHostToDevice));
-        CU_TRY(cudaMemcpy(rep->d_cbase, img.cbase.data(), cbase_bytes, cudaMemcpyHostToDevice));
-        int rc = finish_replica(idx, slot, std::move(rep), img.total, img.nblocks, img.n_super, img.sb_shift);
-        if (rc != MSBWT_OK) { idx->reps.clear(); return rc; }
-    }
-    return MSBWT_OK;
 }
 
 // Suffix table (layout.h): level j+1 from level j with one constrain_range per entry, on the
@@ -561,14 +529,8 @@ msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices,
     int rc;
     std::string why;
     auto idx = std::make_unique<msbwt_index>();
-    const char *host_build = getenv("MSBWT_HOST_BUILD");
     if ((rc = validate_rle(rle, len, why)) != MSBWT_OK) {
         fail(rc, why);
-    } else if (host_build && atoi(host_build) == 1) {
-        HostImage img;
-        rc = build_image_from_rle(rle, len, sb_shift, img, why);
-        if (rc == MSBWT_OK) rc = upload(idx.get(), img, devices, ndev);
-        else fail(rc, why);
     } else {
         rc = build_replicas_on_device(idx.get(), rle, len, sb_shift, devices, ndev);
     }
@@ -775,17 +737,6 @@ extern "C" void msbwt_host_free(void *p) { if (p) cudaFreeHost(p); }
 
 // ================================================================ device-buffer entry points
 
-namespace {
-// MSBWT_FUSED=1 routes the fixed-k device entry point through the fused kernel (fused_kernels.cu).  Off by
-// default: measured on B200 it is slower than pack / seed + search (9.5 ms against 7.4 ms per 100 M 31-mers on
-// the 1.51 Gsymbol BWT) -- the search loop is already 62 % issue-bound and the fused one adds the packing and a
-// third iteration (the table entry) per query to it.
-bool fused_enabled() {
-    const char *e = getenv("MSBWT_FUSED");
-    return e && atoi(e) != 0;
-}
-}  // namespace
-
 extern "C" int msbwt_count_kmers_fixed_device(const msbwt_index *idx, int slot, const uint8_t *d_syms, uint32_t k,
                                               uint64_t n, uint64_t *d_out, uint32_t *d_status, void *stream) {
     if (!idx || slot < 0 || slot >= (int)idx->reps.size()) return fail(MSBWT_EINVAL, "bad handle or slot");
@@ -803,18 +754,6 @@ extern "C" int msbwt_count_kmers_fixed_device(const msbwt_index *idx, int slot, 
     if (!rep.dev_packed_free) CU_TRY(cudaEventCreateWithFlags(&rep.dev_packed_free, cudaEventDisableTiming));
     else CU_TRY(cudaStreamWaitEvent(st, rep.dev_packed_free, 0));
     CU_TRY(cudaMemsetAsync(flag, 0, sizeof(uint32_t), st));
-    if (fused_enabled() && fused_path_applies(rep.view, d_syms, k)) {
-        // one kernel from symbol bytes to counts (fused_kernels.cu); sub-batches of 2^30 keep the 16-byte alignment
-        CU_TRY(rep.dev_packed.reserve(fused_scratch_bytes(per)));
-        for (uint64_t q0 = 0; q0 < n; q0 += per) {
-            const uint64_t m = std::min(per, n - q0);
-            CU_TRY(launch_count_fused(rep.device, rep.view, d_syms + q0 * k, k, m, d_out + q0, flag,
-                                      rep.dev_packed.as<uint32_t>(), st, &g_call_launches));
-            flush_launches();
-        }
-        CU_TRY(cudaEventRecord(rep.dev_packed_free, st));
-        return MSBWT_OK;
-    }
     CU_TRY(rep.dev_packed.reserve(packed_layout(rep.view, k, per).total() * sizeof(uint64_t)));
     for (uint64_t q0 = 0; q0 < n; q0 += per) {  // sub-batches reuse the scratch in stream order
         const uint64_t m = std::min(per, n - q0);

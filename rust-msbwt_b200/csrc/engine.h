@@ -243,11 +243,6 @@ cudaError_t launch_count_oct_wide(int device, const IndexView &ix, const uint64_
 // stats_kernels.cu: live list A over the oct image with the counting instantiation -- d_stats[8] (oct_kernel.cuh)
 cudaError_t launch_count_oct_stats(int device, const IndexView &ix, const uint64_t *d_packed, uint32_t k, uint64_t n,
                                    uint64_t *d_out, unsigned long long *d_stats, cudaStream_t st);
-// the fused path (oct image, k <= 32, 16-byte aligned symbol bytes): one kernel from symbol bytes to counts
-bool fused_path_applies(const IndexView &ix, const uint8_t *d_syms, uint32_t k);
-uint64_t fused_scratch_bytes(uint64_t n);
-cudaError_t launch_count_fused(int device, const IndexView &ix, const uint8_t *d_syms, uint32_t k, uint64_t n,
-                               uint64_t *d_out, uint32_t *d_status, uint32_t *d_scratch, cudaStream_t st, int *launches);
 bool packed_batch_needs_list_b(const IndexView &ix, uint32_t k);
 uint32_t max_host_packed_k();  // seed_packed_kernel handles k-mers of at most this many symbols
 cudaError_t launch_count_bytes(int device, const IndexView &ix, const uint8_t *d_syms,

@@ -10,18 +10,17 @@
 // simply streams through consecutive batches of 32 queries as a software pipeline, nothing diverges, nothing is
 // compacted, and the counts are written back coalesced:
 //
-//   iteration i of a warp (its batches are i = 0, 1, ..; group G_i = the cp.async group committed in iteration i):
-//     C  batch i+1 : range [l, h) from the table entry requested one iteration ago; 40-bit code -> fin_mix40 -> line
-//                    index + tag; the WARP copies the 32 lines into row buffer (i+1) & 1 (8 lanes x 16 bytes per
-//                    line: one 128-byte request per line)
-//     A  batch i+3 : the batch's 32 k symbol bytes -> byte buffer (i+3) & 1 (coalesced 16-byte cp.async)     } G_i
-//     -- cp.async.wait_group 1: G_{i-1} has landed = the lines of batch i and the bytes of batch i+2
-//     B  batch i+2 : every lane packs its k-mer from the byte buffer (SWAR, four symbols per step), and requests
-//                    its table entry (ld.global.nc: an L2 hit, consumed by C in the next iteration -- D below is
-//                    what hides its latency)
+//   iteration i of a warp (its batches are i = 0, 1, ..):
+//     -- cp.async.wait_all: what iteration i-1 issued has landed = the lines of batch i and the bytes of batch i+2
 //     D  batch i   : every lane scans its own line (groups `tag | nruns` + runs, layout.h), writes its count to
 //                    out[32 * batch + lane] (one coalesced 256-byte store per warp), or queues the query for the
 //                    general kernel: overflowed line, range over two buckets
+//     B  batch i+2 : every lane packs its k-mer from the byte buffer (SWAR, four symbols per step), and requests
+//                    its table entry (ld.global.nc: an L2 hit, consumed by C in the next iteration)
+//     C  batch i+1 : range [l, h) from the table entry requested one iteration ago; 40-bit code -> fin_mix40 -> line
+//                    index + tag; the WARP copies the 32 lines into the row buffer (8 lanes x 16 bytes per line: one
+//                    128-byte request per line)
+//     A  batch i+3 : the batch's 32 k symbol bytes -> the byte buffer (coalesced 16-byte cp.async)
 //
 // What the pipeline cannot answer goes where pack_seed_kernel would have put it, in the same scratch layout
 // (engine.h PackedLayout), for launch_count_packed to finish: live list A (all-ACGT: the remaining 20 symbols + the
@@ -42,31 +41,26 @@ constexpr int kFinWarps = 8;                 // warps per CTA
 constexpr int kFinThreads = 32 * kFinWarps;
 constexpr int kFinRowBytes = 144;            // a 128-byte line + 16: the rows of consecutive lanes start 4 banks apart
 constexpr int kFinByteBuf = 32 * 32 + 16;    // 32 k-mers of k <= 32 symbol bytes, + the slack an unaligned 4-byte read needs
-// Two shapes of the same pipeline (template parameter DEEP), chosen by measurement (launch_t):
-//   DEEP = true : two row buffers and two byte buffers per warp -- a warp keeps the lines of batch s+1 in flight while
-//                 it scans those of batch s; 12.3 KB of shared memory per warp, 2 CTAs of 8 warps per SM (16 warps)
-//   DEEP = false: one of each -- a warp waits for its own lines, the OTHER warps of the SM hide that: 6.3 KB per warp
-//                 and 64 registers per thread, 4 CTAs per SM (32 warps).  The loop is bound by the latency of its own
-//                 dependent instructions (ncu, profiles/r2g_*: 640 instructions per batch issue in 5600 cycles per
-//                 warp at 4 warps per scheduler), which only more resident warps can hide.
+// One row buffer and one byte buffer per warp: a warp waits for its own lines and the OTHER warps of the SM hide
+// that.  The loop is bound by the latency of its own dependent instructions (ncu, profiles/r2g_*: 640 instructions
+// per batch issue in 5600 cycles per warp at 4 warps per scheduler), which only more resident warps can hide -- so
+// the shape that keeps the most warps resident: 6.3 KB of shared memory per warp and 64 registers per thread, 4 CTAs
+// of 8 warps per SM (32 warps).
 // WIDE (64-bit positions: an index of 2^32 symbols and more, or one cut into several superblocks): 16-byte table
 // entries, two seed words per queued query, 3 CTAs per SM for the registers the wider ranges take.
-template <bool DEEP, bool WIDE = false> struct FinShape {
-    static constexpr int kBufs = DEEP ? 2 : 1;
-    static constexpr int kQueue = DEEP ? 64 : 32;  // list-A entries a warp stages before it flushes
-    static constexpr int kWarpSmem = kBufs * 32 * kFinRowBytes + kBufs * kFinByteBuf + kQueue * (WIDE ? 28 : 20);
+template <bool WIDE = false> struct FinShape {
+    static constexpr int kQueue = 32;  // list-A entries a warp stages before it flushes
+    static constexpr int kWarpSmem = 32 * kFinRowBytes + kFinByteBuf + kQueue * (WIDE ? 28 : 20);
     static constexpr int kSmem = kFinWarps * kWarpSmem;
-    static constexpr int kCtasPerSm = DEEP ? 2 : (WIDE ? 3 : 4);
+    static constexpr int kCtasPerSm = WIDE ? 3 : 4;
 };
-
-
 
 enum : uint32_t { kKindNone = 0, kKindZero = 1, kKindLine = 2, kKindTwoBuckets = 3 };
 
 // SRC 0: symbol bytes; 1: caller-packed integers (first symbol most significant); 2: host-packed words (last symbol
 // in the top bits).  K = 31: every shift, mask and copy count a constant; K = 0: k_rt (k <= 32).
-template <int SRC, uint32_t K, bool DEEP, bool WIDE = false>
-__global__ void __launch_bounds__(kFinThreads, FinShape<DEEP, WIDE>::kCtasPerSm)
+template <int SRC, uint32_t K, bool WIDE = false>
+__global__ void __launch_bounds__(kFinThreads, FinShape<WIDE>::kCtasPerSm)
 pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_rt, SeedPlan plan, PackedLayout lay,
                        uint64_t *__restrict__ packed, uint64_t *__restrict__ out, uint32_t *__restrict__ status) {
     extern __shared__ __align__(16) uint8_t smem[];
@@ -81,15 +75,14 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
     if (warp_gid >= n_batches) return;
     const uint32_t my_batches = (n_batches - warp_gid + warps_total - 1u) / warps_total;  // batches warp_gid + s * warps_total
 
-    using Shape = FinShape<DEEP, WIDE>;
+    using Shape = FinShape<WIDE>;
     using P = typename Pos<WIDE>::type;                                       // a BWT position
     using E = typename std::conditional<WIDE, ulonglong2, uint2>::type;       // a suffix-table entry {l, h}
-    constexpr uint32_t kBufMask = DEEP ? 1u : 0u;  // buffer of batch s: s & kBufMask
     constexpr int kFinQueue = Shape::kQueue;
     uint8_t *const wsm = smem + warp * Shape::kWarpSmem;
-    uint8_t *const rows = wsm;                                              // kBufs x 32 rows
-    uint8_t *const bytes = wsm + Shape::kBufs * 32 * kFinRowBytes;          // kBufs byte buffers (SRC 0)
-    uint8_t *const queue = bytes + Shape::kBufs * kFinByteBuf;              // kQueue x {u64 word, u64 seed, u32 index}
+    uint8_t *const rows = wsm;                                              // 32 rows
+    uint8_t *const bytes = wsm + 32 * kFinRowBytes;                         // the byte buffer (SRC 0)
+    uint8_t *const queue = bytes + kFinByteBuf;                             // kQueue x {u64 word, u64 seed, u32 index}
     uint64_t *const q_word = reinterpret_cast<uint64_t *>(queue);
     uint64_t *const q_seed = q_word + kFinQueue;                             // l | h << 32; WIDE: l, and h in q_seed_hi
     [[maybe_unused]] uint64_t *const q_seed_hi = q_seed + kFinQueue;
@@ -107,13 +100,13 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
 
     auto first_query = [&](uint32_t s) { return (warp_gid + s * warps_total) * 32u; };
 
-    // ---- A: symbol bytes of batch sequence number s -> byte buffer s & 1 (SRC 0), or this lane's word (SRC 1, 2)
+    // ---- A: symbol bytes of batch sequence number s -> the byte buffer (SRC 0), or this lane's word (SRC 1, 2)
     auto stage_a = [&](uint32_t s, uint64_t &word_reg) {
         if (s >= my_batches) return;
         const uint32_t q0 = first_query(s);
         if constexpr (SRC == 0) {
             const uint8_t *g = reinterpret_cast<const uint8_t *>(src_v) + (size_t)q0 * k;  // 16-byte aligned: 32 k bytes per batch
-            uint8_t *dst = bytes + (s & kBufMask) * kFinByteBuf;
+            uint8_t *dst = bytes;
             if (q0 + 32u <= n) {  // a whole batch: 2 k pieces of 16 bytes, every one of them full
                 cp_async16_hint(dst + 16u * lane, g + 16u * lane, true, stream_pol);
                 if (lane + 32u < 2u * k) cp_async16_hint(dst + 16u * (lane + 32u), g + 16u * (lane + 32u), true, stream_pol);
@@ -143,7 +136,7 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
         const uint32_t q = first_query(s) + lane;
         if (q >= n) return;
         if constexpr (SRC == 0) {
-            const uint8_t *buf = bytes + (s & kBufMask) * kFinByteBuf;
+            const uint8_t *buf = bytes;
             const uint32_t o = lane * k;
             const volatile uint32_t *p = reinterpret_cast<const volatile uint32_t *>(buf + (o & ~3u));
             const uint32_t sh = (o & 3u) * 8u;
@@ -192,7 +185,7 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
         kind = kKindLine;  // refined in stage C, once the entry has arrived
     };
 
-    // ---- C: batch s: the range, the line, and the warp's copy of the 32 lines into row buffer s & 1
+    // ---- C: batch s: the range, the line, and the warp's copy of the 32 lines into the row buffer
     auto stage_c = [&](uint32_t s, uint64_t word, E entry, uint32_t &kind, P &l, P &h, uint32_t &tag) {
         l = entry.x;
         h = entry.y;
@@ -211,13 +204,12 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
         }
         if (s >= my_batches) return;  // (warp-uniform)
         const uint32_t pub = line | (kind == kKindLine ? 0x80000000u : 0u);  // a line index is below 2^31 (checked by the host)
-        uint8_t *const dst_rows = rows + (s & kBufMask) * (32 * kFinRowBytes);
         const uint32_t j = lane & 7u;
 #pragma unroll
         for (uint32_t c = 0; c < 8u; c++) {
             const uint32_t o = 4u * c + (lane >> 3);  // the lane whose line this is
             const uint32_t v = __shfl_sync(kFull, pub, o);
-            cp_async16_hint(dst_rows + o * kFinRowBytes + 16u * j, fin_base + (size_t)(v & 0x7fffffffu) * kFinLineBytes + 16u * j,
+            cp_async16_hint(rows + o * kFinRowBytes + 16u * j, fin_base + (size_t)(v & 0x7fffffffu) * kFinLineBytes + 16u * j,
                             (v >> 31) != 0u, stream_pol);
         }
     };
@@ -264,7 +256,7 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
         // FIRST group of this query's code -- a line holds a few groups, so this is a handful of 4-byte shared-memory
         // reads.  A code with more than 15 runs in the bucket (a 31-mer seen 30 times is ~13 runs of consecutive
         // positions) continues in the groups right behind (layout.h: the groups of one code are adjacent).
-        const uint32_t *roww = reinterpret_cast<const uint32_t *>(rows + (s & kBufMask) * (32 * kFinRowBytes) + lane * kFinRowBytes);
+        const uint32_t *roww = reinterpret_cast<const uint32_t *>(rows + lane * kFinRowBytes);
         uint32_t i1 = 0, matches = 0, used = 0;
         if (kind == kKindLine) {
             const uint2 first = *reinterpret_cast<const uint2 *>(roww);
@@ -322,106 +314,47 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
         }
     };
 
-    if constexpr (!DEEP) {
-        // ---- the shallow pipeline (one row buffer, one byte buffer).  Iteration s: everything issued so far has landed
-        //      (lines of batch s, bytes of batch s+2) -> D(s) -> B(s+2) -> C(s+1) (its table entry was requested an
-        //      iteration ago) -> A(s+3) -> commit.  Register state: batch s in D (d_*), s+1 in C (c_*).
-        uint64_t a_word = 0, b_wordreg = 0, w1 = 0;
-        uint64_t c_word = 0, d_word = 0;
-        E c_entry{};
-        uint32_t c_kind = kKindNone, d_kind = kKindNone, d_tag = 0;
-        P d_l = 0, d_h = 0;
-        auto land = [&]() {
-            asm volatile("cp.async.commit_group;" ::: "memory");
-            asm volatile("cp.async.wait_all;" ::: "memory");
-            __syncwarp();
-        };
-        stage_a(0, b_wordreg);
-        land();
-        E e0;
-        uint32_t k0;
-        stage_b(0, b_wordreg, d_word, e0, k0);                  // B(0)
-        __syncwarp();
-        stage_a(1, w1);
-        land();
-        stage_b(1, w1, c_word, c_entry, c_kind);                // B(1)
-        __syncwarp();
-        stage_c(0, d_word, e0, k0, d_l, d_h, d_tag);            // C(0)
-        d_kind = k0;
-        stage_a(2, b_wordreg);                                  // A(2)
-        for (uint32_t s = 0; s < my_batches; s++) {
-            land();                                             // lines(s), bytes(s+2)
-            stage_d(s, d_word, d_kind, d_l, d_h, d_tag);
-            uint64_t b_word;
-            E b_entry;
-            uint32_t b_kind;
-            stage_b(s + 2, b_wordreg, b_word, b_entry, b_kind); // requests the table entry C(s+2) reads next iteration
-            __syncwarp();                                       // rows were read by D(s), the byte buffer by B(s+2)
-            P n_l, n_h;
-            uint32_t n_tag;
-            stage_c(s + 1, c_word, c_entry, c_kind, n_l, n_h, n_tag);
-            stage_a(s + 3, a_word);
-            b_wordreg = a_word;
-            d_word = c_word; d_kind = c_kind; d_l = n_l; d_h = n_h; d_tag = n_tag;
-            c_word = b_word; c_entry = b_entry; c_kind = b_kind;
-        }
-    } else {
-        // ---- the pipeline.  Register state: batch s in D (d_*), s+1 in C (c_*), s+2 in B; the word of s+3 in flight (SRC 1, 2)
-        uint64_t a_word = 0, b_wordreg = 0;
-        uint64_t c_word = 0, d_word = 0;
-        E c_entry{};
-        uint32_t c_kind = kKindNone, d_kind = kKindNone, d_tag = 0;
-        P d_l = 0, d_h = 0;
-
-        // prologue: bytes of batches 0 and 1 (and 2), B for batch 0 and 1, C for batch 0
-        stage_a(0, b_wordreg);
+    // ---- the pipeline (one row buffer, one byte buffer).  Iteration s: everything issued so far has landed
+    //      (lines of batch s, bytes of batch s+2) -> D(s) -> B(s+2) -> C(s+1) (its table entry was requested an
+    //      iteration ago) -> A(s+3) -> commit.  Register state: batch s in D (d_*), s+1 in C (c_*).
+    uint64_t a_word = 0, b_wordreg = 0, w1 = 0;
+    uint64_t c_word = 0, d_word = 0;
+    E c_entry{};
+    uint32_t c_kind = kKindNone, d_kind = kKindNone, d_tag = 0;
+    P d_l = 0, d_h = 0;
+    auto land = [&]() {
         asm volatile("cp.async.commit_group;" ::: "memory");
-        uint64_t w1 = 0;
-        stage_a(1, w1);
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
+        asm volatile("cp.async.wait_all;" ::: "memory");
         __syncwarp();
-        {   // B(0)
-            uint64_t word;
-            E entry;
-            uint32_t kind;
-            stage_b(0, b_wordreg, word, entry, kind);
-            d_word = word;
-            P l, h;
-            uint32_t tag;
-            stage_c(0, word, entry, kind, l, h, tag);  // C(0): lines of batch 0 -> rows 0
-            d_kind = kind; d_l = l; d_h = h; d_tag = tag;
-        }
-        __syncwarp();        // byte buffer 0 was read by B(0)
-        stage_a(2, a_word);  // bytes(2) -> byte buffer 0
-        asm volatile("cp.async.commit_group;" ::: "memory");   // group: lines(0) + bytes(2)
-        asm volatile("cp.async.wait_group 1;" ::: "memory");   // bytes(1) landed
-        __syncwarp();
-        stage_b(1, w1, c_word, c_entry, c_kind);                // B(1)
-        b_wordreg = a_word;                                     // the word of batch 2 (SRC 1, 2)
-
-        for (uint32_t s = 0; s < my_batches; s++) {
-            // C(s+1): needs the entry requested by B(s+1)
-            P n_l, n_h;
-            uint32_t n_tag;
-            __syncwarp();  // rows (s+1) & 1 were read by D(s-1); byte buffer (s+3) & 1 by B(s+1)
-            stage_c(s + 1, c_word, c_entry, c_kind, n_l, n_h, n_tag);
-            stage_a(s + 3, a_word);
-            asm volatile("cp.async.commit_group;" ::: "memory");   // G_s = lines(s+1) + bytes(s+3)
-            asm volatile("cp.async.wait_group 1;" ::: "memory");   // G_{s-1} (or the prologue's group) landed: lines(s), bytes(s+2)
-            __syncwarp();
-            // B(s+2) BEFORE D(s): the table entry it requests is consumed by C(s+2) at the top of the next iteration, and
-            // D(s)'s line scan in between is what hides that (L2) latency
-            uint64_t b_word;
-            E b_entry;
-            uint32_t b_kind;
-            stage_b(s + 2, b_wordreg, b_word, b_entry, b_kind);
-            b_wordreg = a_word;
-            stage_d(s, d_word, d_kind, d_l, d_h, d_tag);
-            // rotate: s+1 becomes the D batch, s+2 the C batch
-            d_word = c_word; d_kind = c_kind; d_l = n_l; d_h = n_h; d_tag = n_tag;
-            c_word = b_word; c_entry = b_entry; c_kind = b_kind;
-        }
+    };
+    stage_a(0, b_wordreg);
+    land();
+    E e0;
+    uint32_t k0;
+    stage_b(0, b_wordreg, d_word, e0, k0);                  // B(0)
+    __syncwarp();
+    stage_a(1, w1);
+    land();
+    stage_b(1, w1, c_word, c_entry, c_kind);                // B(1)
+    __syncwarp();
+    stage_c(0, d_word, e0, k0, d_l, d_h, d_tag);            // C(0)
+    d_kind = k0;
+    stage_a(2, b_wordreg);                                  // A(2)
+    for (uint32_t s = 0; s < my_batches; s++) {
+        land();                                             // lines(s), bytes(s+2)
+        stage_d(s, d_word, d_kind, d_l, d_h, d_tag);
+        uint64_t b_word;
+        E b_entry;
+        uint32_t b_kind;
+        stage_b(s + 2, b_wordreg, b_word, b_entry, b_kind); // requests the table entry C(s+2) reads next iteration
+        __syncwarp();                                       // rows were read by D(s), the byte buffer by B(s+2)
+        P n_l, n_h;
+        uint32_t n_tag;
+        stage_c(s + 1, c_word, c_entry, c_kind, n_l, n_h, n_tag);
+        stage_a(s + 3, a_word);
+        b_wordreg = a_word;
+        d_word = c_word; d_kind = c_kind; d_l = n_l; d_h = n_h; d_tag = n_tag;
+        c_word = b_word; c_entry = b_entry; c_kind = b_kind;
     }
     asm volatile("cp.async.wait_all;" ::: "memory");
     flush_queue();
@@ -436,12 +369,12 @@ pack_seed_final_kernel(IndexView ix, const void *__restrict__ src_v, uint32_t k_
     }
 }
 
-template <int SRC, uint32_t K, bool DEEP, bool WIDE = false>
+template <int SRC, uint32_t K, bool WIDE = false>
 cudaError_t launch_shape(int device, const IndexView &ix, const void *d_src, uint32_t k, const SeedPlan &plan, const PackedLayout &lay,
                      uint64_t *d_packed, uint64_t *d_out, uint32_t *d_status, cudaStream_t st) {
     static bool prepared[64] = {};
-    constexpr int kFinSmem = FinShape<DEEP, WIDE>::kSmem;
-    const void *fn = (const void *)pack_seed_final_kernel<SRC, K, DEEP, WIDE>;
+    constexpr int kFinSmem = FinShape<WIDE>::kSmem;
+    const void *fn = (const void *)pack_seed_final_kernel<SRC, K, WIDE>;
     if (device < 0 || device >= 64 || !prepared[device]) {
         if (cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, kFinSmem); e != cudaSuccess) return e;
         cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
@@ -452,17 +385,15 @@ cudaError_t launch_shape(int device, const IndexView &ix, const void *d_src, uin
     const uint64_t full = (uint64_t)sm_count(device) * (uint64_t)per_sm;
     const uint64_t need = ((lay.n + 31) / 32 + kFinWarps - 1) / kFinWarps;
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min(need, full));
-    pack_seed_final_kernel<SRC, K, DEEP, WIDE><<<grid, kFinThreads, kFinSmem, st>>>(ix, d_src, k, plan, lay, d_packed, d_out, d_status);
+    pack_seed_final_kernel<SRC, K, WIDE><<<grid, kFinThreads, kFinSmem, st>>>(ix, d_src, k, plan, lay, d_packed, d_out, d_status);
     return cudaGetLastError();
 }
 
 template <int SRC, uint32_t K>
 cudaError_t launch_t(int device, const IndexView &ix, const void *d_src, uint32_t k, const SeedPlan &plan, const PackedLayout &lay,
                      uint64_t *d_packed, uint64_t *d_out, uint32_t *d_status, cudaStream_t st) {
-    if (index_is_wide(ix)) return launch_shape<SRC, 0, false, true>(device, ix, d_src, k, plan, lay, d_packed, d_out, d_status, st);  // 64-bit positions: runtime k, shallow shape
-    const char *env = getenv("MSBWT_FINAL_DEEP");  // =1: the two-buffer shape (A/B measurements)
-    if (env && atoi(env) != 0) return launch_shape<SRC, K, true>(device, ix, d_src, k, plan, lay, d_packed, d_out, d_status, st);
-    return launch_shape<SRC, K, false>(device, ix, d_src, k, plan, lay, d_packed, d_out, d_status, st);
+    if (index_is_wide(ix)) return launch_shape<SRC, 0, true>(device, ix, d_src, k, plan, lay, d_packed, d_out, d_status, st);  // 64-bit positions: runtime k
+    return launch_shape<SRC, K>(device, ix, d_src, k, plan, lay, d_packed, d_out, d_status, st);
 }
 
 }  // namespace

@@ -51,26 +51,13 @@ __host__ __device__ __forceinline__ uint32_t list_a_table_depth(const IndexView 
 }
 
 // ---- four symbols per 32-bit word (SWAR)
-__device__ __forceinline__ uint32_t swar_haszero(uint32_t v) { return (v - 0x01010101u) & ~v & 0x80808080u; }
-// nonzero iff some byte is not one of A,C,G,T = 1,2,3,5
-__device__ __forceinline__ uint32_t swar_non_acgt(uint32_t x) {
-    const uint32_t ge6 = (((x & 0x7F7F7F7Fu) + 0x7A7A7A7Au) | x) & 0x80808080u;
-    return ge6 | swar_haszero(x) | swar_haszero(x ^ 0x04040404u);
-}
-// four ACGT symbol bytes -> 8 bits, byte i at bits 2i (A,C,G,T = 0..3)
-__device__ __forceinline__ uint32_t swar_pack4(uint32_t x) {
-    uint32_t c = (x - 0x01010101u - ((x >> 2) & 0x01010101u)) & 0x03030303u;
-    c = (c | (c >> 6)) & 0x000F000Fu;
-    return (c | (c >> 12)) & 0xFFu;
-}
-
-// The same two jobs in one pass through an 8-entry byte table (PRMT): the four symbol bytes become four selector
-// nibbles, the table answers A,C,G,T = 1,2,3,5 with their 2-bit codes and every other symbol < 8 with 0x80.
-// `acc` collects x | table bytes: the k-mer holds a symbol outside ACGT iff (acc & kSwarBadMask) != 0 at the end
-// (a byte >= 8 shows in x itself, whatever the table then answers).  Returns the four codes packed into the TOP
-// byte (byte i of x at bits 24 + 2i; one multiply: the partial products do not overlap), meaningful only when
-// the word is clean; swar_gather4 collects the top bytes of four such words.  7 instructions per word against
-// 17 for swar_non_acgt + swar_pack4 + the shift into place.
+// Checking four symbol bytes for a symbol outside ACGT and packing them, in one pass through an 8-entry byte table
+// (PRMT): the four symbol bytes become four selector nibbles, the table answers A,C,G,T = 1,2,3,5 with their 2-bit
+// codes and every other symbol < 8 with 0x80.  `acc` collects x | table bytes: the k-mer holds a symbol outside ACGT
+// iff (acc & kSwarBadMask) != 0 at the end (a byte >= 8 shows in x itself, whatever the table then answers).
+// Returns the four codes packed into the TOP byte (byte i of x at bits 24 + 2i; one multiply: the partial products
+// do not overlap), meaningful only when the word is clean; swar_gather4 collects the top bytes of four such words.
+// 7 instructions per word against 17 for a check and a pack in plain SWAR arithmetic and the shift into place.
 constexpr uint32_t kSwarBadMask = 0xF8F8F8F8u;
 __device__ __forceinline__ uint32_t prmt_b32(uint32_t a, uint32_t b, uint32_t sel) {  // no & 0x7777 as in __byte_perm
     uint32_t d;

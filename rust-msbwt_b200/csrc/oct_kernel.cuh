@@ -1,6 +1,6 @@
-// oct_kernel.cuh -- the search kernel over the oct image (layout.h), shared by the two translation units that
-// instantiate it: quad_kernels.cu (packed live list) and fused_kernels.cu (symbol bytes in, counts out).  Two
-// modules because ptxas 12.9 crashes on one that holds both instantiations.
+// oct_kernel.cuh -- the search kernel over the oct image (layout.h), shared by the three translation units that
+// instantiate it: quad_kernels.cu (the search), stats_kernels.cu (the counting instantiation) and wide_kernels.cu
+// (64-bit positions).  One instantiation per module because ptxas 12.9 crashes on a module that holds two.
 #pragma once
 #include "device_rank.cuh"
 #include "engine.h"
@@ -39,7 +39,6 @@ constexpr int kOctRowBytes = 144;    // a 128-byte line + 16: rows of consecutiv
 constexpr int kOctPoolBytes = 640;   // 32 x (u64 symbol word, u64 seed range, u32 original index)
 constexpr int kOctWidePoolBytes = 896;  // WIDE: 32 x (u64 symbol word, u64 l, u64 h, u32 original index)
 constexpr int kOctChunk = 512;       // queries a warp takes from the live list at a time (fewer when the list is short)
-constexpr int kOctRawPoolBytes = 1072;  // fused path: 32 queries x k <= 32 symbol bytes, + the slack an unaligned 36-byte read needs
 
 __device__ __forceinline__ void cp_async16(void *smem, const void *gmem, bool on) {
     const uint32_t dst = (uint32_t)__cvta_generic_to_shared(smem);
@@ -103,12 +102,7 @@ __device__ __forceinline__ uint32_t staged_sector_rank(const uint4 &a, const uin
            __popc(b.w & below_mask(p - 192));
 }
 
-// RAW = false: the queries come packed and seeded from the pack / seed kernels (live list A of `packed`).
-// RAW = true (fused path, k <= 32): the queries come as the caller's symbol bytes (`syms`, n * k); every warp
-// stages 32 of them at a time, each lane packs its own k-mer (SWAR, the same arithmetic as pack_seed_kernel),
-// fetches its suffix-table entry as one more kind of step of the same loop and writes its count to out[query]
-// -- no pack kernel, no live list written and read back.  A k-mer holding a symbol outside ACGT is appended to
-// `exc` (count, then query indices) and counted afterwards by count_exceptions_kernel.
+// The queries come packed and seeded from the pack / seed kernels (live list A of `packed`).
 // STATS = true (stats_kernels.cu, never on a timed path): the same walk also counts what it fetches -- stats[0] oct
 // lines, [1] final-step lines, [2] final-step lines that had overflowed (their query then takes the oct steps),
 // [3] quad steps, [4] distinct 128-byte lines those read, [5] one-symbol steps, [6] distinct 64-byte blocks those
@@ -119,22 +113,20 @@ __device__ __forceinline__ uint32_t staged_sector_rank(const uint4 &a, const uin
 // count the low byte of word 1 (layout.h); such an index has no quad image beside the oct image (36.6 B per position
 // have no room), so remainders, overflowed lines and ranges over two buckets take one-symbol steps.
 constexpr int kOctStatWords = 8;
-template <bool RAW, bool STATS = false, bool WIDE = false>
+template <bool STATS = false, bool WIDE = false>
 __global__ void __launch_bounds__(kCountThreads, WIDE ? 3 : MSBWT_OCT_CTAS)
 count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, PackedLayout lay, uint32_t k,
-                       uint64_t *__restrict__ out, uint32_t *__restrict__ work, const uint8_t *__restrict__ syms,
-                       uint32_t n_raw, uint32_t *__restrict__ exc, unsigned long long *__restrict__ stats = nullptr) {
-    static_assert(!(RAW && WIDE), "the fused path is compiled for 32-bit positions only");
+                       uint64_t *__restrict__ out, uint32_t *__restrict__ work, unsigned long long *__restrict__ stats = nullptr) {
     using P = typename Pos<WIDE>::type;
     extern __shared__ __align__(16) uint8_t smem[];
     __shared__ uint64_t cb_smem[WIDE ? kMaxSuperInSmem * 8 : 4];
     const CBase<WIDE> cb = stage_cbase<WIDE>(ix, cb_smem);
     const uint64_t stream = policy_evict_first();
     constexpr uint32_t kFull = 0xffffffffu;
-    constexpr uint32_t kPool = RAW ? kOctRawPoolBytes : (WIDE ? kOctWidePoolBytes : kOctPoolBytes);
+    constexpr uint32_t kPool = WIDE ? kOctWidePoolBytes : kOctPoolBytes;
     constexpr uint32_t kWarpSmem = 32 * kOctRowBytes + 2 * kPool;
 
-    const uint32_t n = RAW ? n_raw : (uint32_t)packed[lay.live()];  // queries to walk (live list A)
+    const uint32_t n = (uint32_t)packed[lay.live()];  // queries to walk (live list A)
     // CONVERGENCE.  The warp protocol below (a ballot, requests and lines other lanes read from shared memory, four
     // __syncwarp(), a warp-wide scan -- and, when the trouble was found, 24 shuffles per iteration) needs the 32
     // lanes together at every one of those points.  Left alone, ptxas 12.9 "proves" that they are (the divergent
@@ -157,16 +149,13 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
     const uint32_t bshift = ix.oct_shift, bmask = (1u << bshift) - 1u;
     const char *const oct_base = reinterpret_cast<const char *>(ix.oct);
     const char *const quad_base = reinterpret_cast<const char *>(ix.quad);
-    const uint32_t back0 = ix.table_s - depth0;  // which of the kept table levels (RAW)
-    const char *const table_base = reinterpret_cast<const char *>(
-        back0 == 0 ? ix.table : (back0 == 1 ? ix.table2 : (back0 == 2 ? ix.table3 : ix.table4)));
     uint8_t *const rows = smem + (threadIdx.x >> 5) * kWarpSmem;  // 32 rows of kOctRowBytes
     uint8_t *const pools = rows + 32 * kOctRowBytes;               // 2 pools of 32 queries
     const uint4 *const my_row = reinterpret_cast<const uint4 *>(rows + lane * kOctRowBytes);
     // this lane copies bytes [16 j, 16 j + 16) of the lines of rows 4 c + (lane >> 3): of every oct / final-step line
-    // (kind 1), of a quad request (kind 2) when j < 4, of a table entry (kind 3) when j == 0 -- bit `kind` of piece_on
+    // (kind 1) and of a quad request (kind 2) when j < 4 -- bit `kind` of piece_on
     const uint32_t piece_off = 16u * (lane & 7u);
-    const uint32_t piece_on = 2u | ((lane & 7u) < 4u ? 4u : 0u) | ((lane & 7u) == 0u ? 8u : 0u);
+    const uint32_t piece_on = 2u | ((lane & 7u) < 4u ? 4u : 0u);
     const uint32_t piece_hmask = (lane & 7u) >= 2u ? ~0u : 0u;  // pieces 2, 3 of a quad request: the sector of h
 
     // A list that is not long against the grid (the leftovers of the one-request kernel: a percent of the batch; a
@@ -194,25 +183,15 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
     };
     auto load_pool = [&](uint32_t buf, uint32_t base, uint32_t cnt) {
         uint8_t *p = pools + buf * kPool;
-        if constexpr (RAW) {  // cnt * k symbol bytes, 16 at a time (base is a multiple of 32: 16-byte aligned)
-            const uint8_t *src = syms + (uint64_t)base * k;
-            const uint32_t bytes = cnt * k;
-#pragma unroll
-            for (uint32_t c = lane; c < 64u; c += 32u) {
-                const uint32_t at = 16u * c;
-                cp_async16_partial(p + at, src + at, at < bytes ? min(16u, bytes - at) : 0u);
-            }
+        const uint32_t idx = base + lane;
+        const bool on = lane < cnt;
+        cp_async8(p + 8u * lane, w0 + idx, on);
+        cp_async8(p + 256u + 8u * lane, seeds + idx, on);
+        if constexpr (WIDE) {
+            cp_async8(p + 512u + 8u * lane, seeds + lay.n + idx, on);
+            cp_async4(p + 768u + 4u * lane, qidx + idx, on);
         } else {
-            const uint32_t idx = base + lane;
-            const bool on = lane < cnt;
-            cp_async8(p + 8u * lane, w0 + idx, on);
-            cp_async8(p + 256u + 8u * lane, seeds + idx, on);
-            if constexpr (WIDE) {
-                cp_async8(p + 512u + 8u * lane, seeds + lay.n + idx, on);
-                cp_async4(p + 768u + 4u * lane, qidx + idx, on);
-            } else {
-                cp_async4(p + 512u + 4u * lane, qidx + idx, on);
-            }
+            cp_async4(p + 512u + 4u * lane, qidx + idx, on);
         }
     };
     uint32_t seq = 0, a_pos = 0, a_cnt, b_cnt, a_base, b_base;
@@ -237,7 +216,6 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
         }
     };
     bool active = false;
-    bool need_table = false;  // RAW: the next step is the suffix-table lookup
     P l = 0, h = 0;
     uint64_t word = 0, pend = 0;
     uint32_t q = 0;
@@ -270,7 +248,7 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
 
     for (;;) {
         // ---- RETIRE + REFILL (warp-uniform control)
-        if (active && !need_table && (rem == 0 || l == h)) {
+        if (active && (rem == 0 || l == h)) {
             stg_stream(out + q, (uint64_t)(h - l), stream);
             active = false;
         }
@@ -292,52 +270,20 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
                     wd_age = 0;
 #endif
                     if constexpr (STATS) st_cnt[7]++;
-                    if constexpr (RAW) {
-                        q = (from_a ? a_base : b_base) + slot;
-                        // k symbol bytes at p + slot * k -> 2 bits each, the k-mer's last symbol in the top bits
-                        const uint32_t off = slot * k, sh8 = 8u * (off & 3u);
-                        const volatile uint32_t *wsrc = reinterpret_cast<const volatile uint32_t *>(p + (off & ~3u));
-                        uint32_t prev = wsrc[0], bad = 0;
-                        uint64_t le = 0;
-#pragma unroll
-                        for (uint32_t i = 0; i < 8u; i++) {
-                            const uint32_t nxt = wsrc[i + 1];
-                            uint32_t x = __funnelshift_r(prev, nxt, sh8);  // symbols 4i .. 4i+3
-                            prev = nxt;
-                            const uint32_t nvalid = k > 4u * i ? min(4u, k - 4u * i) : 0u;
-                            const uint32_t keep = nvalid >= 4u ? 0xFFFFFFFFu : ((1u << (8u * nvalid)) - 1u);
-                            x = (x & keep) | (0x01010101u & ~keep);  // bytes past the k-mer count as 'A'
-                            bad |= swar_non_acgt(x);
-                            le |= (uint64_t)swar_pack4(x) << (8u * i);
-                        }
-                        word = le << (64u - 2u * k);
-                        if (bad) {  // $, N or an invalid byte: counted by count_exceptions_kernel
-                            exc[1u + atomicAdd(exc, 1u)] = q;
-                            active = false;
-                        } else if (depth0) {
-                            need_table = true;
-                            rem = k;
-                        } else {
-                            l = 0;
-                            h = (uint32_t)ix.total;
-                            rem = k;
-                        }
+                    word = *reinterpret_cast<const volatile uint64_t *>(p + 8u * slot);
+                    const uint64_t lo = *reinterpret_cast<const volatile uint64_t *>(p + 256u + 8u * slot);
+                    const uint32_t qraw = *reinterpret_cast<const volatile uint32_t *>(p + (WIDE ? 768u : 512u) + 4u * slot);
+                    q = qraw & kQidxMask;
+                    no_fin = ((qraw >> 30) & 1u) != 0u;  // pack_seed_final_kernel already found this query's line overflowed
+                    if constexpr (WIDE) {
+                        l = lo;
+                        h = *reinterpret_cast<const volatile uint64_t *>(p + 512u + 8u * slot);
                     } else {
-                        word = *reinterpret_cast<const volatile uint64_t *>(p + 8u * slot);
-                        const uint64_t lo = *reinterpret_cast<const volatile uint64_t *>(p + 256u + 8u * slot);
-                        const uint32_t qraw = *reinterpret_cast<const volatile uint32_t *>(p + (WIDE ? 768u : 512u) + 4u * slot);
-                        q = qraw & kQidxMask;
-                        no_fin = ((qraw >> 30) & 1u) != 0u;  // pack_seed_final_kernel already found this query's line overflowed
-                        if constexpr (WIDE) {
-                            l = lo;
-                            h = *reinterpret_cast<const volatile uint64_t *>(p + 512u + 8u * slot);
-                        } else {
-                            l = (uint32_t)lo;
-                            h = (uint32_t)(lo >> 32);
-                        }
-                        rem = rem0;
-                        if (rem > (uint32_t)kPairSymsPerWord) pend = ldg_stream(wx + q, stream);
+                        l = (uint32_t)lo;
+                        h = (uint32_t)(lo >> 32);
                     }
+                    rem = rem0;
+                    if (rem > (uint32_t)kPairSymsPerWord) pend = ldg_stream(wx + q, stream);
                 }
                 const uint32_t taken = min((uint32_t)__popc(want), avail);
                 if (taken >= avail_a) {  // pool A is used up: B becomes A, the next pool is staged into A's buffer
@@ -374,8 +320,7 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
         // ---- ISSUE (branch-free): every lane publishes what its query needs, the warp fetches it
         // (a range over two buckets, like an overflowed line, takes its kOctSyms symbols as quad steps and, for
         // the last two of ten, one-symbol steps)
-        const bool is_table = RAW && active && need_table;
-        const bool live = active && !is_table && rem != 0 && l != h;
+        const bool live = active && rem != 0 && l != h;
         const P bl = l >> bshift, bh = h >> bshift;
         // exactly kFinSyms symbols left: ONE final-step line answers the count (no rank needed for the last step)
         const bool is_fin = live && fin_base != nullptr && rem == (uint32_t)kFinSyms && forced == 0u && !no_fin &&
@@ -388,16 +333,14 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
         const uint32_t codem = peek((uint32_t)kOctSyms);
         const uint32_t code8 = peek(4u);
         const uint32_t sl = WIDE ? 0u : (uint32_t)l / (uint32_t)kQuadSyms, sh = WIDE ? 0u : (uint32_t)h / (uint32_t)kQuadSyms;
-        const uint64_t entry = RAW ? (word >> (64u - 2u * (depth0 ? depth0 : 1u))) : 0ull;  // suffix-table index
         const char *p0 = is_oct ? oct_base + ((size_t)codem * ix.nbuck8 + bl) * kOctLineBytes
                                 : quad_base + ((size_t)code8 * ix.nsec4 + sl) * kQuadSectorBytes;
-        if (is_table) p0 = table_base + ((entry * 8u) & ~15ull);
         if (is_fin) p0 = fin_base + ((((size_t)(l >> fshift)) << flb) | (size_t)(fin_mixed & ((1ull << flb) - 1ull))) * kFinLineBytes;
         // kind: 1 oct line or final-step line (all eight 16-byte pieces), 2 quad (the sector of l into bytes 0..31 of the
-        // row, the sector of h into 32..63), 3 table entry (its 16 bytes into bytes 0..15), 0 nothing.  h_adj (quad): what
-        // pieces 2 and 3 add to `p0 + 16 j` to land in the sector of h -- its byte distance from the sector of l, less the 32
-        // bytes the two pieces already skipped (mod 2^32: 16 j >= 32 there, the sum is never negative)
-        const uint32_t kind = is_table ? 3u : ((is_oct || is_fin) ? 1u : (is_quad ? 2u : 0u));
+        // row, the sector of h into 32..63), 0 nothing.  h_adj (quad): what pieces 2 and 3 add to `p0 + 16 j` to land in
+        // the sector of h -- its byte distance from the sector of l, less the 32 bytes the two pieces already skipped
+        // (mod 2^32: 16 j >= 32 there, the sum is never negative)
+        const uint32_t kind = (is_oct || is_fin) ? 1u : (is_quad ? 2u : 0u);
         const uint32_t h_adj = is_quad ? (sh - sl) * (uint32_t)kQuadSectorBytes - 32u : 0u;
         if constexpr (STATS) {
             st_cnt[0] += is_oct;
@@ -442,14 +385,7 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
         // ---- CONSUME (each lane ranks in its own staged line)
         bool fin_scan = false;                 // this lane's final-step line is good: its runs are summed in phase 2
         uint32_t fin_at = 0, fin_left = 0;     // header word of the first group of its code, groups of that code
-        if (is_table) {
-            const uint4 e = my_row[0];
-            l = (entry & 1ull) ? e.z : e.x;
-            h = (entry & 1ull) ? e.w : e.y;
-            word <<= 2u * depth0;
-            rem = rem0;
-            need_table = false;
-        } else if (is_fin) {
+        if (is_fin) {
             const uint4 first = my_row[0];
             const uint32_t used = first.x;  // <= 31 in any line the builder wrote
             if (used == kFinOverflow) {
@@ -570,7 +506,6 @@ count_kmers_oct_kernel(IndexView ix, const uint64_t *__restrict__ packed, Packed
 
 // dynamic shared memory per CTA
 constexpr int kOctSmemPacked = (kCountThreads / 32) * (32 * kOctRowBytes + 2 * kOctPoolBytes);
-constexpr int kOctSmemRaw = (kCountThreads / 32) * (32 * kOctRowBytes + 2 * kOctRawPoolBytes);
 constexpr int kOctSmemWide = (kCountThreads / 32) * (32 * kOctRowBytes + 2 * kOctWidePoolBytes);
 
 // one full wave of CTAs for a kernel with `smem` bytes of dynamic shared memory, fewer if there is less work

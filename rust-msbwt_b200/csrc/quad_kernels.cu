@@ -121,16 +121,16 @@ cudaError_t launch_count_quad(int device, const IndexView &ix, const uint64_t *d
     if (ix.oct) {
         static bool prepared[64] = {};  // per device: 4 CTAs x 47 KB of staging per SM need the large shared-memory configuration
         if (device < 0 || device >= 64 || !prepared[device]) {
-            cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kOctSmemPacked);
-            cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+            cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<>, cudaFuncAttributeMaxDynamicSharedMemorySize, kOctSmemPacked);
+            cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
             if (device >= 0 && device < 64) prepared[device] = true;
         }
         // the chunk dispenser lives in the scratch buffer next to the live counters (engine bookkeeping: the
         // buffer is the engine's own scratch, `const` only towards the caller's data in it)
         uint32_t *work = reinterpret_cast<uint32_t *>(const_cast<uint64_t *>(d_packed) + lay.work());
         if (cudaError_t e = cudaMemsetAsync(work, 0, sizeof(uint32_t), st); e != cudaSuccess) return e;
-        const unsigned grid = oct_grid(device, (const void *)count_kmers_oct_kernel<false>, kOctSmemPacked, lay.n);
-        count_kmers_oct_kernel<false><<<grid, kCountThreads, kOctSmemPacked, st>>>(ix, d_packed, lay, k, d_out, work, nullptr, 0u, nullptr);
+        const unsigned grid = oct_grid(device, (const void *)count_kmers_oct_kernel<>, kOctSmemPacked, lay.n);
+        count_kmers_oct_kernel<><<<grid, kCountThreads, kOctSmemPacked, st>>>(ix, d_packed, lay, k, d_out, work);
         return cudaGetLastError();
     }
     return launch_count_quad_t<false>(device, ix, d_packed, lay, k, d_out, st);

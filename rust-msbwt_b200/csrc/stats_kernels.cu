@@ -1,4 +1,4 @@
-// stats_kernels.cu -- the COUNTING instantiation of the oct search kernel (count_kmers_oct_kernel<false, true>,
+// stats_kernels.cu -- the COUNTING instantiation of the oct search kernel (count_kmers_oct_kernel<true>,
 // oct_kernel.cuh): the same walk over live list A that also counts every index line it fetches.  Measurement aid
 // for bench.py's roofline accounting (the exact algorithmic traffic of the implemented algorithm on a batch);
 // never on a timed path.  A translation unit of its own because ptxas 12.9 crashes on a module that holds two
@@ -14,15 +14,15 @@ cudaError_t launch_count_oct_stats(int device, const IndexView &ix, const uint64
     const PackedLayout lay = packed_layout(ix, k, n);
     static bool prepared[64] = {};
     if (device < 0 || device >= 64 || !prepared[device]) {
-        if (cudaError_t e = cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kOctSmemPacked); e != cudaSuccess) return e;
-        cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<false, true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        if (cudaError_t e = cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kOctSmemPacked); e != cudaSuccess) return e;
+        cudaFuncSetAttribute((const void *)count_kmers_oct_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
         if (device >= 0 && device < 64) prepared[device] = true;
     }
     uint32_t *work = reinterpret_cast<uint32_t *>(const_cast<uint64_t *>(d_packed) + lay.work());
     if (cudaError_t e = cudaMemsetAsync(work, 0, sizeof(uint32_t), st); e != cudaSuccess) return e;
     if (cudaError_t e = cudaMemsetAsync(d_stats, 0, kOctStatWords * sizeof(unsigned long long), st); e != cudaSuccess) return e;
-    const unsigned grid = oct_grid(device, (const void *)count_kmers_oct_kernel<false, true>, kOctSmemPacked, lay.n);
-    count_kmers_oct_kernel<false, true><<<grid, kCountThreads, kOctSmemPacked, st>>>(ix, d_packed, lay, k, d_out, work, nullptr, 0u, nullptr, d_stats);
+    const unsigned grid = oct_grid(device, (const void *)count_kmers_oct_kernel<true>, kOctSmemPacked, lay.n);
+    count_kmers_oct_kernel<true><<<grid, kCountThreads, kOctSmemPacked, st>>>(ix, d_packed, lay, k, d_out, work, d_stats);
     return cudaGetLastError();
 }
 

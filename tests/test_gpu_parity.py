@@ -441,13 +441,3 @@ def test_device_built_image_equals_host_built_image(sb_shift):
         assert g.get_total_size() == o.get_total_size()
         assert [g.get_symbol_count(s) for s in range(6)] == [o.get_symbol_count(s) for s in range(6)]
         assert [g.start_index(s) for s in range(6)] == [o.start_index(s) for s in range(6)]
-
-
-def test_host_build_path_still_answers_identically(monkeypatch, midsize):
-    from harness import synth
-    reads, g, o = midsize
-    monkeypatch.setenv("MSBWT_HOST_BUILD", "1")
-    h = M.RleBWT()
-    h.load_vector(o.rle_bytes())
-    q = synth.make_queries(reads, 25, 5000, 5000).cpu().numpy()
-    assert (h.count_kmers_fixed(q, 25) == g.count_kmers_fixed(q, 25)).all()

@@ -50,11 +50,11 @@ def test_every_warp_cooperative_search_kernel_keeps_its_warp_syncs(sass_counts):
         assert got, "no such kernel in the library"
         return got
 
-    # the oct search kernel: packed, fused (RAW), counting (STATS) and WIDE instantiations -- per iteration a ballot, the
+    # the oct search kernel: packed, counting (STATS) and WIDE instantiations -- per iteration a ballot, the
     # line requests exchanged through shared memory, cp.async rows read by other lanes, four __syncwarp(), the warp-wide
     # scan of the final-step lines (vote + reduce); ptxas's conservative build carries a WARPSYNC.COLLECTIVE for each
     oct_kernels = pick(lambda k: "count_kmers_oct_kernel<" in k)
-    assert len(oct_kernels) == 4
+    assert len(oct_kernels) == 3
     for name, c in oct_kernels.items():
         assert c["VOTE"] >= 4 and c["WARPSYNC"] >= 8, (name, c)
     # quads of lanes (pair image) and lane pairs (one-step blocks, LANES = 2) combine their parts through shuffles
