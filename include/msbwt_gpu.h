@@ -75,25 +75,23 @@ msbwt_index *msbwt_index_create_from_npy(const char *path, const int *devices, i
  * but never implemented, src/msbwt_core.rs:133-146); k-mers whose last s symbols are ACGT
  * start from it, bit-exactly.  -1 = automatic (ceil(log4(N/32)), at most 13 -- deepened up to 15 for
  * an index that lives in HBM, while the tables stay below 4x the block images and a quarter of the
- * free device memory; the MSBWT_SUFFIX_TABLE_S environment variable overrides), 0 = none, 1..15
- * explicit. */
+ * free device memory), 0 = none, 1..15 explicit. */
 msbwt_index *msbwt_index_create_ex(const uint8_t *rle, uint64_t len, const int *devices, int ndev,
                                    uint32_t superblock_shift, int suffix_table_s, int *err);
 
 /* The same with every knob in one growable struct (set struct_size = sizeof(msbwt_options)).
  * `pair_index`: the PAIR image -- one 128-byte line per 96 BWT positions that answers TWO
  * constrain_range steps with one line fill (layout.h) -- is built next to the one-step blocks when
- * the index lives in HBM (-1 = automatic: one-step blocks + suffix table > 2 x L2; the
- * MSBWT_PAIR_INDEX=0|1 environment variable overrides), 0 = never, 1 = always.  Results are
- * identical either way.  `kernel_lanes`: 0 = automatic, 1 or 2 (see msbwt_kernel_lanes).
+ * the index lives in HBM (-1 = automatic: one-step blocks + suffix table > 2 x L2), 0 = never,
+ * 1 = always.  Results are identical either way.  `kernel_lanes`: 0 = automatic, 1 or 2 (see msbwt_kernel_lanes).
  * `quad_index`: the QUAD image -- one occurrence bit-vector per 4-symbol code in self-contained
  * 32-byte sectors (layout.h), FOUR constrain_range steps per line fill, 256*N/7 bytes -- replaces the
  * pair image (-1 = automatic: the index lives in HBM and the image is <= 64 GB and <= half the free
- * device memory; MSBWT_QUAD_INDEX=0|1 overrides), 0 = never, 1 = always.  Results are identical.
+ * device memory), 0 = never, 1 = always.  Results are identical.
  * `oct_index`: the OCT image -- one 128-byte line of explicit occurrence RUNS per (m-symbol code, 2^b-position
  * bucket), m = msbwt_oct_symbols() = 10 constrain_range steps per line fill, 128 * 4^m * (N / 2^b + 1) bytes --
  * is built next to the quad image (-1 = automatic: whenever the quad image is built and the oct image fits a quarter
- * of the device memory left; MSBWT_OCT_INDEX=0|1 overrides), 0 = never, 1 = always (implies quad_index).  An index
+ * of the device memory left), 0 = never, 1 = always (implies quad_index).  An index
  * whose positions need 64 bits (2^32 symbols and more -- the reference is u64 throughout, src/msbwt_core.rs:18-24 --
  * or several superblocks) gets the same lines with 40-bit checkpoints, built by walking LF through the one-step
  * blocks, and no quad image (36.6 bytes per position have no room): automatic when it lives in HBM and the images
@@ -105,15 +103,25 @@ msbwt_index *msbwt_index_create_ex(const uint8_t *rle, uint64_t len, const int *
  * serves remainders of 4..9 symbols and the oct kernel's rare fallbacks, which one-symbol ranks answer as well.
  * -1 = automatic (kept when quad + 40 bytes per symbol for the other images fit 70 % of the device: 55 GB at
  * 1.51 Gsymbols; dropped at 3.02 Gsymbols, where it would be 110 GB), 0 = drop it once the images are built,
- * 1 = keep (MSBWT_KEEP_QUAD=0|1 overrides the automatic choice).  Results are identical either way.
+ * 1 = keep.  Results are identical either way.
  * `final_index`: the FINAL-STEP image on top of the oct image -- the LAST 20 symbols a count_kmer consumes need no
  * rank, only the number of positions of [l, h) preceded by those 20 symbols, so one hashed 128-byte line of explicit
  * runs per (20-symbol code, 2^16-position bucket) answers them: a 31-mer is one L2-resident depth-11 table entry +
- * ONE line fill.  -1 = automatic (built whenever the oct image is; MSBWT_FINAL_INDEX=0|1 overrides), 0 = never,
+ * ONE line fill.  -1 = automatic (built whenever the oct image is), 0 = never,
  * 1 = always (create fails if it cannot be built).  A line whose groups do not fit, or a range over two buckets,
  * takes the two oct steps instead, so results are identical on any input.  `final_bucket_shift` (8..16, 0 = 16) and
  * `final_lines_log2` (12..20 lines per bucket; 0 = automatic: 13 = 16 bytes per symbol when that fits 30 % of
- * the device memory, else 12 = 8 bytes per symbol). */
+ * the device memory, else 12 = 8 bytes per symbol).
+ * Environment: ten variables set the same knobs for every create call, the ones without an msbwt_options
+ * argument included -- MSBWT_SUFFIX_TABLE_S (suffix_table_s), MSBWT_PAIR_INDEX (pair_index), MSBWT_QUAD_INDEX
+ * (quad_index), MSBWT_OCT_INDEX (oct_index), MSBWT_OCT_BUCKET_SHIFT (oct_bucket_shift), MSBWT_KEEP_QUAD
+ * (keep_quad_index), MSBWT_FINAL_INDEX (final_index), MSBWT_FINAL_BUCKET_SHIFT (final_bucket_shift),
+ * MSBWT_FINAL_LINES_LOG2 (final_lines_log2) and MSBWT_LANES (kernel_lanes).  One rule for all ten: a variable
+ * applies only when its field is automatic (suffix_table_s < 0; pair_index, quad_index, oct_index,
+ * keep_quad_index, final_index = -1; the shifts and final_lines_log2 = 0; kernel_lanes neither 1 nor 2), and then
+ * means exactly what setting the field would.  Values are read as integers: the suffix table depth is clamped to
+ * 0..15, any value of MSBWT_PAIR_INDEX / MSBWT_QUAD_INDEX / MSBWT_OCT_INDEX other than 0 means 1, and any value
+ * of MSBWT_LANES other than 2 means 1. */
 typedef struct msbwt_options {
     uint32_t struct_size;
     uint32_t superblock_shift; /* 0 = default */
@@ -146,7 +154,7 @@ int msbwt_device_ordinal(const msbwt_index *idx, int slot);
 uint64_t msbwt_index_bytes(const msbwt_index *idx); /* device bytes per replica, suffix table included */
 int msbwt_suffix_table_s(const msbwt_index *idx);     /* suffix table depth in use (0 = none) */
 /* lanes per query of the search kernel chosen for this index: 1 = one thread per query (index
- * L2-resident), 2 = a lane pair per query (index in HBM); MSBWT_LANES=1|2 overrides at create */
+ * L2-resident), 2 = a lane pair per query (index in HBM); msbwt_options.kernel_lanes sets it */
 int msbwt_kernel_lanes(const msbwt_index *idx);
 int msbwt_pair_index(const msbwt_index *idx); /* 1 when the pair image is in use */
 int msbwt_quad_index(const msbwt_index *idx); /* 1 when the quad image is in use (it replaces the pair image) */
@@ -164,6 +172,17 @@ int msbwt_debug_copy_final_image(const msbwt_index *idx, int slot, uint64_t *nli
                                  uint32_t *lines_log2, uint64_t *overflow_lines, uint32_t *lines /* nlines * 32, or NULL */);
 /* the same policy without an index: `steps` = symbols per step of the image (1, 2, 4 or msbwt_oct_symbols()); -1 otherwise */
 int msbwt_debug_table_depth(uint32_t k, uint32_t table_s, uint32_t steps);
+/* The layout policy without a device: what create plans for one replica from `opts` (NULL = all automatic) and the
+ * environment, for an index of `total` symbols (`wide` != 0: 64-bit positions) whose bare replica -- block image,
+ * aux and superblock counts -- takes `block_bytes`, on a device with `l2_bytes` of L2, `free_bytes` free and
+ * `device_bytes` in all.  plan[0..14] = suffix-table depth before the deepening for HBM, depth fixed by the caller or
+ * the environment (not deepened), index in HBM, wide oct route, quad route, oct image on the quad route, final-step
+ * image, pair image alone, keep the quad image under the oct image, oct image required, final-step image required,
+ * log2 of final-step lines per bucket, kernel lanes, oct bucket shift (0 = automatic), final-step bucket shift.  The quad,
+ * oct-on-quad and pair fields say what is built when the wide oct route is not taken or runs out of memory.
+ * EINVAL when nplan < 15 or opts is invalid. */
+int msbwt_debug_plan_layout(const msbwt_options *opts, uint64_t total, int wide, uint64_t block_bytes,
+                            uint64_t l2_bytes, uint64_t free_bytes, uint64_t device_bytes, int32_t *plan, int nplan);
 
 /* ---- queries from HOST buffers (the drop-in calls) ---- */
 

@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <iterator>
 #include <thread>
 
 #include "handle.h"
@@ -169,60 +170,132 @@ struct Options {
     int keep_quad = -1; // under an oct image: -1 auto, 0 drop the quad image once the other images are built, 1 keep it
     int fin = -1;       // final-step image on top of the oct image: -1 auto (on), 0 off, 1 on (fail if it cannot be built)
     int fin_shift = 0;  // 0 = 16
-    int fin_lb = 0;     // 0 auto (13 = 16 B/symbol when that fits a quarter of the device, else 12 = 8 B/symbol)
+    int fin_lb = 0;     // 0 auto (13 = 16 B/symbol when that fits 30 % of the device, else 12 = 8 B/symbol)
     int lanes = 0;      // 0 auto, 1, 2
 };
 
-// `explicit_choice` is set when the caller or the environment fixed the depth
-int pick_table_s(uint64_t total, int requested, bool *explicit_choice) {
-    *explicit_choice = true;
-    if (requested >= 0) return requested > kMaxTableS ? kMaxTableS : requested;
-    if (const char *env = getenv("MSBWT_SUFFIX_TABLE_S")) {
-        int v = atoi(env);
-        return v < 0 ? 0 : (v > kMaxTableS ? kMaxTableS : v);
-    }
-    *explicit_choice = false;
-    int s = 0;
-    while (s < kAutoMaxTableS && (1ull << (2 * s)) < total / 32) s++;
-    return s;
+// The environment fills the layout knobs the caller left automatic, before the layout is planned: each variable means
+// what the same value of its msbwt_options field means (include/msbwt_gpu.h)
+void fill_from_env(Options &o) {
+    auto env_int = [](const char *name, int fallback) { const char *e = getenv(name); return e ? atoi(e) : fallback; };
+    const char *e;
+    if (o.table_s < 0 && (e = getenv("MSBWT_SUFFIX_TABLE_S"))) o.table_s = std::clamp(atoi(e), 0, kMaxTableS);
+    if (o.lanes != 1 && o.lanes != 2 && (e = getenv("MSBWT_LANES"))) o.lanes = atoi(e) == 2 ? 2 : 1;
+    if (o.pair == -1 && (e = getenv("MSBWT_PAIR_INDEX"))) o.pair = atoi(e) != 0;
+    if (o.quad == -1 && (e = getenv("MSBWT_QUAD_INDEX"))) o.quad = atoi(e) != 0;
+    if (o.oct == -1 && (e = getenv("MSBWT_OCT_INDEX"))) o.oct = atoi(e) != 0;
+    if (o.keep_quad == -1) o.keep_quad = env_int("MSBWT_KEEP_QUAD", -1);
+    if (o.fin == -1) o.fin = env_int("MSBWT_FINAL_INDEX", -1);
+    if (!o.fin_shift) o.fin_shift = env_int("MSBWT_FINAL_BUCKET_SHIFT", 16);
+    if (!o.fin_lb) o.fin_lb = env_int("MSBWT_FINAL_LINES_LOG2", 0);
+    if (!o.oct_shift) o.oct_shift = env_int("MSBWT_OCT_BUCKET_SHIFT", 0);
+}
+
+// What the policy reads of a device: its L2 size and its memory before any optional image is built
+struct DeviceSizes {
+    uint64_t l2 = 0, free = 0, total = 0;
+};
+
+DeviceSizes device_sizes(int device) {
+    int l2 = 0;
+    size_t free_b = 0, total_b = 0;
+    if (cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, device) != cudaSuccess || l2 <= 0) l2 = 96 << 20;
+    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) free_b = total_b = 0;
+    return {(uint64_t)l2, free_b, total_b};
+}
+
+// Free memory of the current device as a build stage finds it (0 when it cannot be read)
+uint64_t free_bytes_now() {
+    size_t free_b = 0, total_b = 0;
+    return cudaMemGetInfo(&free_b, &total_b) == cudaSuccess ? free_b : 0;
+}
+
+// The images a replica gets, its suffix-table depth and its kernel lanes (msbwt_debug_plan_layout writes these fields)
+struct Layout {
+    int table_s = 0;            // before the deepening for HBM (deepen_table_for_hbm)
+    bool explicit_s = false;    // the caller or the environment fixed the depth: it is not deepened
+    bool hbm = false;           // one-step blocks + suffix table > 2 x L2
+    bool wide_oct = false;      // 64-bit positions: oct (and final-step) lines by walking LF, no quad image
+    bool quad = false;          // the quad route (pair -> quad [-> oct -> final-step]), when no wide images were built
+    bool oct = false;           // oct lines on top of the quad image
+    bool fin = false;           // final-step lines on top of the oct lines
+    bool pair = false;          // the pair image alone
+    bool keep_quad = false;     // the quad image stays once the oct lines exist
+    bool oct_required = false;  // oct_index = 1: no 8 GB reserve beside the oct lines; the wide route must succeed
+    bool fin_required = false;  // final_index = 1: create fails without the final-step lines
+    int fin_lb = 0;             // log2 of the final-step lines per bucket
+    int lanes = 1;
+    int oct_shift = 0, fin_shift = 0;
+};
+
+// The layout policy: a function of the options (the environment folded in), the index's size, the bytes of its bare
+// replica (block image) and the device's sizes, and nothing else.
+Layout plan_layout(const Options &opt, uint64_t N, bool wide, uint64_t block_bytes, const DeviceSizes &dev) {
+    Layout p;
+    p.explicit_s = opt.table_s >= 0;
+    p.table_s = p.explicit_s ? std::min(opt.table_s, kMaxTableS) : 0;
+    while (!p.explicit_s && p.table_s < kAutoMaxTableS && (1ull << (2 * p.table_s)) < N / 32) p.table_s++;
+    const uint64_t one_step = block_bytes + (p.table_s > 0 ? (1ull << (2 * p.table_s)) * (wide ? 16 : 8) : 0);
+    // Kernel mapping (kernels.cu): one thread per query while blocks + table are (mostly) L2-resident,
+    // a lane pair per query -- one coalesced 64-byte request per block -- once they live in HBM.
+    p.hbm = one_step > 2 * dev.l2;
+    p.lanes = opt.lanes == 1 || opt.lanes == 2 ? opt.lanes : (p.hbm ? 2 : 1);
+
+    // 64-bit positions: the oct and final-step images when the index lives in HBM, the caller pinned no other layout,
+    // and the two images at their coarsest settings plus the builders' scratch fit the free device memory.
+    p.oct_required = opt.oct == 1;
+    p.wide_oct = wide && (opt.oct == 1 || (opt.oct != 0 && opt.pair == -1 && opt.quad == -1 && p.hbm && (N >> 40) == 0 &&
+                                           oct_image_bytes(N, kOctMaxShift) + fin_image_bytes(N, 16, 12) + 12 * N +
+                                                   (8ull << 30) <= dev.free));
+
+    // The quad image (layout.h: one 32-byte sector per FOUR steps, 256 * N / 7 bytes) halves the line fills of the pair
+    // image again.  Automatic choice: the one-step index does not fit L2 (measured on the 151 Msymbol BWT, 1.7 x L2:
+    // 10.2 G queries/s through quad sectors + a depth-15 table in HBM against 7.3 G through the mostly L2-resident
+    // one-step blocks), the image stays below 64 GB (measured, profiles/r1_gather_big.json: random reads keep 93 % of
+    // their rate over a 64 GB buffer and lose three quarters of it over 128 GB) and below half of the free device
+    // memory.  When the oct image will sit on top (32-bit positions, not switched off) the quad image only serves
+    // fallbacks and remainders, the randomly read footprint is the oct image + the suffix table, and the quad image may
+    // take up to 65 % of the free memory (110 GB for configs[4]'s 3.02 Gsymbol BWT).  A pinned pair_index pins the
+    // layout: no quad image.
+    const bool narrow_oct = !wide && opt.oct != 0;
+    const uint64_t quad_bytes = quad_image_bytes(N);
+    if (opt.oct == 1 || opt.quad == 1) p.quad = true;
+    else if (opt.quad == 0 || opt.pair == 0 || opt.pair == 1) p.quad = false;
+    else p.quad = one_step > dev.l2 && (narrow_oct ? quad_bytes <= dev.free / 100 * 65
+                                                   : quad_bytes <= (64ull << 30) && quad_bytes <= dev.free / 2);
+    // The oct image (layout.h: one 128-byte line per kOctSyms = 10 steps) rides on the quad image, 32-bit positions
+    // only; the final-step image rides on the oct image.
+    p.oct = p.quad && narrow_oct;
+    p.fin = (p.oct || p.wide_oct) && opt.fin != 0;
+    p.fin_required = opt.fin == 1;
+    // The pair image (layout.h: one 128-byte line per two steps) pays off once the index lives in HBM;
+    // an L2-resident index is served faster by the 64-byte one-step blocks (smaller footprint).
+    p.pair = !p.quad && (opt.pair == 0 || opt.pair == 1 ? opt.pair == 1 : p.hbm);
+    // Under the oct image the quad image only serves remainders of 4..9 symbols and the rare fallbacks of the oct
+    // kernel, which one-symbol ranks answer as well: it is kept when quad + 40 B/symbol for the other two images fit
+    // 70 % of the device (55 GB at 1.51 Gsymbols), dropped otherwise (110 GB at 3.02 Gsymbols).
+    p.keep_quad = opt.keep_quad != -1 ? opt.keep_quad != 0 : quad_bytes + 40 * N <= dev.total / 10 * 7;
+    // Lines per final-step bucket: 2^13, 16 bytes per symbol (0.8 % of the read-sampled 31-mers find their line
+    // overflowed and take the oct steps), when that fits 30 % of the device (48 GB at 3.02 Gsymbols), else 2^12, 8 bytes
+    // per symbol (6.5 %)
+    p.fin_lb = opt.fin_lb ? opt.fin_lb : (fin_image_bytes(N, opt.fin_shift, 13) <= dev.total / 10 * 3 ? 13 : 12);
+    p.oct_shift = opt.oct_shift;
+    p.fin_shift = opt.fin_shift;
+    return p;
 }
 
 // An index that lives in HBM pays one 128-byte line fill per pair step whatever it does, and HBM is
 // large: every two further table levels remove one of those steps from every query.  Deepen the
-// automatic choice while the tables (depth s and s-1) stay below 4x the block images and a quarter
-// of the free device memory.
-int deepen_table_for_hbm(int s, uint64_t image_bytes, size_t entry_bytes) {
-    size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return s;
-    const uint64_t budget = std::min<uint64_t>(4 * image_bytes, free_b / 4);
+// automatic choice while the tables (depth s and s-1) stay below 4x the block and multi-step images and a
+// quarter of the free device memory once those images exist.
+int deepen_table_for_hbm(int s, uint64_t image_bytes, size_t entry_bytes, uint64_t free_bytes) {
+    const uint64_t budget = std::min<uint64_t>(4 * image_bytes, free_bytes / 4);
     while (s < kMaxTableS) {
         const uint64_t next = ((1ull << (2 * (s + 1))) + (1ull << (2 * s))) * entry_bytes;
         if (next > budget) break;
         s++;
     }
     return s;
-}
-
-// Kernel mapping (kernels.cu): one thread per query while blocks + table are (mostly) L2-resident,
-// a lane pair per query -- one coalesced 64-byte request per block -- once they live in HBM.
-bool lives_in_hbm(int device, uint64_t index_bytes) {
-    int l2 = 0;
-    if (cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, device) != cudaSuccess || l2 <= 0) l2 = 96 << 20;
-    return index_bytes > 2ull * (uint64_t)l2;
-}
-
-int pick_lanes(int device, uint64_t index_bytes, int requested) {
-    if (requested == 1 || requested == 2) return requested;
-    if (const char *env = getenv("MSBWT_LANES")) return atoi(env) == 2 ? 2 : 1;
-    return lives_in_hbm(device, index_bytes) ? 2 : 1;
-}
-
-// The pair image (layout.h: one 128-byte line per two steps) pays off once the index lives in HBM;
-// an L2-resident index is served faster by the 64-byte one-step blocks (smaller footprint).
-bool pick_pair(int device, uint64_t index_bytes, int requested) {
-    if (requested == 0 || requested == 1) return requested == 1;
-    if (const char *env = getenv("MSBWT_PAIR_INDEX")) return atoi(env) != 0;
-    return lives_in_hbm(device, index_bytes);
 }
 
 int build_pair(msbwt_index *idx, Replica &rep, uint8_t **keep_codes = nullptr) {
@@ -236,39 +309,6 @@ int build_pair(msbwt_index *idx, Replica &rep, uint8_t **keep_codes = nullptr) {
     return MSBWT_OK;
 }
 
-// The quad image (layout.h: one 32-byte sector per FOUR steps, 256 * N / 7 bytes) halves the line fills
-// of the pair image again.  Automatic choice: the one-step index does not fit L2 (measured on the
-// 151 Msymbol BWT, 1.7 x L2: 10.2 G queries/s through quad sectors + a depth-15 table in HBM against 7.3 G
-// through the mostly L2-resident one-step blocks), the image stays below 64 GB (measured,
-// profiles/r1_gather_big.json: random reads keep 93 % of their rate over a 64 GB buffer and lose three
-// quarters of it over 128 GB) and below half of the free device memory.  When the oct image will sit on top
-// (`with_oct`: 32-bit positions, not switched off) the quad image only serves fallbacks and remainders, the
-// randomly read footprint is the oct image + the suffix table, and the quad image may take up to 65 % of the
-// free memory (110 GB for configs[4]'s 3.02 Gsymbol BWT).
-bool pick_quad(int device, uint64_t index_bytes, uint64_t total, int requested, int pair_requested, bool with_oct) {
-    if (requested == 0 || requested == 1) return requested == 1;
-    if (pair_requested == 0 || pair_requested == 1) return false;  // the caller pinned the layout
-    if (const char *env = getenv("MSBWT_QUAD_INDEX")) return atoi(env) != 0;
-    int l2 = 0;
-    if (cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, device) != cudaSuccess || l2 <= 0) l2 = 96 << 20;
-    if (index_bytes <= (uint64_t)l2) return false;
-    size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return false;
-    const uint64_t need = quad_image_bytes(total);
-    if (with_oct) return need <= free_b / 100 * 65;
-    return need <= (64ull << 30) && need <= free_b / 2;
-}
-
-// The oct image (layout.h: one 128-byte line per kOctSyms = 10 steps) rides on the quad image: same
-// automatic condition, 32-bit positions only; it may take the device memory left after the quad image minus its
-// own build scratch and 8 GB (the builder picks coarser buckets, or builds nothing, beyond that).
-bool pick_oct(const IndexView &view, int requested) {
-    if (index_is_wide(view)) return false;
-    if (requested == 0 || requested == 1) return requested == 1;
-    if (const char *env = getenv("MSBWT_OCT_INDEX")) return atoi(env) != 0;
-    return true;
-}
-
 void build_trace(const char *what) {
     static const bool on = getenv("MSBWT_TRACE") != nullptr;
     if (!on) return;
@@ -277,38 +317,16 @@ void build_trace(const char *what) {
     fprintf(stderr, "[msbwt] index build: %s (%.1f GB of device memory free)\n", what, (double)free_b / 1e9);
 }
 
-int env_int(const char *name, int fallback) {
-    const char *e = getenv(name);
-    return e ? atoi(e) : fallback;
-}
-
-// The environment fills the image knobs the caller left unset (-1, or 0 for the shifts), before any builder reads them
-void fill_from_env(Options &o) {
-    if (o.keep_quad == -1) o.keep_quad = env_int("MSBWT_KEEP_QUAD", -1);
-    if (o.fin == -1) o.fin = env_int("MSBWT_FINAL_INDEX", -1);
-    if (!o.fin_shift) o.fin_shift = env_int("MSBWT_FINAL_BUCKET_SHIFT", 16);
-    if (!o.fin_lb) o.fin_lb = env_int("MSBWT_FINAL_LINES_LOG2", 0);
-    if (!o.oct_shift) o.oct_shift = env_int("MSBWT_OCT_BUCKET_SHIFT", 0);
-}
-
-// Lines per final-step bucket: 2^13, 16 bytes per symbol (0.8 % of the read-sampled 31-mers find their line overflowed
-// and take the oct steps), when that fits 30 % of the device (48 GB at 3.02 Gsymbols), else 2^12, 8 bytes per symbol
-// (6.5 %)
-int fin_lines_log2(const Options &opt, uint64_t N, uint64_t device_bytes) {
-    if (opt.fin_lb) return opt.fin_lb;
-    return fin_image_bytes(N, opt.fin_shift, 13) <= device_bytes / 10 * 3 ? 13 : 12;
-}
-
 // The final-step lines on top of the oct image, from the 20-symbol codes (owned by the builder from here on).  Running out
 // of device memory leaves the index without this image unless the caller required it.
-int build_fin(Replica &rep, const Options &opt, uint64_t *codes20, int flb) {
+int build_fin(Replica &rep, const Layout &p, uint64_t *codes20) {
     std::string why;
     int n = 0;
-    int rc = build_fin_lines_on_device(rep.device, rep.view.total, codes20, opt.fin_shift, flb, rep.fin, why, &n);
+    int rc = build_fin_lines_on_device(rep.device, rep.view.total, codes20, p.fin_shift, p.fin_lb, rep.fin, why, &n);
     g_launches += (uint64_t)n;
     if (rc != MSBWT_OK) {
         free_fin_image(rep.fin);
-        if (rc == MSBWT_ENOMEM && opt.fin != 1) { cudaGetLastError(); return MSBWT_OK; }
+        if (rc == MSBWT_ENOMEM && !p.fin_required) { cudaGetLastError(); return MSBWT_OK; }
         return fail(rc, why);
     }
     refresh_view(rep);
@@ -321,34 +339,25 @@ int build_fin(Replica &rep, const Options &opt, uint64_t *codes20, int flb) {
 //   pair image + pair codes -> quad image + quad codes (pair image dropped) -> 10-symbol codes (quad codes dropped)
 //   -> 20-symbol codes -> [quad image dropped unless it is kept] -> oct lines -> final-step lines.
 // The quad image is what the builders walk LF^4 with; afterwards it only serves remainders of 4..9 symbols and the
-// rare fallbacks (overflowed line, range over two buckets) of the oct kernel, which one-symbol ranks answer as
-// well.  It is kept when everything fits comfortably (`keep_quad` -1: quad + 40 B/symbol for the other two images
-// within 70 % of the device memory: 55 GB at 1.51 Gsymbols), dropped otherwise (110 GB at 3.02 Gsymbols) -- and
+// rare fallbacks (overflowed line, range over two buckets) of the oct kernel.  It is dropped unless `keep_quad` -- and
 // always kept when there is no oct image on top (N >= 2^32, or switched off): then it is the search image.
-int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
+int build_multi_step(msbwt_index *idx, Replica &rep, const Layout &p) {
     uint8_t *codes2 = nullptr;
     if (int rc = build_pair(idx, rep, &codes2); rc != MSBWT_OK) return rc;
     DeviceGuard guard(rep.device);
     DevicePtr<uint8_t> codes2_owner(codes2);
-    const bool want_oct = pick_oct(rep.view, opt.oct);
-    const bool want_fin = want_oct && opt.fin != 0;
     uint16_t *codes4 = nullptr;
     std::string why;
     int n = 0;
     build_trace("quad image");
-    int rc = build_quad_image_on_device(rep.device, rep.view, codes2, rep.quad, why, &n, want_oct ? &codes4 : nullptr);
+    int rc = build_quad_image_on_device(rep.device, rep.view, codes2, rep.quad, why, &n, p.oct ? &codes4 : nullptr);
     g_launches += (uint64_t)n;
     free_pair_image(rep.pair);
     if (rc != MSBWT_OK) { free_quad_image(rep.quad); if (codes4) cudaFree(codes4); return fail(rc, why); }
     refresh_view(rep);
-    if (!want_oct) return MSBWT_OK;
+    if (!p.oct) return MSBWT_OK;
 
     const uint64_t N = rep.view.total;
-    size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { free_b = 0; total_b = 0; }
-    int keep_quad = opt.keep_quad;
-    if (keep_quad == -1) keep_quad = quad_image_bytes(N) + 40 * N <= (uint64_t)total_b / 10 * 7 ? 1 : 0;
-
     // 10-symbol codes (4 B per position), then 20-symbol codes (8 B per position): both walk LF^4 through the quad image
     uint32_t *codes10 = nullptr;
     n = 0;
@@ -358,13 +367,12 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
     if (rc != MSBWT_OK) return fail(rc, why);
     DevicePtr<uint32_t> codes10_owner(codes10);
     codes2_owner.reset();
-    const int flb = fin_lines_log2(opt, N, total_b);
     uint64_t *codes20 = nullptr;
-    if (want_fin) {
+    if (p.fin) {
         n = 0;
         rc = build_fin_codes_on_device(rep.device, rep.view, codes10, &codes20, why, &n);
         g_launches += (uint64_t)n;
-        if (rc == MSBWT_ENOMEM && opt.fin != 1) {  // no room for the codes: the index works without this image
+        if (rc == MSBWT_ENOMEM && !p.fin_required) {  // no room for the codes: the index works without this image
             cudaGetLastError();
             codes20 = nullptr;
         } else if (rc != MSBWT_OK) {
@@ -372,7 +380,7 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
         }
     }
     DevicePtr<uint64_t> codes20_owner(codes20);
-    if (!keep_quad) {
+    if (!p.keep_quad) {
         build_trace("dropping the quad image");
         free_quad_image(rep.quad);
         refresh_view(rep);
@@ -381,13 +389,13 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
     // oct lines: what is left after the final-step lines, their sort scratch (about 16 B per position, of which the
     // 12 B per position of the two code arrays are free again by then) and 8 GB for the suffix table and the query
     // pipeline; the builder picks coarser buckets, or builds nothing, beyond that
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) free_b = 0;
-    const uint64_t fin_need = codes20 ? fin_image_bytes(N, opt.fin_shift, flb) + 4 * N : 0;
-    const uint64_t reserve = fin_need + (opt.oct == 1 ? 0 : (8ull << 30));
+    const uint64_t free_b = free_bytes_now();
+    const uint64_t fin_need = codes20 ? fin_image_bytes(N, p.fin_shift, p.fin_lb) + 4 * N : 0;
+    const uint64_t reserve = fin_need + (p.oct_required ? 0 : (8ull << 30));
     const uint64_t budget = free_b > reserve ? free_b - reserve : 0;
     n = 0;
     build_trace("oct lines");
-    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, opt.oct_shift, budget, rep.oct, why, &n);
+    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, p.oct_shift, budget, rep.oct, why, &n);
     g_launches += (uint64_t)n;
     codes10_owner.reset();
     if (rc != MSBWT_OK) { free_oct_image(rep.oct); return fail(rc, why); }
@@ -396,7 +404,7 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
         return MSBWT_OK;
     }
     refresh_view(rep);
-    if (codes20) return build_fin(rep, opt, codes20_owner.release(), flb);
+    if (codes20) return build_fin(rep, p, codes20_owner.release());
     build_trace("multi-step images done");
     return MSBWT_OK;
 }
@@ -407,16 +415,16 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Options &opt) {
 // blocks (oct_builder.cu build_oct_codes_by_walk, fin_builder.cu build_fin_codes_by_walk), and the search kernel
 // (wide_kernels.cu) takes remainders and fallbacks as one-symbol steps.
 //   10-symbol codes -> oct lines -> 20-symbol codes (10-symbol codes dropped) -> final-step lines.
-// `required` false (automatic choice): running out of device memory leaves the index without these images
-// (*built = false, MSBWT_OK) and the caller falls back to the pair image.
-int build_multi_step_wide(Replica &rep, const Options &opt, bool required, bool *built) {
+// Unless `oct_required`, running out of device memory leaves the index without these images (*built = false,
+// MSBWT_OK) and the caller falls back to the quad or pair route.
+int build_multi_step_wide(Replica &rep, const Layout &p, bool *built) {
     *built = false;
     DeviceGuard guard(rep.device);
     const uint64_t N = rep.view.total;
     std::string why;
     int n = 0;
     auto soft = [&](int rc) {  // out of memory on an automatic build: the index works without these images
-        if (rc == MSBWT_ENOMEM && !required) { cudaGetLastError(); return true; }
+        if (rc == MSBWT_ENOMEM && !p.oct_required) { cudaGetLastError(); return true; }
         return false;
     };
 
@@ -427,29 +435,27 @@ int build_multi_step_wide(Replica &rep, const Options &opt, bool required, bool 
     if (rc != MSBWT_OK) return soft(rc) ? MSBWT_OK : fail(rc, why);
     DevicePtr<uint32_t> codes10_owner(codes10);
 
-    size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { free_b = 0; total_b = 0; }
-    const int flb = fin_lines_log2(opt, N, total_b);
+    const uint64_t free_b = free_bytes_now();
     // what the final-step image will need after the oct lines exist: its lines, the 20-symbol codes (8 B per
     // position) and the run records + sort scratch (4 B per position once the codes are gone)
-    const uint64_t fin_need = opt.fin != 0 ? fin_image_bytes(N, opt.fin_shift, flb) + 12 * N : 0;
-    const uint64_t reserve = fin_need + (opt.oct == 1 ? 0 : (8ull << 30));
+    const uint64_t fin_need = p.fin ? fin_image_bytes(N, p.fin_shift, p.fin_lb) + 12 * N : 0;
+    const uint64_t reserve = fin_need + (p.oct_required ? 0 : (8ull << 30));
     const uint64_t budget = free_b > reserve ? free_b - reserve : 0;
     n = 0;
     build_trace("oct lines");
-    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, opt.oct_shift, budget, rep.oct, why, &n);
+    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, p.oct_shift, budget, rep.oct, why, &n);
     g_launches += (uint64_t)n;
     if (rc != MSBWT_OK) {
         free_oct_image(rep.oct);
         return soft(rc) ? MSBWT_OK : fail(rc, why);
     }
     if (!rep.oct.lines) {
-        if (required) return fail(MSBWT_ENOMEM, "no room for the oct image of this index");
+        if (p.oct_required) return fail(MSBWT_ENOMEM, "no room for the oct image of this index");
         return MSBWT_OK;
     }
     refresh_view(rep);
     *built = true;
-    if (opt.fin == 0) return MSBWT_OK;
+    if (!p.fin) return MSBWT_OK;
 
     uint64_t *codes20 = nullptr;
     n = 0;
@@ -457,22 +463,10 @@ int build_multi_step_wide(Replica &rep, const Options &opt, bool required, bool 
     g_launches += (uint64_t)n;
     codes10_owner.reset();
     if (rc != MSBWT_OK) {
-        if (rc == MSBWT_ENOMEM && opt.fin != 1) { cudaGetLastError(); return MSBWT_OK; }
+        if (rc == MSBWT_ENOMEM && !p.fin_required) { cudaGetLastError(); return MSBWT_OK; }
         return fail(rc, why);
     }
-    return build_fin(rep, opt, codes20, flb);
-}
-
-// Automatic choice for an index with 64-bit positions: it lives in HBM, the caller pinned no other layout, and the
-// two images at their coarsest settings plus the builders' scratch fit the free device memory.
-bool pick_wide_oct(int device, uint64_t index_bytes, uint64_t total, const Options &opt) {
-    if (opt.oct == 0 || opt.oct == 1) return opt.oct == 1;
-    if (const char *env = getenv("MSBWT_OCT_INDEX")) { if (atoi(env) == 0) return false; }
-    if (opt.pair != -1 || opt.quad != -1 || getenv("MSBWT_PAIR_INDEX") || getenv("MSBWT_QUAD_INDEX")) return false;
-    if (!lives_in_hbm(device, index_bytes) || (total >> 40) != 0) return false;
-    size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return false;
-    return oct_image_bytes(total, kOctMaxShift) + fin_image_bytes(total, 16, 12) + 12 * total + (8ull << 30) <= free_b;
+    return build_fin(rep, p, codes20);
 }
 
 int build_suffix_table(Replica &rep, int s) {
@@ -523,8 +517,6 @@ int build_suffix_table(Replica &rep, int s) {
 
 msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices, int ndev, Options opt, int *err) {
     fill_from_env(opt);
-    const uint32_t sb_shift = opt.sb_shift;
-    const int table_s = opt.table_s;
     g_last_error.clear();
     int rc;
     std::string why;
@@ -532,46 +524,35 @@ msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices,
     if ((rc = validate_rle(rle, len, why)) != MSBWT_OK) {
         fail(rc, why);
     } else {
-        rc = build_replicas_on_device(idx.get(), rle, len, sb_shift, devices, ndev);
+        rc = build_replicas_on_device(idx.get(), rle, len, opt.sb_shift, devices, ndev);
     }
     if (rc == MSBWT_OK) {
-        bool explicit_s = false;
-        const int s0 = pick_table_s(idx->total, table_s, &explicit_s);
-        const bool wide = index_is_wide(idx->reps[0]->view);
-        const uint64_t one_step_bytes = replica_bytes(*idx->reps[0]) + (s0 > 0 ? (1ull << (2 * s0)) * (wide ? 16 : 8) : 0);
         rc = for_each_replica_slot(idx->reps.size(), [&](size_t slot) -> int {
-            auto &rep = idx->reps[slot];
-            int s = s0;
-            bool quad;
+            Replica &rep = *idx->reps[slot];
+            DeviceGuard guard(rep.device);
+            const uint64_t N = rep.view.total;
+            const bool wide = index_is_wide(rep.view);
+            // Planned from the device's free memory before any optional image exists.  A wide build that runs out of
+            // memory frees everything it allocated, and cudaMalloc / cudaFree keep no cache, so the quad route after it
+            // meets the same free memory.
+            const Layout p = plan_layout(opt, N, wide, replica_bytes(rep), device_sizes(rep.device));
             bool wide_oct = false;
-            {
-                DeviceGuard guard(rep->device);
-                if (wide && pick_wide_oct(rep->device, one_step_bytes, idx->total, opt)) {
-                    if (int r = build_multi_step_wide(*rep, opt, opt.oct == 1, &wide_oct); r != MSBWT_OK) return r;
-                }
-                const char *oct_env = getenv("MSBWT_OCT_INDEX");
-                const bool with_oct = idx->total < (1ull << 32) && !index_is_wide(rep->view) && opt.oct != 0 &&
-                                      (opt.oct == 1 || !oct_env || atoi(oct_env) != 0);
-                quad = !wide_oct && (opt.oct == 1 || pick_quad(rep->device, one_step_bytes, idx->total, opt.quad, opt.pair, with_oct));
+            if (p.wide_oct) {
+                if (int r = build_multi_step_wide(rep, p, &wide_oct); r != MSBWT_OK) return r;
             }
-            if (wide_oct) {
-                if (!explicit_s) {
-                    DeviceGuard guard(rep->device);
-                    s = std::min(deepen_table_for_hbm(s0, idx->reps[0]->view.nblocks * kBlockBytes + oct_image_bytes(idx->total, rep->oct.shift), 16), kOctAutoTableS);
-                }
-            } else if (quad || pick_pair(rep->device, one_step_bytes, opt.pair)) {
-                if (int r = quad ? build_multi_step(idx.get(), *rep, opt) : build_pair(idx.get(), *rep); r != MSBWT_OK) return r;
-                if (!explicit_s && (quad || lives_in_hbm(rep->device, one_step_bytes))) {
-                    DeviceGuard guard(rep->device);
-                    const uint64_t multi = quad ? quad_image_bytes(idx->total) : rep->view.npair * kPairBytes;
-                    s = deepen_table_for_hbm(s0, idx->reps[0]->view.nblocks * kBlockBytes + multi, wide ? 16 : 8);
-                    // with ten symbols per oct line a 31-mer wants the depth-11 level (33 MB, L2-resident): the
-                    // deepest of the four kept levels need not go beyond 14 (2.1 GB instead of 8.6 GB at 15)
-                    if (rep->view.oct) s = std::min(s, kOctAutoTableS);
-                }
+            if (!wide_oct && (p.quad || p.pair)) {
+                if (int r = p.quad ? build_multi_step(idx.get(), rep, p) : build_pair(idx.get(), rep); r != MSBWT_OK) return r;
             }
-            if (int r = build_suffix_table(*rep, s); r != MSBWT_OK) return r;
-            rep->lanes = pick_lanes(rep->device, one_step_bytes, opt.lanes);
+            int s = p.table_s;
+            if (!p.explicit_s && (wide_oct || p.quad || (p.pair && p.hbm))) {
+                const uint64_t multi = wide_oct ? oct_image_bytes(N, rep.oct.shift) : p.quad ? quad_image_bytes(N) : rep.view.npair * kPairBytes;
+                s = deepen_table_for_hbm(s, rep.view.nblocks * kBlockBytes + multi, wide ? 16 : 8, free_bytes_now());
+                // with ten symbols per oct line a 31-mer wants the depth-11 level (33 MB, L2-resident): the
+                // deepest of the four kept levels need not go beyond 14 (2.1 GB instead of 8.6 GB at 15)
+                if (rep.view.oct) s = std::min(s, kOctAutoTableS);
+            }
+            if (int r = build_suffix_table(rep, s); r != MSBWT_OK) return r;
+            rep.lanes = p.lanes;
             return MSBWT_OK;
         });
     }
@@ -689,8 +670,7 @@ extern "C" uint64_t msbwt_oct_overflow_lines(const msbwt_index *idx) { return (i
 extern "C" uint64_t msbwt_oct_overflow_occurrences(const msbwt_index *idx) { return (idx && !idx->reps.empty()) ? idx->reps[0]->oct.overflow_occurrences : 0; }
 extern "C" uint64_t msbwt_oct_runs(const msbwt_index *idx) { return (idx && !idx->reps.empty()) ? idx->reps[0]->oct.runs : 0; }
 extern "C" int msbwt_oct_symbols(void) { return kOctSyms; }
-// final-step image (layout.h): built by default on top of the oct image; final_index = 0 (or MSBWT_FINAL_INDEX=0) turns
-// it off
+// final-step image (layout.h): built by default on top of the oct image; final_index = 0 turns it off
 extern "C" int msbwt_final_index(const msbwt_index *idx) {
     return (idx && !idx->reps.empty() && idx->reps[0]->view.fin) ? 1 : 0;
 }
@@ -716,6 +696,21 @@ extern "C" int msbwt_debug_table_depth(uint32_t k, uint32_t table_s, uint32_t st
     if (steps == (uint32_t)kOctSyms) return (int)oct_table_depth(k, table_s);
     if (steps == 1 || steps == 2 || steps == 4) return (int)acgt_table_depth(k, table_s, steps);
     return -1;
+}
+// the layout policy on its own (no device needed): what create plans for a replica from these options, the environment
+// and these sizes
+extern "C" int msbwt_debug_plan_layout(const msbwt_options *opts, uint64_t total, int wide, uint64_t block_bytes,
+                                       uint64_t l2_bytes, uint64_t free_bytes, uint64_t device_bytes, int32_t *plan, int nplan) {
+    g_last_error.clear();
+    Options o;
+    if (int rc = parse_options(opts, o); rc != MSBWT_OK) return rc;
+    fill_from_env(o);
+    const Layout p = plan_layout(o, total, wide != 0, block_bytes, DeviceSizes{l2_bytes, free_bytes, device_bytes});
+    const int32_t v[] = {p.table_s,   p.explicit_s,   p.hbm,          p.wide_oct, p.quad,  p.oct,       p.fin,      p.pair,
+                         p.keep_quad, p.oct_required, p.fin_required, p.fin_lb,   p.lanes, p.oct_shift, p.fin_shift};
+    if (!plan || nplan < (int)std::size(v)) return fail(MSBWT_EINVAL, "plan_layout: plan must hold 15 values");
+    std::copy(std::begin(v), std::end(v), plan);
+    return MSBWT_OK;
 }
 extern "C" int msbwt_table_depth_for_k(const msbwt_index *idx, uint32_t k) {
     return (idx && !idx->reps.empty()) ? (int)list_a_table_depth(idx->reps[0]->view, k) : 0;

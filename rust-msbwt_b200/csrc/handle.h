@@ -95,7 +95,7 @@ struct Replica {
     QuadImage quad;            // 32-byte quad sectors (layout.h), when the index lives in HBM and the image fits
     OctImage oct;              // 128-byte oct lines (layout.h), next to the quad image when positions are 32-bit
     FinImage fin;              // final-step lines (layout.h), built by default on top of the oct image; final_index = 0
-                               // (or MSBWT_FINAL_INDEX=0) turns them off
+                               // turns them off
     int lanes = 1;           // kernel mapping: 1 = thread per query, 2 = lane pair per query (kernels.cu)
     uint64_t *d_cbase = nullptr;
     IndexView view{};

@@ -127,6 +127,7 @@ def load_library():
         "msbwt_oct_symbols": (i32, []),
         "msbwt_table_depth_for_k": (i32, [vp, u32]),
         "msbwt_debug_table_depth": (i32, [u32, u32, u32]),
+        "msbwt_debug_plan_layout": (i32, [C.POINTER(Options), u64, i32, u64, u64, u64, u64, vp, i32]),
         "msbwt_count_kmers_u64": (i32, [vp, vp, u32, u64, vp]),
         "msbwt_count_kmers_fixed_u32": (i32, [vp, vp, u32, u64, vp]),
         "msbwt_count_kmers_u64_u32": (i32, [vp, vp, u32, u64, vp]),
@@ -175,7 +176,7 @@ EXPORTED_SYMBOLS = (
     "msbwt_index_create_from_rle", "msbwt_index_create_from_npy", "msbwt_index_create_ex", "msbwt_index_create_opts",
     "msbwt_index_create_from_npy_opts", "msbwt_count_kmers_packed_stats_device", "msbwt_seed_kmers_u64_device", "msbwt_debug_pack_stats", "msbwt_count_kmers_fixed_u32", "msbwt_count_kmers_u64_u32",
     "msbwt_pair_index", "msbwt_debug_copy_pair_image", "msbwt_quad_index", "msbwt_debug_copy_quad_image", "msbwt_oct_index", "msbwt_oct_overflow_lines",
-    "msbwt_oct_overflow_occurrences", "msbwt_oct_runs", "msbwt_oct_bucket_shift", "msbwt_oct_symbols", "msbwt_table_depth_for_k", "msbwt_debug_table_depth", "msbwt_count_kmers_u64", "msbwt_final_index", "msbwt_debug_copy_final_image",
+    "msbwt_oct_overflow_occurrences", "msbwt_oct_runs", "msbwt_oct_bucket_shift", "msbwt_oct_symbols", "msbwt_table_depth_for_k", "msbwt_debug_table_depth", "msbwt_debug_plan_layout", "msbwt_count_kmers_u64", "msbwt_final_index", "msbwt_debug_copy_final_image",
     "msbwt_debug_copy_oct_image", "msbwt_constrain_ranges_fanout", "msbwt_constrain_ranges_fanout_device",
     "msbwt_count_read_kmers", "msbwt_last_transfer_bytes", "msbwt_host_pack_threads",
     "msbwt_debug_host_pack",

@@ -59,6 +59,7 @@ extern "C" {
     pub fn msbwt_oct_symbols() -> c_int;
     pub fn msbwt_table_depth_for_k(idx: *const msbwt_index, k: u32) -> c_int;
     pub fn msbwt_debug_table_depth(k: u32, table_s: u32, steps: u32) -> c_int;
+    pub fn msbwt_debug_plan_layout(opts: *const msbwt_options, total: u64, wide: c_int, block_bytes: u64, l2_bytes: u64, free_bytes: u64, device_bytes: u64, plan: *mut i32, nplan: c_int) -> c_int;
     pub fn msbwt_final_index(idx: *const msbwt_index) -> c_int;
     pub fn msbwt_debug_copy_final_image(idx: *const msbwt_index, slot: c_int, nlines: *mut u64, bucket_shift: *mut u32, lines_log2: *mut u32, overflow_lines: *mut u64, lines: *mut u32) -> c_int;
     pub fn msbwt_count_kmers_u64(idx: *const msbwt_index, kmers: *const u64, k: u32, n: u64, out: *mut u64) -> c_int;
