@@ -401,6 +401,31 @@ void msbwt_buffer_free(uint8_t *p);
  * *kmers / *counts are NULL. */
 int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist, uint32_t nbins,
                         uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers);
+/* The canonical k-mer spectrum: msbwt_kmer_spectrum with each k-mer counted on both strands, as `jellyfish count -C`
+ * and KMC count the reads.  For a k-mer X in msbwt_count_kmers_u64's encoding, rc(X) reverses its k 2-bit groups and
+ * maps each code c to 3 - c; canon(X) = min(X, rc(X)) as integers; the canonical count is
+ * C(X) = count_kmer(X) + count_kmer(rc(X)) when X != rc(X), and count_kmer(X) when X is its own reverse complement (a
+ * palindrome, possible for even k only).  S_c = { canon(X) : C(X) >= min_count }, each pair {X, rc(X)} once as its
+ * canonical member; *n_kmers = |S_c|, hist counts C over S_c with msbwt_kmer_spectrum's bin rules (the last bin holds
+ * C >= nbins - 1, bins below min_count and hist[0] are 0), and *kmers / *counts are S_c and its canonical counts.
+ * Every N-free k-window of every read adds exactly 1 to exactly one canonical k-mer, so for an index built from reads
+ * sum of c * hist[c] is the number of N-free k-windows, and reverse-complementing any subset of the reads before the
+ * index is built changes neither S_c, nor the counts, nor hist.  This differs from msbwt_count_read_kmers with
+ * strands == 2 on palindromes, which that call counts twice.  An index that already holds the reads' reverse
+ * complements gets every count doubled here: for such an index msbwt_kmer_spectrum already is the two-strand spectrum.
+ * Arguments, EINVAL cases (nothing written), ownership of the list (release each buffer with msbwt_buffer_free) and
+ * concurrency are msbwt_kmer_spectrum's.  The list is in a deterministic order (two calls return identical arrays);
+ * no other order is promised.
+ * The walk is msbwt_kmer_spectrum's with the k-mer values, pruned at ceil(min_count / 2) (a pair reaching min_count has
+ * a member counting at least that).  Its k-mers are staged on the device, 2^22 at a time, and each staged batch is
+ * resolved there: the count of every rc(X) comes from the query path, so the call reads whatever images
+ * msbwt_count_kmers_u64 reads (suffix table, oct and final-step images, one-step blocks), not only the one-step blocks.
+ * Device memory: the list mode of msbwt_kmer_spectrum at min_count ceil(min_count / 2) (also for the histogram alone),
+ * plus, per staged k-mer, 8 + 8 bytes for its reverse complement and that one's count, 1 flag byte and the query
+ * path's scratch of 20 bytes (28 with 64-bit positions): 155 MB (189 MB) for 2^22 staged k-mers, fewer when the index
+ * holds fewer than 2^22 * ceil(min_count / 2) symbols. */
+int msbwt_kmer_spectrum_canonical(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist,
+                                  uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers);
 
 /* ---- the data format either side of the path: src/bwt_converter.rs ----
  * convert_to_vec (:26-80): a text BWT over `$ACGNT` (newlines are skipped and do not end a run) -> msbwt RLE bytes

@@ -140,17 +140,20 @@ class RleBWT {
         return out;
     }
     // the k-mer spectrum (hist: nbins entries, the last one = count >= nbins - 1) and, with want_list, the k-mers with
-    // count >= min_count and their counts in co-lexicographic order (k <= 32; msbwt_count_kmers_u64's encoding)
+    // count >= min_count and their counts in co-lexicographic order (k <= 32; msbwt_count_kmers_u64's encoding);
+    // canonical: both strands, once per pair {X, rc X} (msbwt_kmer_spectrum_canonical; the list in no promised order)
     struct KmerSpectrum {
         std::vector<uint64_t> hist, kmers, counts;
         uint64_t n_kmers = 0;
     };
-    KmerSpectrum kmer_spectrum(uint32_t k, uint64_t min_count = 1, uint32_t nbins = 10001, bool want_list = false) const {
+    KmerSpectrum kmer_spectrum(uint32_t k, uint64_t min_count = 1, uint32_t nbins = 10001, bool want_list = false,
+                               bool canonical = false) const {
         KmerSpectrum out;
         out.hist.assign(nbins, 0);
         uint64_t *km = nullptr, *cn = nullptr;
-        check(msbwt_kmer_spectrum(h_, k, min_count, nbins ? out.hist.data() : nullptr, nbins, want_list ? &km : nullptr,
-                                  want_list ? &cn : nullptr, &out.n_kmers));
+        check((canonical ? msbwt_kmer_spectrum_canonical : msbwt_kmer_spectrum)(
+            h_, k, min_count, nbins ? out.hist.data() : nullptr, nbins, want_list ? &km : nullptr,
+            want_list ? &cn : nullptr, &out.n_kmers));
         if (km) {
             out.kmers.assign(km, km + out.n_kmers);
             out.counts.assign(cn, cn + out.n_kmers);

@@ -1102,8 +1102,8 @@ extern "C" int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const 
     return MSBWT_OK;
 }
 
-extern "C" int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist, uint32_t nbins,
-                                   uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
+static int kmer_spectrum_call(const msbwt_index *idx, bool canonical, uint32_t k, uint64_t min_count, uint64_t *hist,
+                              uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
     g_last_error.clear();
     if (!idx || idx->reps.empty()) return fail(MSBWT_EINVAL, "bad handle");
     if (!k || k > 32) return fail(MSBWT_EINVAL, "kmer_spectrum: k must be in 1..32");
@@ -1114,16 +1114,26 @@ extern "C" int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t 
     if (!kmers != !counts) return fail(MSBWT_EINVAL, "kmer_spectrum: kmers and counts must be both NULL or both set");
     *n_kmers = 0;
     if (kmers) *kmers = *counts = nullptr;
-    // replica 0's images are read-only after create; the call has its own stream and scratch, so it takes no lock and
-    // runs beside the query entry points
+    // replica 0's images are read-only after create; the call has its own stream and scratch (the canonical lookups
+    // too: no lane of the replica), so it takes no lock and runs beside the query entry points
     const Replica &rep = *idx->reps[0];
     DeviceGuard guard(rep.device);
     std::string why;
     int launches = 0;
-    const int rc = kmer_spectrum_on_device(rep.device, rep.view, k, min_count, hist, nbins, kmers, counts, n_kmers, why,
-                                           &launches);
+    const int rc = kmer_spectrum_on_device(rep.device, rep.view, rep.lanes, canonical, k, min_count, hist, nbins, kmers,
+                                           counts, n_kmers, why, &launches);
     g_launches += (uint64_t)launches;
     return rc == MSBWT_OK ? rc : fail(rc, why);
+}
+
+extern "C" int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist, uint32_t nbins,
+                                   uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
+    return kmer_spectrum_call(idx, false, k, min_count, hist, nbins, kmers, counts, n_kmers);
+}
+
+extern "C" int msbwt_kmer_spectrum_canonical(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist,
+                                             uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
+    return kmer_spectrum_call(idx, true, k, min_count, hist, nbins, kmers, counts, n_kmers);
 }
 
 extern "C" void msbwt_buffer_free(uint8_t *p) { free(p); }

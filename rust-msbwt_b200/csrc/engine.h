@@ -167,9 +167,11 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
 // ---- spectrum.cu: the k-mer spectrum of an index (one replica, on the current device): hist[nbins] (nbins may be 0)
 // and *n_kmers; when `kmers` is not null, also the k-mers with count >= min_count and their counts in co-lexicographic
 // order (*kmers, *counts: malloc'd host arrays the caller frees, null when there are none).  1 <= k <= 32, min_count >= 1.
-int kmer_spectrum_on_device(int device, const IndexView &ix, uint32_t k, uint64_t min_count, uint64_t *hist,
-                            uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers, std::string &why,
-                            int *launches);
+// `canonical`: the same over canonical pairs {X, rc X} (msbwt_kmer_spectrum_canonical), whose reverse-complement
+// lookups run on the query path with `lanes` (the replica's kernel mapping) on the call's own stream and scratch.
+int kmer_spectrum_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
+                            uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers,
+                            std::string &why, int *launches);
 
 // return an msbwt_status; on failure `why` explains
 int validate_rle(const uint8_t *rle, uint64_t len, std::string &why);

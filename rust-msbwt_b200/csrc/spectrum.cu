@@ -23,6 +23,13 @@
 //             of width >= min_count, so no buffer needs more than N / min_count entries either: small indexes
 //             allocate little.
 // Only the one-step blocks are read, which every index has, whatever other images it carries.
+//
+// Canonical spectrum (msbwt_kmer_spectrum_canonical): the same walk with the k-mer values, pruned at
+// ceil(min_count / 2), stages every k-mer Y it lists.  Each full staging buffer (and the last one) is resolved on the
+// device: rc(Y) of every staged Y, count_kmer(rc Y) through the query path (launch_seed_u64 + launch_count_packed,
+// so every image of the index is read there), then canonical_resolve_kernel keeps one member of every pair
+// {Y, rc Y} whose summed count reaches min_count.  Batches of up to 2^22 lookups keep the query kernels at their
+// bulk rate, where the walk's slices can be small.
 #include <cub/device/device_select.cuh>
 
 #include <algorithm>
@@ -129,6 +136,65 @@ spectrum_emit_kernel(IndexView ix, const Node<typename Pos<WIDE>::type, LIST> *_
         if (bins[t]) atomicAdd(&hist[t], (unsigned long long)bins[t]);
 }
 
+// rc(v) of a k-mer in msbwt_count_kmers_u64's encoding: every code c becomes 3 - c (= c ^ 3) and the k 2-bit groups
+// are reversed.  The bit reversal also swaps the two bits inside each group, so they are swapped back.
+__device__ __forceinline__ uint64_t revcomp_kmer(uint64_t v, uint32_t k) {
+    uint64_t r = __brevll(~v);
+    r = ((r >> 1) & 0x5555555555555555ull) | ((r & 0x5555555555555555ull) << 1);
+    return r >> (64 - 2 * k);  // the complemented zero bits above the k-mer end up below it
+}
+
+__global__ void __launch_bounds__(kCountThreads)
+canonical_revcomp_kernel(const uint64_t *__restrict__ kmers, uint32_t n, uint32_t k, uint64_t *__restrict__ rc) {
+    for (uint32_t i = blockIdx.x * kCountThreads + threadIdx.x; i < n; i += gridDim.x * kCountThreads)
+        rc[i] = revcomp_kmer(kmers[i], k);
+}
+
+// One staged batch of the canonical spectrum: Y = kmers[i] with count_kmer(Y) = counts[i] >= half, and
+// rc_counts[i] = count_kmer(rc Y).  Y stands for its pair {Y, rc Y} when it is the canonical member, or when rc Y
+// was not listed (count below half), so exactly one listed member of every pair stands for it.  Its canonical count
+// C is c_Y + c_rc, or c_Y alone for a palindrome.  With C >= min_count the pair is binned (as in spectrum_emit_kernel)
+// and counted, and with `keep` it is written in place over rc_kmers[i] / rc_counts[i] as (canon Y, C) and flagged
+// for the compaction.
+__global__ void __launch_bounds__(kCountThreads)
+canonical_resolve_kernel(const uint64_t *__restrict__ kmers, const uint64_t *__restrict__ counts, uint32_t n, uint32_t k,
+                         uint64_t half, uint64_t min_count, uint32_t nbins, uint32_t smem_bins,
+                         unsigned long long *__restrict__ hist, unsigned long long *__restrict__ n_kmers,
+                         uint64_t *__restrict__ rc_kmers, uint64_t *__restrict__ rc_counts, uint8_t *__restrict__ keep) {
+    extern __shared__ uint32_t bins[];
+    __shared__ uint32_t survivors[kCountThreads];
+    for (uint32_t t = threadIdx.x; t < smem_bins; t += blockDim.x) bins[t] = 0;
+    __syncthreads();
+    uint32_t mine = 0;
+    for (uint32_t i = blockIdx.x * kCountThreads + threadIdx.x; i < n; i += gridDim.x * kCountThreads) {
+        const uint64_t y = kmers[i], r = revcomp_kmer(y, k), c_rc = rc_counts[i];
+        const uint64_t c = y == r ? counts[i] : counts[i] + c_rc;
+        const bool ok = (y <= r || c_rc < half) && c >= min_count;
+        if (ok) {
+            mine++;
+            if (nbins) {
+                const uint32_t b = (uint32_t)min(c, (uint64_t)(nbins - 1));
+                if (b < smem_bins) atomicAdd(&bins[b], 1u);
+                else atomicAdd(&hist[b], 1ull);
+            }
+        }
+        if (keep) {
+            rc_kmers[i] = min(y, r);
+            rc_counts[i] = c;
+            keep[i] = ok;
+        }
+    }
+    survivors[threadIdx.x] = mine;  // summed through shared memory, as in spectrum_emit_kernel
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned long long sum = 0;
+        for (int t = 0; t < kCountThreads; t++) sum += survivors[t];
+        if (sum) atomicAdd(n_kmers, sum);
+    }
+    for (uint32_t t = threadIdx.x; t < smem_bins; t += blockDim.x)
+        if (bins[t]) atomicAdd(&hist[t], (unsigned long long)bins[t]);
+}
+
 #define S_TRY(expr)                                                                        \
     do {                                                                                   \
         cudaError_t e_ = (expr);                                                           \
@@ -174,16 +240,25 @@ uint64_t slice_parents() {
     return kSliceParents;
 }
 
+// `canonical` (LIST only): the walk lists every k-mer with count >= walk_min and stages it; each staged batch is then
+// resolved into canonical pairs (canonical_resolve_kernel), which alone are binned, counted and, with `kmers`, listed
 template <bool WIDE, bool LIST>
-int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count, uint64_t *hist, uint32_t nbins,
-                 uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers, std::string &why, int *launches) {
+int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
+                 uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers,
+                 std::string &why, int *launches) {
     using P = typename Pos<WIDE>::type;
     using NodeT = Node<P, LIST>;
     const uint64_t B = slice_parents();
-    // survivors of one slice: at most 4 per parent, and at most N / min_count (disjoint ranges of that width)
-    const uint64_t cap = std::max<uint64_t>(1, std::min<uint64_t>(4 * B, ix.total / min_count));
-    const uint64_t staging = LIST ? std::max(cap, std::min(kStagingKmers, ix.total / min_count)) : 0;
+    const bool want_list = kmers != nullptr;
+    // A pair with C >= min_count has a member with count >= ceil(min_count / 2); a pair whose members both count less
+    // has C <= min_count - 1.  So the canonical walk prunes at ceil(min_count / 2), exactly.
+    const uint64_t walk_min = canonical ? min_count / 2 + (min_count & 1) : min_count;  // (min_count + 1) / 2 wraps at 2^64 - 1
+    // survivors of one slice: at most 4 per parent, and at most N / walk_min (disjoint ranges of that width)
+    const uint64_t cap = std::max<uint64_t>(1, std::min<uint64_t>(4 * B, ix.total / walk_min));
+    const uint64_t staging = LIST ? std::max(cap, std::min(kStagingKmers, ix.total / walk_min)) : 0;
     const uint32_t smem_bins = std::min(nbins, kSmemBins);
+    // the walk's emission bins nothing in canonical mode: the resolve kernel does
+    const uint32_t emit_bins = canonical ? 0 : nbins, emit_smem_bins = canonical ? 0 : smem_bins;
 
     HostU64 out_kmers, out_counts;  // declared first: released after the stream has drained
     DeviceScratch scratch;
@@ -200,11 +275,22 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
     S_TRY(scratch.alloc(&d_keep, std::min(B, cap)));
     unsigned long long *d_hist = nullptr, *d_count = nullptr;
     S_TRY(scratch.alloc(&d_hist, std::max<uint32_t>(nbins, 1)));
-    S_TRY(scratch.alloc(&d_count, 2));  // [0] k-mers emitted, [1] survivors of the last compaction
+    // [0] k-mers emitted, [1] survivors of the last compaction, [2] k-mers the canonical walk staged
+    S_TRY(scratch.alloc(&d_count, 3));
     uint64_t *d_stage_kmers = nullptr, *d_stage_counts = nullptr;
     if (LIST) {
         S_TRY(scratch.alloc(&d_stage_kmers, staging));
         S_TRY(scratch.alloc(&d_stage_counts, staging));
+    }
+    // canonical: the staged k-mers' reverse complements and their counts (then the resolved pairs, in place), the
+    // resolve flags and the query path's scratch for one staged batch
+    uint64_t *d_rc_kmers = nullptr, *d_rc_counts = nullptr, *d_packed = nullptr;
+    uint8_t *d_resolved = nullptr;
+    if (canonical) {
+        S_TRY(scratch.alloc(&d_rc_kmers, staging));
+        S_TRY(scratch.alloc(&d_rc_counts, staging));
+        S_TRY(scratch.alloc(&d_resolved, staging));
+        S_TRY(scratch.alloc(&d_packed, packed_layout(ix, k, staging).total()));
     }
     size_t temp_bytes = 0, need = 0;
     const int max_items = (int)(4 * std::min(B, cap));
@@ -213,7 +299,8 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
     temp_bytes = std::max(temp_bytes, need);
     if (LIST) {
         S_TRY(cub::DeviceSelect::Flagged(nullptr, need, (const uint64_t *)nullptr, (const uint8_t *)nullptr,
-                                         (uint64_t *)nullptr, (unsigned long long *)nullptr, max_items, st.s));
+                                         (uint64_t *)nullptr, (unsigned long long *)nullptr,
+                                         canonical ? std::max(max_items, (int)staging) : max_items, st.s));
         temp_bytes = std::max(temp_bytes, need);
     }
     void *d_temp = nullptr;
@@ -224,13 +311,17 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
     root.h = (P)ix.total;
     S_TRY(cudaMemcpyAsync(level[0], &root, sizeof(NodeT), cudaMemcpyHostToDevice, st.s));
     S_TRY(cudaMemsetAsync(d_hist, 0, std::max<uint32_t>(nbins, 1) * sizeof(unsigned long long), st.s));
-    S_TRY(cudaMemsetAsync(d_count, 0, 2 * sizeof(unsigned long long), st.s));
+    S_TRY(cudaMemsetAsync(d_count, 0, 3 * sizeof(unsigned long long), st.s));
 
     const unsigned grid_expand = persistent_grid(device, (const void *)spectrum_expand_kernel<WIDE, LIST>, kCountThreads,
                                                  std::min(B, cap), kCountThreads);
     const unsigned grid_emit = persistent_grid(device, (const void *)spectrum_emit_kernel<WIDE, LIST>, kCountThreads,
                                                std::min(B, cap), kCountThreads);
-    const size_t emit_smem = std::max<uint32_t>(smem_bins, 1) * sizeof(uint32_t);
+    const unsigned grid_resolve = canonical ? persistent_grid(device, (const void *)canonical_resolve_kernel,
+                                                              kCountThreads, staging, kCountThreads) : 0;
+    const size_t emit_smem = std::max<uint32_t>(emit_smem_bins, 1) * sizeof(uint32_t);
+    const size_t resolve_smem = std::max<uint32_t>(smem_bins, 1) * sizeof(uint32_t);
+    const bool with_b = canonical && packed_batch_needs_list_b(ix, k);
     std::vector<uint64_t> fill(k, 0), next(k, 0);
     fill[0] = 1;
     uint64_t staged = 0, listed = 0;
@@ -247,6 +338,35 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
         staged = 0;
         return MSBWT_OK;
     };
+    // canonical: count the staged k-mers' reverse complements on the query path, resolve the pairs, and with the list
+    // compact the emitted ones into the staging buffers for flush()
+    auto resolve = [&]() -> int {
+        if (!staged) return MSBWT_OK;
+        const uint32_t n = (uint32_t)staged;
+        staged = 0;
+        const unsigned g = std::min<unsigned>(grid_resolve, (n + kCountThreads - 1) / kCountThreads);
+        canonical_revcomp_kernel<<<g, kCountThreads, 0, st.s>>>(d_stage_kmers, n, k, d_rc_kmers);
+        S_TRY(cudaGetLastError());
+        S_TRY(launch_seed_u64(ix, d_rc_kmers, k, n, d_packed, d_rc_counts, st.s));
+        S_TRY(launch_count_packed(device, ix, lanes, d_packed, k, n, d_rc_counts, st.s, launches, with_b));
+        canonical_resolve_kernel<<<g, kCountThreads, resolve_smem, st.s>>>(
+            d_stage_kmers, d_stage_counts, n, k, walk_min, min_count, nbins, smem_bins, d_hist, d_count, d_rc_kmers,
+            d_rc_counts, want_list ? d_resolved : nullptr);
+        S_TRY(cudaGetLastError());
+        if (launches) *launches += 3;  // reverse complements, seed, resolve
+        if (!want_list) return MSBWT_OK;
+        S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const uint64_t *)d_rc_kmers, (const uint8_t *)d_resolved,
+                                         d_stage_kmers, d_count + 1, (int)n, st.s));
+        S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const uint64_t *)d_rc_counts, (const uint8_t *)d_resolved,
+                                         d_stage_counts, d_count + 1, (int)n, st.s));
+        if (launches) *launches += 4;
+        unsigned long long emitted = 0;
+        S_TRY(cudaMemcpyAsync(&emitted, d_count + 1, sizeof(emitted), cudaMemcpyDeviceToHost, st.s));
+        S_TRY(cudaStreamSynchronize(st.s));
+        staged = emitted;
+        return flush();
+    };
+    auto drain = [&]() { return canonical ? resolve() : flush(); };
     for (;;) {
         int d = (int)k - 1;
         while (d >= 0 && next[d] == fill[d]) d--;
@@ -258,7 +378,7 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
         const unsigned grid = std::min<unsigned>(grid_expand, (m + kCountThreads - 1) / kCountThreads);
         if ((uint32_t)d + 1 < k) {
             NodeT *children = (NodeT *)d_children;
-            spectrum_expand_kernel<WIDE, LIST><<<grid, kCountThreads, 0, st.s>>>(ix, slice, m, shift, min_count, children, d_keep);
+            spectrum_expand_kernel<WIDE, LIST><<<grid, kCountThreads, 0, st.s>>>(ix, slice, m, shift, walk_min, children, d_keep);
             S_TRY(cudaGetLastError());
             S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const NodeT *)children, (const uint8_t *)d_keep,
                                              level[d + 1], d_count + 1, (int)(4 * m), st.s));
@@ -272,13 +392,14 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
             uint64_t *ck = (uint64_t *)d_children, *cc = ck + 4 * (uint64_t)m;
             const unsigned g = std::min<unsigned>(grid_emit, (m + kCountThreads - 1) / kCountThreads);
             spectrum_emit_kernel<WIDE, LIST><<<g, kCountThreads, emit_smem, st.s>>>(
-                ix, slice, m, shift, min_count, nbins, smem_bins, d_hist, d_count, ck, cc, d_keep);
+                ix, slice, m, shift, walk_min, emit_bins, emit_smem_bins, d_hist, canonical ? d_count + 2 : d_count, ck, cc,
+                d_keep);
             S_TRY(cudaGetLastError());
             if (launches) (*launches)++;
             if (LIST) {
                 const uint64_t most = std::min<uint64_t>(4 * (uint64_t)m, cap);  // survivors this slice can have
                 if (staged + most > staging)
-                    if (int rc = flush(); rc != MSBWT_OK) return rc;
+                    if (int rc = drain(); rc != MSBWT_OK) return rc;
                 S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const uint64_t *)ck, (const uint8_t *)d_keep,
                                                  d_stage_kmers + staged, d_count + 1, (int)(4 * m), st.s));
                 S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const uint64_t *)cc, (const uint8_t *)d_keep,
@@ -292,17 +413,17 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
         }
     }
     if (LIST)
-        if (int rc = flush(); rc != MSBWT_OK) return rc;
+        if (int rc = drain(); rc != MSBWT_OK) return rc;
     unsigned long long total_kmers = 0;
     S_TRY(cudaMemcpyAsync(&total_kmers, d_count, sizeof(total_kmers), cudaMemcpyDeviceToHost, st.s));
     if (nbins) S_TRY(cudaMemcpyAsync(hist, d_hist, nbins * sizeof(uint64_t), cudaMemcpyDeviceToHost, st.s));
     S_TRY(cudaStreamSynchronize(st.s));
-    if (LIST && listed != total_kmers) {
+    if (want_list && listed != total_kmers) {
         why = "kmer spectrum: the list and the histogram disagree";
         return MSBWT_ECUDA;
     }
     *n_kmers = total_kmers;
-    if (LIST) {
+    if (want_list) {
         *kmers = listed ? out_kmers.p : nullptr;
         *counts = listed ? out_counts.p : nullptr;
         if (listed) out_kmers.p = out_counts.p = nullptr;
@@ -312,15 +433,20 @@ int spectrum_run(int device, const IndexView &ix, uint32_t k, uint64_t min_count
 
 }  // namespace
 
-int kmer_spectrum_on_device(int device, const IndexView &ix, uint32_t k, uint64_t min_count, uint64_t *hist,
-                            uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers, std::string &why,
-                            int *launches) {
-    const bool list = kmers != nullptr;
+int kmer_spectrum_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
+                            uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers,
+                            std::string &why, int *launches) {
+    // the canonical walk always carries the k-mer values: the pairs are resolved from them
+    const bool list = canonical || kmers != nullptr;
     if (index_is_wide(ix))
-        return list ? spectrum_run<true, true>(device, ix, k, min_count, hist, nbins, kmers, counts, n_kmers, why, launches)
-                    : spectrum_run<true, false>(device, ix, k, min_count, hist, nbins, kmers, counts, n_kmers, why, launches);
-    return list ? spectrum_run<false, true>(device, ix, k, min_count, hist, nbins, kmers, counts, n_kmers, why, launches)
-                : spectrum_run<false, false>(device, ix, k, min_count, hist, nbins, kmers, counts, n_kmers, why, launches);
+        return list ? spectrum_run<true, true>(device, ix, lanes, canonical, k, min_count, hist, nbins, kmers, counts,
+                                               n_kmers, why, launches)
+                    : spectrum_run<true, false>(device, ix, lanes, false, k, min_count, hist, nbins, kmers, counts,
+                                                n_kmers, why, launches);
+    return list ? spectrum_run<false, true>(device, ix, lanes, canonical, k, min_count, hist, nbins, kmers, counts,
+                                            n_kmers, why, launches)
+                : spectrum_run<false, false>(device, ix, lanes, false, k, min_count, hist, nbins, kmers, counts, n_kmers,
+                                             why, launches);
 }
 
 }  // namespace msbwt

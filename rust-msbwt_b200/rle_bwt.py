@@ -156,6 +156,7 @@ def load_library():
         "msbwt_build_rle_bwt_ragged": (i32, [vp, vp, u64, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64)]),
         "msbwt_merge_rle_bwts": (i32, [vp, u64, vp, u64, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(u32)]),
         "msbwt_kmer_spectrum": (i32, [vp, u32, u64, vp, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
+        "msbwt_kmer_spectrum_canonical": (i32, [vp, u32, u64, vp, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_buffer_free": (None, [vp]),
         "msbwt_convert_to_rle": (i32, [vp, u64, C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_save_rle_npy": (i32, [vp, u64, C.c_char_p]),
@@ -185,7 +186,7 @@ EXPORTED_SYMBOLS = (
     "msbwt_count_kmers_fixed", "msbwt_constrain_ranges", "msbwt_count_kmers_fixed_device",
     "msbwt_constrain_ranges_device", "msbwt_packed_bytes", "msbwt_pack_kmers_device",
     "msbwt_count_kmers_packed_device", "msbwt_launch_count", "msbwt_gather_bench", "msbwt_l2_fetch_granularity", "msbwt_debug_build_image", "msbwt_debug_copy_image",
-    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_merge_rle_bwts", "msbwt_kmer_spectrum", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
+    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_merge_rle_bwts", "msbwt_kmer_spectrum", "msbwt_kmer_spectrum_canonical", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
     "msbwt_save_runs_npy",
     "msbwt_host_free", "msbwt_last_error", "msbwt_abi_version",
 )
@@ -421,15 +422,16 @@ class RleBWT:
                "count_read_kmers")
         return out
 
-    def _kmer_spectrum(self, k: int, min_count: int, nbins: int, with_list: bool):
+    def _kmer_spectrum(self, k: int, min_count: int, nbins: int, with_list: bool, canonical: bool = False):
         L = load_library()
         if k < 0 or min_count < 0 or nbins < 0:
             raise MsbwtError(EINVAL, "k, min_count and nbins must not be negative")
         hist = np.zeros(nbins, dtype=np.uint64)
         km, cn, n = C.c_void_p(0), C.c_void_p(0), C.c_uint64(0)
-        _check(L.msbwt_kmer_spectrum(self.handle, k, min_count, _p(hist) if nbins else None, nbins,
-                                     C.byref(km) if with_list else None, C.byref(cn) if with_list else None, C.byref(n)),
-               "kmer_spectrum")
+        fn = L.msbwt_kmer_spectrum_canonical if canonical else L.msbwt_kmer_spectrum
+        _check(fn(self.handle, k, min_count, _p(hist) if nbins else None, nbins,
+                  C.byref(km) if with_list else None, C.byref(cn) if with_list else None, C.byref(n)),
+               "kmer_spectrum_canonical" if canonical else "kmer_spectrum")
         if not with_list:
             return hist, None, None
         try:
@@ -440,16 +442,20 @@ class RleBWT:
             L.msbwt_buffer_free(cn)
         return hist, kmers, counts
 
-    def kmer_spectrum(self, k: int, min_count: int = 1, nbins: int = 10001) -> np.ndarray:
+    def kmer_spectrum(self, k: int, min_count: int = 1, nbins: int = 10001, canonical: bool = False) -> np.ndarray:
         """The k-mer spectrum: hist[c] = number of distinct ACGT k-mers (k <= 32) occurring exactly c times (count_kmer),
         the last bin holding those occurring nbins - 1 times or more; bins below min_count are 0.  Computed on the
-        device by a pruned backward search; no k-mer crosses the link."""
-        return self._kmer_spectrum(k, min_count, nbins, False)[0]
+        device by a pruned backward search; no k-mer crosses the link.  canonical=True counts each k-mer on both
+        strands, once per pair {X, rc X}: count_kmer(X) + count_kmer(rc X), or count_kmer(X) for a palindrome
+        (msbwt_kmer_spectrum_canonical), the spectrum `jellyfish count -C` gives for the reads."""
+        return self._kmer_spectrum(k, min_count, nbins, False, canonical)[0]
 
-    def list_kmers(self, k: int, min_count: int = 2) -> tuple[np.ndarray, np.ndarray]:
+    def list_kmers(self, k: int, min_count: int = 2, canonical: bool = False) -> tuple[np.ndarray, np.ndarray]:
         """(kmers u64, counts u64): every ACGT k-mer (k <= 32) with count_kmer >= min_count, as count_kmers_u64 takes
-        them (A,C,G,T = 0..3, first symbol most significant), in co-lexicographic order (by the last symbol first)."""
-        _, kmers, counts = self._kmer_spectrum(k, min_count, 0, True)
+        them (A,C,G,T = 0..3, first symbol most significant), in co-lexicographic order (by the last symbol first).
+        canonical=True: the canonical k-mers min(X, rc X) whose canonical count (see kmer_spectrum) is >= min_count,
+        with that count, in a deterministic order and no other promised."""
+        _, kmers, counts = self._kmer_spectrum(k, min_count, 0, True, canonical)
         return kmers, counts
 
     # -- device-buffer entry points (raw pointers: torch `.data_ptr()` / stream handles)
