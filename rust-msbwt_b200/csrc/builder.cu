@@ -145,21 +145,14 @@ __global__ void stamp_checkpoints_kernel(const uint64_t *__restrict__ before, ui
     aux[b * 2 + 1] = rel[4];
 }
 
-#define B_TRY(expr)                                                                        \
-    do {                                                                                   \
-        cudaError_t e_ = (expr);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            why = std::string(#expr) + ": " + cudaGetErrorString(e_);                      \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;           \
-        }                                                                                  \
-    } while (0)
+#define B_TRY(e) CU_TRY(e)
 
 }  // namespace
 
-int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift, DeviceImage &img, std::string &why) {
-    if (len && !h_rle) { why = "rle is NULL"; return MSBWT_EINVAL; }
+int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift, DeviceImage &img) {
+    if (len && !h_rle) return fail(MSBWT_EINVAL, "rle is NULL");
     if (sb_shift == 0) sb_shift = kDefaultSuperShift;
-    if (sb_shift > (uint32_t)kDefaultSuperShift) { why = "superblock_shift > 25 would overflow the u32 block counters"; return MSBWT_EINVAL; }
+    if (sb_shift > (uint32_t)kDefaultSuperShift) return fail(MSBWT_EINVAL, "superblock_shift > 25 would overflow the u32 block counters");
     DeviceScratch tmp;
     uint8_t *d_rle = nullptr;
     uint64_t *d_before = nullptr, *d_run_byte = nullptr, *d_nruns = nullptr, *d_run_pos = nullptr;
@@ -178,7 +171,7 @@ int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift,
         B_TRY(cudaGetLastError());
         uint32_t flag = 0;
         B_TRY(cudaMemcpy(&flag, d_flag, sizeof(flag), cudaMemcpyDeviceToHost));
-        if (flag) { why = "RLE stream has a symbol >= 6 or a run longer than 2^60 symbols"; return MSBWT_EFORMAT; }
+        if (flag) return fail(MSBWT_EFORMAT, "RLE stream has a symbol >= 6 or a run longer than 2^60 symbols");
 
         // 1. positions: exclusive sum over len + 1 items (the extra item yields the total)
         cub::CountingInputIterator<uint64_t> idx(0);
@@ -191,7 +184,7 @@ int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift,
         uint64_t last_before = 0;
         B_TRY(cudaMemcpy(&last_before, d_before + (len - 1), sizeof(uint64_t), cudaMemcpyDeviceToHost));
         total = last_before + Contribution{h_rle}(len - 1);
-        if (total >> 62) { why = "BWT longer than 2^62 symbols"; return MSBWT_EFORMAT; }
+        if (total >> 62) return fail(MSBWT_EFORMAT, "BWT longer than 2^62 symbols");
 
         // 2. run table
         B_TRY(tmp.alloc(&d_run_byte, len));
@@ -251,7 +244,7 @@ int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift,
         start.c[s] = sum;
         sum += img.counts[s];
     }
-    if (sum != total) { why = "internal error: block counts do not add up to the stream total"; return MSBWT_ECUDA; }
+    if (sum != total) return fail(MSBWT_ECUDA, "internal error: block counts do not add up to the stream total");
 
     // 5. checkpoints
     stamp_checkpoints_kernel<<<(unsigned)((img.nblocks + 255) / 256), 256>>>(

@@ -200,14 +200,7 @@ __global__ void emit_rle_kernel(const uint8_t *__restrict__ bwt, const uint64_t 
     while (len) { *out++ = (uint8_t)(sym | ((len & 31u) << 3)); len >>= 5; }
 }
 
-#define W_TRY(expr)                                                                        \
-    do {                                                                                   \
-        cudaError_t e_ = (expr);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            why = std::string("bwt build: ") + #expr + ": " + cudaGetErrorString(e_);      \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;           \
-        }                                                                                  \
-    } while (0)
+#define W_TRY(e) CU_TRY_IN("bwt build: ", e)
 
 constexpr unsigned kGridCap = 148 * 32;
 unsigned grid_for(uint64_t n, unsigned threads = 256) {
@@ -216,8 +209,7 @@ unsigned grid_for(uint64_t n, unsigned threads = 256) {
 
 // sorts (key, id) pairs by the 63 key bits, stably; ids end up in ids.Current()
 template <class IdT>
-int sort_pass(cub::DoubleBuffer<uint64_t> &keys, cub::DoubleBuffer<IdT> &ids, uint64_t n, void *d_temp, size_t temp_bytes,
-              std::string &why) {
+int sort_pass(cub::DoubleBuffer<uint64_t> &keys, cub::DoubleBuffer<IdT> &ids, uint64_t n, void *d_temp, size_t temp_bytes) {
     W_TRY(cub::DeviceRadixSort::SortPairs(d_temp, temp_bytes, keys, ids, (int64_t)n, 0, 63));
     return MSBWT_OK;
 }
@@ -226,8 +218,7 @@ int sort_pass(cub::DoubleBuffer<uint64_t> &keys, cub::DoubleBuffer<IdT> &ids, ui
 // nullptr: every read has l1 suffixes
 template <class IdT>
 int suffix_sort_and_emit(const uint64_t *d_sorted, uint64_t n_reads, uint64_t n, uint32_t l1, uint32_t stride_words, uint32_t key_words,
-                         const uint64_t *d_starts, const uint64_t *d_counts, uint8_t *d_bwt, DeviceScratch &tmp, std::string &why,
-                         int *launches) {
+                         const uint64_t *d_starts, const uint64_t *d_counts, uint8_t *d_bwt, DeviceScratch &tmp) {
     uint64_t *k0 = nullptr, *k1 = nullptr;
     IdT *v0 = nullptr, *v1 = nullptr;
     W_TRY(tmp.alloc(&k0, n));
@@ -246,8 +237,8 @@ int suffix_sort_and_emit(const uint64_t *d_sorted, uint64_t n_reads, uint64_t n,
     for (uint32_t w = key_words; w-- > 0;) {
         suffix_keys_kernel<IdT><<<grid_for(n), 256>>>(d_sorted, ids.Current(), n, l1, stride_words, w, keys.Current());
         W_TRY(cudaGetLastError());
-        if (int rc = sort_pass<IdT>(keys, ids, n, d_temp, temp_bytes, why); rc != MSBWT_OK) return rc;
-        if (launches) *launches += 2;
+        if (int rc = sort_pass<IdT>(keys, ids, n, d_temp, temp_bytes); rc != MSBWT_OK) return rc;
+        g_launches += 2;
     }
     emit_bwt_kernel<IdT><<<grid_for(n), 256>>>(d_sorted, ids.Current(), n, l1, stride_words, d_bwt);
     W_TRY(cudaGetLastError());
@@ -261,8 +252,7 @@ int suffix_sort_and_emit(const uint64_t *d_sorted, uint64_t n_reads, uint64_t n,
 // d_bwt: n symbol bytes on the current device -> *d_rle_out, a cudaMalloc'd buffer of *rle_len msbwt RLE bytes
 // (src/bwt_converter.rs:52-56; the caller frees it).  Shared by the builder above and the merge (bwt_merge.cu), so
 // both emit the same canonical encoding.
-int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, uint64_t *rle_len, std::string &why,
-                         int *launches) {
+int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, uint64_t *rle_len) {
     *d_rle_out = nullptr;
     *rle_len = 0;
     if (!n) return MSBWT_OK;
@@ -330,7 +320,7 @@ int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, 
     emit_rle_kernel<<<(unsigned)((n_runs + 255) / 256), 256>>>(d_bwt, d_starts, d_byte_offsets, n_runs, n, d_rle);
     if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) { cudaFree(d_rle); W_TRY(e); }
     if (cudaError_t e = cudaDeviceSynchronize(); e != cudaSuccess) { cudaFree(d_rle); W_TRY(e); }
-    if (launches) *launches += 4;
+    g_launches += 4;
     *d_rle_out = d_rle;
     *rle_len = bytes;
     return MSBWT_OK;
@@ -341,14 +331,14 @@ int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, 
 // offsets on the device).  On success *d_rle_out is a cudaMalloc'd buffer of *rle_len RLE bytes (the caller frees it)
 // and *total = the number of symbols of the BWT (every read's length + 1).
 int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, uint64_t n_reads, uint32_t read_len,
-                            uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, std::string &why, int *launches) {
+                            uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total) {
     *d_rle_out = nullptr;
     *rle_len = 0;
     *total = 0;
     if (!n_reads) return MSBWT_OK;
-    if ((!read_len && !d_offsets) || (read_len && !d_reads)) { why = "bwt build: empty reads or NULL buffer"; return MSBWT_EINVAL; }
-    if (n_reads >> 32) { why = "bwt build: more than 2^32 reads"; return MSBWT_EINVAL; }
-    if (read_len == 0xFFFFFFFFu) { why = "bwt build: read too long"; return MSBWT_EINVAL; }
+    if ((!read_len && !d_offsets) || (read_len && !d_reads)) return fail(MSBWT_EINVAL, "bwt build: empty reads or NULL buffer");
+    if (n_reads >> 32) return fail(MSBWT_EINVAL, "bwt build: more than 2^32 reads");
+    if (read_len == 0xFFFFFFFFu) return fail(MSBWT_EINVAL, "bwt build: read too long");
     const uint32_t l1 = read_len + 1;
     uint64_t n = n_reads * l1;  // (reads of different lengths: the suffixes that exist, counted below)
     const uint32_t words = (l1 + kKeySyms - 1) / kKeySyms;  // key words per read ('$' included)
@@ -368,8 +358,8 @@ int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, u
     W_TRY(cudaGetLastError());
     uint32_t bad = 0;
     W_TRY(cudaMemcpy(&bad, d_bad, sizeof(bad), cudaMemcpyDeviceToHost));
-    if (bad) { why = "bwt build: a read holds '$' (0) or a symbol >= 6"; return MSBWT_EINVAL; }
-    if (launches) (*launches)++;
+    if (bad) return fail(MSBWT_EINVAL, "bwt build: a read holds '$' (0) or a symbol >= 6");
+    g_launches++;
 
     // 2. sort the reads
     {
@@ -390,8 +380,8 @@ int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, u
         for (uint32_t w = words; w-- > 0;) {
             read_keys_kernel<<<(unsigned)((n_reads + 255) / 256), 256>>>(d_packed, ids.Current(), n_reads, stride_words, w, keys.Current());
             W_TRY(cudaGetLastError());
-            if (int rc = sort_pass<uint32_t>(keys, ids, n_reads, d_temp, temp_bytes, why); rc != MSBWT_OK) return rc;
-            if (launches) *launches += 2;
+            if (int rc = sort_pass<uint32_t>(keys, ids, n_reads, d_temp, temp_bytes); rc != MSBWT_OK) return rc;
+            g_launches += 2;
         }
         permute_reads_kernel<<<(unsigned)((n_reads * stride_words + 255) / 256), 256>>>(d_packed, ids.Current(), n_reads, stride_words, d_sorted);
         W_TRY(cudaGetLastError());
@@ -420,13 +410,13 @@ int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, u
     W_TRY(tmp.alloc(&d_bwt, n));
     // (a suffix id is read rank * l1 + offset in the padded layout, whatever the reads' own lengths)
     const int rc = ((n_reads * l1) >> 32)
-                       ? suffix_sort_and_emit<uint64_t>(d_sorted, n_reads, n, l1, stride_words, words, d_suffix_starts, d_suffix_counts, d_bwt, tmp, why, launches)
-                       : suffix_sort_and_emit<uint32_t>(d_sorted, n_reads, n, l1, stride_words, words, d_suffix_starts, d_suffix_counts, d_bwt, tmp, why, launches);
+                       ? suffix_sort_and_emit<uint64_t>(d_sorted, n_reads, n, l1, stride_words, words, d_suffix_starts, d_suffix_counts, d_bwt, tmp)
+                       : suffix_sort_and_emit<uint32_t>(d_sorted, n_reads, n, l1, stride_words, words, d_suffix_starts, d_suffix_counts, d_bwt, tmp);
     if (rc != MSBWT_OK) return rc;
     tmp.release(d_sorted);
 
     // 4b. run table -> RLE bytes
-    if (int rc2 = encode_rle_on_device(d_bwt, n, d_rle_out, rle_len, why, launches); rc2 != MSBWT_OK) return rc2;
+    if (int rc2 = encode_rle_on_device(d_bwt, n, d_rle_out, rle_len); rc2 != MSBWT_OK) return rc2;
     *total = n;
     return MSBWT_OK;
 }

@@ -196,29 +196,21 @@ struct ImageOwner {
     ~ImageOwner() { free_device_image(img); }
 };
 
-#define M_TRY(expr)                                                                        \
-    do {                                                                                   \
-        cudaError_t e_ = (expr);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            why = std::string("bwt merge: ") + #expr + ": " + cudaGetErrorString(e_);      \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;           \
-        }                                                                                  \
-    } while (0)
+#define M_TRY(e) CU_TRY_IN("bwt merge: ", e)
 
 }  // namespace
 
 int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8_t *h_rle_b, uint64_t len_b,
-                             uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, uint32_t *iterations,
-                             std::string &why, int *launches) {
+                             uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, uint32_t *iterations) {
     *d_rle_out = nullptr;
     *rle_len = 0;
     *total = 0;
     *iterations = 0;
     ImageOwner A, B;
-    if (int rc = build_image_on_device(h_rle_a, len_a, 0, A.img, why); rc != MSBWT_OK) { why = "input A: " + why; return rc; }
-    if (int rc = build_image_on_device(h_rle_b, len_b, 0, B.img, why); rc != MSBWT_OK) { why = "input B: " + why; return rc; }
+    if (int rc = build_image_on_device(h_rle_a, len_a, 0, A.img); rc != MSBWT_OK) return fail(rc, "input A: " + g_last_error);
+    if (int rc = build_image_on_device(h_rle_b, len_b, 0, B.img); rc != MSBWT_OK) return fail(rc, "input B: " + g_last_error);
     const uint64_t n_a = A.img.total, n = A.img.total + B.img.total;
-    if (n >> 62) { why = "bwt merge: the merged BWT would hold 2^62 symbols or more"; return MSBWT_EFORMAT; }
+    if (n >> 62) return fail(MSBWT_EFORMAT, "bwt merge: the merged BWT would hold 2^62 symbols or more");
     if (!n) return MSBWT_OK;
     const IndexView va = view_of(A.img), vb = view_of(B.img);
 
@@ -241,7 +233,7 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
     M_TRY(cudaGetLastError());
     tile_zeros_kernel<<<grid, kMergeThreads>>>(reinterpret_cast<const uint4 *>(cur), nullptr, n, n_tiles, d_zeros, d_changed);
     M_TRY(cudaGetLastError());
-    if (launches) *launches += 2;
+    g_launches += 2;
     // the iteration ends after at most N_A + N_B passes; more means a broken invariant, not a slow input
     for (uint64_t it = 1;; it++) {
         M_TRY(cub::DeviceScan::ExclusiveSum(d_temp, temp_bytes, d_zeros, d_zbefore, (int64_t)n_tiles));
@@ -252,7 +244,7 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
         tile_zeros_kernel<<<grid, kMergeThreads>>>(reinterpret_cast<const uint4 *>(next), reinterpret_cast<const uint4 *>(cur),
                                                    n, n_tiles, d_zeros, d_changed);
         M_TRY(cudaGetLastError());
-        if (launches) *launches += 3;
+        g_launches += 3;
         uint32_t changed = 0;
         M_TRY(cudaMemcpy(&changed, d_changed, sizeof(changed), cudaMemcpyDeviceToHost));
         std::swap(cur, next);
@@ -260,7 +252,7 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
             *iterations = (uint32_t)std::min<uint64_t>(it, 0xFFFFFFFFull);
             break;
         }
-        if (it > n) { why = "bwt merge: internal error: the interleave did not reach its fixed point"; return MSBWT_ECUDA; }
+        if (it > n) return fail(MSBWT_ECUDA, "bwt merge: internal error: the interleave did not reach its fixed point");
     }
 
     // the merged symbols, then the images and bit-vectors are no longer needed
@@ -271,11 +263,11 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
     merge_pass_kernel<true><<<grid, kMergeThreads>>>(va, vb, cur, d_zbefore, n, n_tiles, nullptr, d_bwt);
     M_TRY(cudaGetLastError());
     M_TRY(cudaDeviceSynchronize());
-    if (launches) *launches += 2;
+    g_launches += 2;
     bufs.release_all();
     free_device_image(A.img);
     free_device_image(B.img);
-    if (int rc = encode_rle_on_device(d_bwt, n, d_rle_out, rle_len, why, launches); rc != MSBWT_OK) return rc;
+    if (int rc = encode_rle_on_device(d_bwt, n, d_rle_out, rle_len); rc != MSBWT_OK) return rc;
     *total = n;
     return MSBWT_OK;
 }

@@ -20,7 +20,6 @@ using namespace msbwt;
 
 namespace msbwt {
 thread_local std::string g_last_error;
-thread_local int g_call_launches = 0;
 std::atomic<uint64_t> g_launches{0};
 int codec_fail(int code, const std::string &msg) { return fail(code, msg); }  // codec.cpp reports through the same thread-local
 }  // namespace msbwt
@@ -120,9 +119,7 @@ int build_replicas_on_device(msbwt_index *idx, const uint8_t *rle, uint64_t len,
     int rc = for_each_replica_slot(devs.size(), [&](size_t i) -> int {
         DeviceGuard guard(devs[i]);
         DeviceImage img;
-        std::string why;
-        int r = build_image_on_device(rle, len, sb_shift, img, why);
-        if (r != MSBWT_OK) { free_device_image(img); return fail(r, why); }
+        if (int r = build_image_on_device(rle, len, sb_shift, img); r != MSBWT_OK) { free_device_image(img); return r; }
         auto rep = std::make_unique<Replica>();
         rep->device = devs[i];
         rep->d_blocks = img.blocks;
@@ -300,13 +297,21 @@ int deepen_table_for_hbm(int s, uint64_t image_bytes, size_t entry_bytes, uint64
 
 int build_pair(msbwt_index *idx, Replica &rep, uint8_t **keep_codes = nullptr) {
     DeviceGuard guard(rep.device);
-    std::string why;
-    int n = 0;
-    int rc = build_pair_image_on_device(rep.device, rep.view, idx->start, rep.pair, why, &n, keep_codes);
-    g_launches += (uint64_t)n;
-    if (rc != MSBWT_OK) { free_pair_image(rep.pair); return fail(rc, why); }
+    if (int rc = build_pair_image_on_device(rep.device, rep.view, idx->start, rep.pair, keep_codes); rc != MSBWT_OK) {
+        free_pair_image(rep.pair);
+        return rc;
+    }
     refresh_view(rep);
     return MSBWT_OK;
+}
+
+// Out of device memory for an image the caller did not require: the index works without it.  Clears the CUDA error and
+// the builder's message, so that the create still succeeds with an empty msbwt_last_error().
+bool absorb_oom(int rc, bool required) {
+    if (rc != MSBWT_ENOMEM || required) return false;
+    cudaGetLastError();
+    g_last_error.clear();
+    return true;
 }
 
 void build_trace(const char *what) {
@@ -320,14 +325,9 @@ void build_trace(const char *what) {
 // The final-step lines on top of the oct image, from the 20-symbol codes (owned by the builder from here on).  Running out
 // of device memory leaves the index without this image unless the caller required it.
 int build_fin(Replica &rep, const Layout &p, uint64_t *codes20) {
-    std::string why;
-    int n = 0;
-    int rc = build_fin_lines_on_device(rep.device, rep.view.total, codes20, p.fin_shift, p.fin_lb, rep.fin, why, &n);
-    g_launches += (uint64_t)n;
-    if (rc != MSBWT_OK) {
+    if (int rc = build_fin_lines_on_device(rep.device, rep.view.total, codes20, p.fin_shift, p.fin_lb, rep.fin); rc != MSBWT_OK) {
         free_fin_image(rep.fin);
-        if (rc == MSBWT_ENOMEM && !p.fin_required) { cudaGetLastError(); return MSBWT_OK; }
-        return fail(rc, why);
+        return absorb_oom(rc, p.fin_required) ? MSBWT_OK : rc;
     }
     refresh_view(rep);
     build_trace("multi-step images done");
@@ -347,37 +347,25 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Layout &p) {
     DeviceGuard guard(rep.device);
     DevicePtr<uint8_t> codes2_owner(codes2);
     uint16_t *codes4 = nullptr;
-    std::string why;
-    int n = 0;
     build_trace("quad image");
-    int rc = build_quad_image_on_device(rep.device, rep.view, codes2, rep.quad, why, &n, p.oct ? &codes4 : nullptr);
-    g_launches += (uint64_t)n;
+    int rc = build_quad_image_on_device(rep.device, rep.view, codes2, rep.quad, p.oct ? &codes4 : nullptr);
     free_pair_image(rep.pair);
-    if (rc != MSBWT_OK) { free_quad_image(rep.quad); if (codes4) cudaFree(codes4); return fail(rc, why); }
+    if (rc != MSBWT_OK) { free_quad_image(rep.quad); if (codes4) cudaFree(codes4); return rc; }
     refresh_view(rep);
     if (!p.oct) return MSBWT_OK;
 
     const uint64_t N = rep.view.total;
     // 10-symbol codes (4 B per position), then 20-symbol codes (8 B per position): both walk LF^4 through the quad image
     uint32_t *codes10 = nullptr;
-    n = 0;
     build_trace("10-symbol codes");
-    rc = build_oct_codes_on_device(rep.device, rep.view, codes4, codes2, &codes10, why, &n);  // frees codes4
-    g_launches += (uint64_t)n;
-    if (rc != MSBWT_OK) return fail(rc, why);
+    rc = build_oct_codes_on_device(rep.device, rep.view, codes4, codes2, &codes10);  // frees codes4
+    if (rc != MSBWT_OK) return rc;
     DevicePtr<uint32_t> codes10_owner(codes10);
     codes2_owner.reset();
     uint64_t *codes20 = nullptr;
-    if (p.fin) {
-        n = 0;
-        rc = build_fin_codes_on_device(rep.device, rep.view, codes10, &codes20, why, &n);
-        g_launches += (uint64_t)n;
-        if (rc == MSBWT_ENOMEM && !p.fin_required) {  // no room for the codes: the index works without this image
-            cudaGetLastError();
-            codes20 = nullptr;
-        } else if (rc != MSBWT_OK) {
-            return fail(rc, why);
-        }
+    if (p.fin) {  // no room for the codes: codes20 stays null and the index works without this image
+        rc = build_fin_codes_on_device(rep.device, rep.view, codes10, &codes20);
+        if (rc != MSBWT_OK && !absorb_oom(rc, p.fin_required)) return rc;
     }
     DevicePtr<uint64_t> codes20_owner(codes20);
     if (!p.keep_quad) {
@@ -393,12 +381,10 @@ int build_multi_step(msbwt_index *idx, Replica &rep, const Layout &p) {
     const uint64_t fin_need = codes20 ? fin_image_bytes(N, p.fin_shift, p.fin_lb) + 4 * N : 0;
     const uint64_t reserve = fin_need + (p.oct_required ? 0 : (8ull << 30));
     const uint64_t budget = free_b > reserve ? free_b - reserve : 0;
-    n = 0;
     build_trace("oct lines");
-    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, p.oct_shift, budget, rep.oct, why, &n);
-    g_launches += (uint64_t)n;
+    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, p.oct_shift, budget, rep.oct);
     codes10_owner.reset();
-    if (rc != MSBWT_OK) { free_oct_image(rep.oct); return fail(rc, why); }
+    if (rc != MSBWT_OK) { free_oct_image(rep.oct); return rc; }
     if (!rep.oct.lines) {  // no room at all: the quad image serves alone and must stay
         if (!rep.view.quad) return fail(MSBWT_ENOMEM, "no room for the oct image after the quad image was dropped (MSBWT_KEEP_QUAD=1 keeps it)");
         return MSBWT_OK;
@@ -421,18 +407,10 @@ int build_multi_step_wide(Replica &rep, const Layout &p, bool *built) {
     *built = false;
     DeviceGuard guard(rep.device);
     const uint64_t N = rep.view.total;
-    std::string why;
-    int n = 0;
-    auto soft = [&](int rc) {  // out of memory on an automatic build: the index works without these images
-        if (rc == MSBWT_ENOMEM && !p.oct_required) { cudaGetLastError(); return true; }
-        return false;
-    };
-
     uint32_t *codes10 = nullptr;
     build_trace("10-symbol codes (walk)");
-    int rc = build_oct_codes_by_walk(rep.device, rep.view, &codes10, why, &n);
-    g_launches += (uint64_t)n;
-    if (rc != MSBWT_OK) return soft(rc) ? MSBWT_OK : fail(rc, why);
+    int rc = build_oct_codes_by_walk(rep.device, rep.view, &codes10);
+    if (rc != MSBWT_OK) return absorb_oom(rc, p.oct_required) ? MSBWT_OK : rc;
     DevicePtr<uint32_t> codes10_owner(codes10);
 
     const uint64_t free_b = free_bytes_now();
@@ -441,13 +419,11 @@ int build_multi_step_wide(Replica &rep, const Layout &p, bool *built) {
     const uint64_t fin_need = p.fin ? fin_image_bytes(N, p.fin_shift, p.fin_lb) + 12 * N : 0;
     const uint64_t reserve = fin_need + (p.oct_required ? 0 : (8ull << 30));
     const uint64_t budget = free_b > reserve ? free_b - reserve : 0;
-    n = 0;
     build_trace("oct lines");
-    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, p.oct_shift, budget, rep.oct, why, &n);
-    g_launches += (uint64_t)n;
+    rc = build_oct_lines_on_device(rep.device, rep.view, codes10, p.oct_shift, budget, rep.oct);
     if (rc != MSBWT_OK) {
         free_oct_image(rep.oct);
-        return soft(rc) ? MSBWT_OK : fail(rc, why);
+        return absorb_oom(rc, p.oct_required) ? MSBWT_OK : rc;
     }
     if (!rep.oct.lines) {
         if (p.oct_required) return fail(MSBWT_ENOMEM, "no room for the oct image of this index");
@@ -458,14 +434,9 @@ int build_multi_step_wide(Replica &rep, const Layout &p, bool *built) {
     if (!p.fin) return MSBWT_OK;
 
     uint64_t *codes20 = nullptr;
-    n = 0;
-    rc = build_fin_codes_by_walk(rep.device, rep.view, codes10, &codes20, why, &n);
-    g_launches += (uint64_t)n;
+    rc = build_fin_codes_by_walk(rep.device, rep.view, codes10, &codes20);
     codes10_owner.reset();
-    if (rc != MSBWT_OK) {
-        if (rc == MSBWT_ENOMEM && !p.fin_required) { cudaGetLastError(); return MSBWT_OK; }
-        return fail(rc, why);
-    }
+    if (rc != MSBWT_OK) return absorb_oom(rc, p.fin_required) ? MSBWT_OK : rc;
     return build_fin(rep, p, codes20);
 }
 
@@ -500,7 +471,6 @@ int build_suffix_table(Replica &rep, int s) {
     e = cudaMemcpy(level[0], wide ? (const void *)root : (const void *)root32, eb, cudaMemcpyHostToDevice);
     for (int j = 0; j < s && e == cudaSuccess; j++) {
         e = launch_table_extend(rep.device, rep.view, level[(size_t)j], level[(size_t)j + 1], (uint32_t)(1ull << (2 * (j + 1))), nullptr);
-        g_launches++;
     }
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
@@ -518,14 +488,9 @@ int build_suffix_table(Replica &rep, int s) {
 msbwt_index *create_common(const uint8_t *rle, uint64_t len, const int *devices, int ndev, Options opt, int *err) {
     fill_from_env(opt);
     g_last_error.clear();
-    int rc;
-    std::string why;
     auto idx = std::make_unique<msbwt_index>();
-    if ((rc = validate_rle(rle, len, why)) != MSBWT_OK) {
-        fail(rc, why);
-    } else {
-        rc = build_replicas_on_device(idx.get(), rle, len, opt.sb_shift, devices, ndev);
-    }
+    int rc = validate_rle(rle, len);
+    if (rc == MSBWT_OK) rc = build_replicas_on_device(idx.get(), rle, len, opt.sb_shift, devices, ndev);
     if (rc == MSBWT_OK) {
         rc = for_each_replica_slot(idx->reps.size(), [&](size_t slot) -> int {
             Replica &rep = *idx->reps[slot];
@@ -615,10 +580,7 @@ extern "C" msbwt_index *msbwt_index_create_opts(const uint8_t *rle, uint64_t len
 extern "C" msbwt_index *msbwt_index_create_from_npy(const char *path, const int *devices, int ndev, int *err) {
     g_last_error.clear();
     std::vector<uint8_t> payload;
-    std::string why;
-    int rc = read_npy_payload(path, payload, why);
-    if (rc != MSBWT_OK) {
-        fail(rc, why);
+    if (int rc = read_npy_payload(path, payload); rc != MSBWT_OK) {
         if (err) *err = rc;
         return nullptr;
     }
@@ -634,10 +596,7 @@ extern "C" msbwt_index *msbwt_index_create_from_npy_opts(const char *path, const
         return nullptr;
     }
     std::vector<uint8_t> payload;
-    std::string why;
-    int rc = read_npy_payload(path, payload, why);
-    if (rc != MSBWT_OK) {
-        fail(rc, why);
+    if (int rc = read_npy_payload(path, payload); rc != MSBWT_OK) {
         if (err) *err = rc;
         return nullptr;
     }
@@ -753,10 +712,7 @@ extern "C" int msbwt_count_kmers_fixed_device(const msbwt_index *idx, int slot, 
     for (uint64_t q0 = 0; q0 < n; q0 += per) {  // sub-batches reuse the scratch in stream order
         const uint64_t m = std::min(per, n - q0);
         CU_TRY(launch_pack_seed(rep.view, d_syms + q0 * k, k, m, rep.dev_packed.as<uint64_t>(), d_out + q0, flag, st));
-        g_launches++;
-        CU_TRY(launch_count_packed(rep.device, rep.view, rep.lanes, rep.dev_packed.as<uint64_t>(), k, m, d_out + q0, st,
-                                   &g_call_launches));
-        flush_launches();
+        CU_TRY(launch_count_packed(rep.device, rep.view, rep.lanes, rep.dev_packed.as<uint64_t>(), k, m, d_out + q0, st));
     }
     CU_TRY(cudaEventRecord(rep.dev_packed_free, st));
     return MSBWT_OK;
@@ -775,7 +731,6 @@ extern "C" int msbwt_pack_kmers_device(const msbwt_index *idx, int slot, const u
     Replica &rep = *idx->reps[slot];
     DeviceGuard guard(rep.device);
     CU_TRY(launch_pack_seed(rep.view, d_syms, k, n, d_packed, d_out, d_status, (cudaStream_t)stream));
-    g_launches++;
     return MSBWT_OK;
 }
 
@@ -790,7 +745,6 @@ extern "C" int msbwt_seed_kmers_u64_device(const msbwt_index *idx, int slot, con
     Replica &rep = *idx->reps[slot];
     DeviceGuard guard(rep.device);
     CU_TRY(launch_seed_u64(rep.view, d_kmers, k, n, d_packed, d_out, (cudaStream_t)stream));
-    g_launches++;
     return MSBWT_OK;
 }
 
@@ -802,8 +756,7 @@ extern "C" int msbwt_count_kmers_packed_device(const msbwt_index *idx, int slot,
     if (!n) return MSBWT_OK;
     Replica &rep = *idx->reps[slot];
     DeviceGuard guard(rep.device);
-    CU_TRY(launch_count_packed(rep.device, rep.view, rep.lanes, d_packed, k, n, d_out, (cudaStream_t)stream, &g_call_launches));
-    flush_launches();
+    CU_TRY(launch_count_packed(rep.device, rep.view, rep.lanes, d_packed, k, n, d_out, (cudaStream_t)stream));
     return MSBWT_OK;
 }
 
@@ -839,7 +792,6 @@ extern "C" int msbwt_count_kmers_packed_stats_device(const msbwt_index *idx, int
     if (!n) return MSBWT_OK;
     DeviceGuard guard(rep.device);
     CU_TRY(launch_count_oct_stats(rep.device, rep.view, d_packed, k, n, d_out, (unsigned long long *)d_stats, (cudaStream_t)stream));
-    g_launches++;
     return MSBWT_OK;
 }
 
@@ -851,8 +803,7 @@ extern "C" int msbwt_constrain_ranges_device(const msbwt_index *idx, int slot, c
     if (!n) return MSBWT_OK;
     Replica &rep = *idx->reps[slot];
     DeviceGuard guard(rep.device);
-    CU_TRY(launch_constrain_ranges(rep.device, rep.view, d_sym, d_l, d_h, n, d_out_l, d_out_h, (cudaStream_t)stream, &g_call_launches));
-    flush_launches();
+    CU_TRY(launch_constrain_ranges(rep.device, rep.view, d_sym, d_l, d_h, n, d_out_l, d_out_h, (cudaStream_t)stream));
     return MSBWT_OK;
 }
 
@@ -875,9 +826,7 @@ extern "C" int msbwt_debug_build_image(const uint8_t *rle, uint64_t len, uint32_
     g_last_error.clear();
     if (!nblocks || !n_super) return fail(MSBWT_EINVAL, "NULL size outputs");
     HostImage img;
-    std::string why;
-    int rc = build_image_from_rle(rle, len, superblock_shift, img, why);
-    if (rc != MSBWT_OK) return fail(rc, why);
+    if (int rc = build_image_from_rle(rle, len, superblock_shift, img); rc != MSBWT_OK) return rc;
     *nblocks = img.nblocks;
     *n_super = img.n_super;
     if (blocks) memcpy(blocks, img.blocks.data(), img.blocks.size() * sizeof(uint32_t));
@@ -972,8 +921,7 @@ extern "C" int msbwt_constrain_ranges_fanout_device(const msbwt_index *idx, int 
     if (!n) return MSBWT_OK;
     Replica &rep = *idx->reps[slot];
     DeviceGuard guard(rep.device);
-    CU_TRY(launch_constrain_fanout(rep.device, rep.view, d_l, d_h, n, d_out_l, d_out_h, (cudaStream_t)stream, &g_call_launches));
-    flush_launches();
+    CU_TRY(launch_constrain_fanout(rep.device, rep.view, d_l, d_h, n, d_out_l, d_out_h, (cudaStream_t)stream));
     return MSBWT_OK;
 }
 
@@ -1028,12 +976,9 @@ int build_rle_bwt_common(const uint8_t *reads, const uint64_t *offsets, uint64_t
         }
     }
     uint8_t *d_rle = nullptr;
-    std::string why;
-    int n = 0;
-    int rc = build_rle_bwt_on_device(d_reads, d_offsets, n_reads, read_len, &d_rle, rle_len, total, why, &n);
-    g_launches += (uint64_t)n;
+    int rc = build_rle_bwt_on_device(d_reads, d_offsets, n_reads, read_len, &d_rle, rle_len, total);
     DevicePtr<uint8_t> d_rle_owner(d_rle);
-    if (rc != MSBWT_OK) return fail(rc, why);
+    if (rc != MSBWT_OK) return rc;
     return rle_to_host(d_rle, *rle_len, rle);
 }
 }  // namespace
@@ -1089,12 +1034,9 @@ extern "C" int msbwt_merge_rle_bwts(const uint8_t *rle_a, uint64_t len_a, const 
     uint8_t *d_rle = nullptr;
     uint64_t len = 0, n = 0;
     uint32_t passes = 0;
-    std::string why;
-    int launches = 0;
-    int rc = merge_rle_bwts_on_device(rle_a, len_a, rle_b, len_b, &d_rle, &len, &n, &passes, why, &launches);
-    g_launches += (uint64_t)launches;
+    int rc = merge_rle_bwts_on_device(rle_a, len_a, rle_b, len_b, &d_rle, &len, &n, &passes);
     DevicePtr<uint8_t> d_rle_owner(d_rle);
-    if (rc != MSBWT_OK) return fail(rc, why);
+    if (rc != MSBWT_OK) return rc;
     if (int r = rle_to_host(d_rle, len, rle); r != MSBWT_OK) return r;
     *rle_len = len;
     *total = n;
@@ -1118,12 +1060,8 @@ static int kmer_spectrum_call(const msbwt_index *idx, bool canonical, uint32_t k
     // too: no lane of the replica), so it takes no lock and runs beside the query entry points
     const Replica &rep = *idx->reps[0];
     DeviceGuard guard(rep.device);
-    std::string why;
-    int launches = 0;
-    const int rc = kmer_spectrum_on_device(rep.device, rep.view, rep.lanes, canonical, k, min_count, hist, nbins, kmers,
-                                           counts, n_kmers, why, &launches);
-    g_launches += (uint64_t)launches;
-    return rc == MSBWT_OK ? rc : fail(rc, why);
+    return kmer_spectrum_on_device(rep.device, rep.view, rep.lanes, canonical, k, min_count, hist, nbins, kmers, counts,
+                                   n_kmers);
 }
 
 extern "C" int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist, uint32_t nbins,
@@ -1145,6 +1083,5 @@ extern "C" int msbwt_gather_bench(int device, const void *d_buf, uint64_t buf_by
     if (!d_buf || !d_sink) return fail(MSBWT_EINVAL, "NULL device buffer");
     DeviceGuard guard(device);
     CU_TRY(launch_gather(device, d_buf, buf_bytes, granule, n_gathers, seed, d_sink, (cudaStream_t)stream));
-    g_launches++;
     return MSBWT_OK;
 }

@@ -1,17 +1,42 @@
 // engine.h -- internal interface between the C ABI (capi.cu), the host-side layout
 // builder (loader.cu) and the kernels (kernels.cu).
+//
+// Errors and launch counts are reported where they happen.  A failing function returns an msbwt_status and leaves
+// its message in g_last_error (msbwt_last_error) through fail() or CU_TRY.  Every launch wrapper, image builder and the
+// spectrum add the kernels they launch to g_launches (msbwt_launch_count); the block image of create (builder.cu) is
+// the one build step that is not counted.
 #pragma once
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <atomic>
 #include <cstdint>
 #include <memory>
 #include <string>
 #include <vector>
 
+#include "../../include/msbwt_gpu.h"
 #include "layout.h"
 
 namespace msbwt {
+
+extern thread_local std::string g_last_error;
+extern std::atomic<uint64_t> g_launches;
+
+inline int fail(int code, const std::string &msg) {
+    g_last_error = msg;
+    return code;
+}
+
+// return MSBWT_ENOMEM (out of device memory) or MSBWT_ECUDA, with "<prefix><expr>: <CUDA error>" as the message
+#define CU_TRY_IN(prefix, expr)                                                                   \
+    do {                                                                                          \
+        cudaError_t e_ = (expr);                                                                  \
+        if (e_ != cudaSuccess)                                                                    \
+            return fail(e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA,             \
+                        std::string(prefix) + #expr + ": " + cudaGetErrorString(e_));            \
+    } while (0)
+#define CU_TRY(expr) CU_TRY_IN("", expr)
 
 // one cudaMalloc'd buffer, freed when it goes out of scope unless release()d
 struct CudaFree {
@@ -34,6 +59,12 @@ struct DeviceScratch {
     void release(void *p) {
         auto it = std::find(ptrs.begin(), ptrs.end(), p);
         if (it != ptrs.end()) { cudaFree(p); ptrs.erase(it); }
+    }
+    // unlists p without freeing it: whoever it is handed to owns it from here on
+    template <class T> T *take(T *p) {
+        auto it = std::find(ptrs.begin(), ptrs.end(), (void *)p);
+        if (it != ptrs.end()) ptrs.erase(it);
+        return p;
     }
     void release_all() {
         for (void *p : ptrs) cudaFree(p);
@@ -74,7 +105,7 @@ struct DeviceImage {
     uint32_t n_super = 0;
     uint32_t sb_shift = kDefaultSuperShift;
 };
-int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift, DeviceImage &img, std::string &why);
+int build_image_on_device(const uint8_t *h_rle, uint64_t len, uint32_t sb_shift, DeviceImage &img);
 void free_device_image(DeviceImage &img);
 
 // ---- pair_builder.cu: one-step image (resident on the current device) -> pair image ----
@@ -87,7 +118,7 @@ struct PairImage {
 // `keep_codes` (optional): receives the per-position pair-code bytes (16 | code, or 0 when invalid;
 // npair * 96 of them, device memory the caller must cudaFree) -- the quad builder's input.
 int build_pair_image_on_device(int device, const IndexView &ix, const uint64_t start[kAlphabet], PairImage &img,
-                               std::string &why, int *launches, uint8_t **keep_codes = nullptr);
+                               uint8_t **keep_codes = nullptr);
 void free_pair_image(PairImage &img);
 
 // ---- quad_builder.cu: pair image + pair codes (resident on the current device) -> quad image ----
@@ -103,7 +134,7 @@ uint64_t quad_image_bytes(uint64_t total);
 // `keep_codes` (optional): receives the per-position quad codes (0x100 | code, or 0 when invalid; device
 // memory the caller must cudaFree) -- the oct builder's input.
 int build_quad_image_on_device(int device, const IndexView &ix, const uint8_t *d_codes2, QuadImage &img,
-                               std::string &why, int *launches, uint16_t **keep_codes = nullptr);
+                               uint16_t **keep_codes = nullptr);
 void free_quad_image(QuadImage &img);
 
 // ---- oct_builder.cu: quad image + quad codes (resident on the current device) -> oct image ----
@@ -120,14 +151,14 @@ uint64_t oct_image_bytes(uint64_t total, int shift);
 // the symbols is not ACGT (4 bytes per position, device memory the caller frees).  `d_codes4` = the quad builder's
 // keep_codes, OWNED by this call; `d_codes2` = the pair builder's keep_codes (borrowed).  N < 2^32 only.
 int build_oct_codes_on_device(int device, const IndexView &ix, uint16_t *d_codes4, const uint8_t *d_codes2,
-                              uint32_t **d_codes10, std::string &why, int *launches);
+                              uint32_t **d_codes10);
 // stage 1 without a quad image: the same codes by walking LF through the one-step blocks (any index; the only way when
 // N >= 2^32, whose quad image has no room)
-int build_oct_codes_by_walk(int device, const IndexView &ix, uint32_t **d_codes10, std::string &why, int *launches);
+int build_oct_codes_by_walk(int device, const IndexView &ix, uint32_t **d_codes10);
 // stage 2 (needs only the one-step blocks and the codes): the lines.  `requested_shift` 0 = automatic (layout.h).
 // When even the coarsest buckets exceed `max_bytes` nothing is built (img.lines stays null) and MSBWT_OK is returned.
 int build_oct_lines_on_device(int device, const IndexView &ix, const uint32_t *d_codes10, int requested_shift,
-                              uint64_t max_bytes, OctImage &img, std::string &why, int *launches);
+                              uint64_t max_bytes, OctImage &img);
 void free_oct_image(OctImage &img);
 
 // ---- fin_builder.cu: the oct builder's 10-symbol codes -> final-step lines (layout.h) ----
@@ -141,28 +172,23 @@ struct FinImage {
 uint64_t fin_image_bytes(uint64_t total, int shift, int lb);
 // stage 1 (needs the quad image and the one-step blocks): the kFinSyms-symbol code of every position,
 // `1 << kFinCodeBits | code` or 0 (8 bytes per position, device memory OWNED by stage 2)
-int build_fin_codes_on_device(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20,
-                              std::string &why, int *launches);
-int build_fin_codes_by_walk(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20,
-                            std::string &why, int *launches);
+int build_fin_codes_on_device(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20);
+int build_fin_codes_by_walk(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20);
 // stage 2 (needs only the codes, which it frees as soon as the run records exist): the lines
-int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20, int shift, int lb, FinImage &img,
-                              std::string &why, int *launches);
+int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20, int shift, int lb, FinImage &img);
 void free_fin_image(FinImage &img);
 
 // ---- bwt_build.cu: reads (device) -> RLE bytes of their multi-string BWT (device).  d_offsets == nullptr: n_reads reads
 // of read_len symbols each; otherwise read r = d_reads[d_offsets[r] .. d_offsets[r + 1]) and read_len = the longest ----
 int build_rle_bwt_on_device(const uint8_t *d_reads, const uint64_t *d_offsets, uint64_t n_reads, uint32_t read_len,
-                            uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, std::string &why, int *launches);
+                            uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total);
 // n symbol bytes (device) -> their msbwt RLE bytes (a cudaMalloc'd device buffer the caller frees); step 4b of the builder
-int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, uint64_t *rle_len, std::string &why,
-                         int *launches);
+int encode_rle_on_device(const uint8_t *d_bwt, uint64_t n, uint8_t **d_rle_out, uint64_t *rle_len);
 
 // ---- bwt_merge.cu: two RLE byte streams (host) -> RLE bytes of their Holt-McMillan merge (device buffer the caller
 // frees); *iterations = interleave passes run, the last of which changed nothing ----
 int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8_t *h_rle_b, uint64_t len_b,
-                             uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, uint32_t *iterations,
-                             std::string &why, int *launches);
+                             uint8_t **d_rle_out, uint64_t *rle_len, uint64_t *total, uint32_t *iterations);
 
 // ---- spectrum.cu: the k-mer spectrum of an index (one replica, on the current device): hist[nbins] (nbins may be 0)
 // and *n_kmers; when `kmers` is not null, also the k-mers with count >= min_count and their counts in co-lexicographic
@@ -170,13 +196,12 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
 // `canonical`: the same over canonical pairs {X, rc X} (msbwt_kmer_spectrum_canonical), whose reverse-complement
 // lookups run on the query path with `lanes` (the replica's kernel mapping) on the call's own stream and scratch.
 int kmer_spectrum_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
-                            uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers,
-                            std::string &why, int *launches);
+                            uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers);
 
-// return an msbwt_status; on failure `why` explains
-int validate_rle(const uint8_t *rle, uint64_t len, std::string &why);
-int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, HostImage &img, std::string &why);
-int read_npy_payload(const char *path, std::vector<uint8_t> &payload, std::string &why);
+// ---- loader.cu: RLE stream checks, the host builder (msbwt_debug_build_image) and the .npy reader ----
+int validate_rle(const uint8_t *rle, uint64_t len);
+int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, HostImage &img);
+int read_npy_payload(const char *path, std::vector<uint8_t> &payload);
 
 // ---- kernels.cu ----
 cudaError_t launch_pack_seed(const IndexView &ix, const uint8_t *d_syms, uint32_t k, uint64_t n, uint64_t *d_packed,
@@ -217,10 +242,9 @@ struct PackedLayout {
 inline PackedLayout packed_layout(const IndexView &ix, uint32_t k, uint64_t n) {
     return PackedLayout{n, words_for_k(k), index_is_wide(ix) ? 2u : 1u};
 }
-// `launches` (optional) is incremented once per kernel launch issued.  Runs the pair kernel over
-// list A (when the index has a pair image) and the one-step kernel over list B.
+// Runs the pair kernel over list A (when the index has a pair image) and the one-step kernel over list B.
 cudaError_t launch_count_packed(int device, const IndexView &ix, int lanes, const uint64_t *d_packed, uint32_t k,
-                                uint64_t n, uint64_t *d_out, cudaStream_t st, int *launches, bool with_b = true);
+                                uint64_t n, uint64_t *d_out, cudaStream_t st, bool with_b = true);
 // host-packed batches (hostpack.cpp): words[w * n + q], 2-bit ACGT symbols, the k-mer's last symbol in the
 // top bits of word 0 -> live list A (same scratch layout as launch_pack_seed produces)
 cudaError_t launch_seed_packed(const IndexView &ix, const uint64_t *d_words, uint32_t k, uint64_t n,
@@ -249,15 +273,15 @@ bool packed_batch_needs_list_b(const IndexView &ix, uint32_t k);
 uint32_t max_host_packed_k();  // seed_packed_kernel handles k-mers of at most this many symbols
 cudaError_t launch_count_bytes(int device, const IndexView &ix, const uint8_t *d_syms,
                                const uint64_t *d_offsets, uint64_t n, uint64_t *d_out, uint32_t *d_status,
-                               cudaStream_t st, int *launches);
+                               cudaStream_t st);
 cudaError_t launch_constrain_ranges(int device, const IndexView &ix, const uint8_t *d_sym, const uint64_t *d_l,
                                     const uint64_t *d_h, uint64_t n, uint64_t *d_out_l, uint64_t *d_out_h,
-                                    cudaStream_t st, int *launches);
+                                    cudaStream_t st);
 // ext_kernels.cu: the four constrain_range calls (A,C,G,T) of every range from one fetch of its blocks
 // (out[4 * i + j]); the k-mers of every window of every read (and their reverse complements) as symbol bytes;
 // per-window sums of the two strands' counts
 cudaError_t launch_constrain_fanout(int device, const IndexView &ix, const uint64_t *d_l, const uint64_t *d_h,
-                                    uint64_t n, uint64_t *d_out_l, uint64_t *d_out_h, cudaStream_t st, int *launches);
+                                    uint64_t n, uint64_t *d_out_l, uint64_t *d_out_h, cudaStream_t st);
 cudaError_t launch_expand_read_kmers(int device, const uint8_t *d_reads, uint32_t read_len, uint64_t n_reads, uint32_t k,
                                      uint32_t strands, uint8_t *d_syms, cudaStream_t st);
 cudaError_t launch_sum_strands(int device, const uint64_t *d_per_query, uint64_t n_windows, uint64_t *d_out, cudaStream_t st);

@@ -97,12 +97,13 @@ narrow_counts_kernel(const uint64_t *__restrict__ in, uint64_t n, uint32_t *__re
 cudaError_t launch_narrow_counts(int device, const uint64_t *d_in, uint64_t n, uint32_t *d_out, cudaStream_t st) {
     if (!n) return cudaSuccess;
     const unsigned grid = (unsigned)std::min<uint64_t>((n + 255) / 256, (uint64_t)sm_count(device) * 16);
+    g_launches++;
     narrow_counts_kernel<<<grid, 256, 0, st>>>(d_in, n, d_out);
     return cudaGetLastError();
 }
 
 cudaError_t launch_constrain_fanout(int device, const IndexView &ix, const uint64_t *d_l, const uint64_t *d_h,
-                                    uint64_t n, uint64_t *d_out_l, uint64_t *d_out_h, cudaStream_t st, int *launches) {
+                                    uint64_t n, uint64_t *d_out_l, uint64_t *d_out_h, cudaStream_t st) {
     for (uint64_t q0 = 0; q0 < n; q0 += kMaxPerLaunch) {
         const uint32_t m = (uint32_t)((n - q0) < kMaxPerLaunch ? (n - q0) : kMaxPerLaunch);
         if (index_is_wide(ix)) {
@@ -112,7 +113,7 @@ cudaError_t launch_constrain_fanout(int device, const IndexView &ix, const uint6
             const unsigned grid = persistent_grid(device, (const void *)constrain_fanout_kernel<false>, kCountThreads, m, kCountThreads);
             constrain_fanout_kernel<false><<<grid, kCountThreads, 0, st>>>(ix, d_l + q0, d_h + q0, m, d_out_l + 4 * q0, d_out_h + 4 * q0);
         }
-        if (launches) (*launches)++;
+        g_launches++;
         if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) return e;
     }
     return cudaSuccess;
@@ -123,6 +124,7 @@ cudaError_t launch_expand_read_kmers(int device, const uint8_t *d_reads, uint32_
     const uint64_t total = n_reads * (uint64_t)(read_len - k + 1) * strands;
     if (!total) return cudaSuccess;
     const unsigned grid = (unsigned)std::min<uint64_t>((total * k / 16 + 256) / 256, (uint64_t)sm_count(device) * 16);
+    g_launches++;
     expand_read_kmers_kernel<<<grid, 256, 0, st>>>(d_reads, read_len, n_reads, k, strands, d_syms);
     return cudaGetLastError();
 }
@@ -130,6 +132,7 @@ cudaError_t launch_expand_read_kmers(int device, const uint8_t *d_reads, uint32_
 cudaError_t launch_sum_strands(int device, const uint64_t *d_per_query, uint64_t n_windows, uint64_t *d_out, cudaStream_t st) {
     if (!n_windows) return cudaSuccess;
     const unsigned grid = (unsigned)std::min<uint64_t>((n_windows + 255) / 256, (uint64_t)sm_count(device) * 16);
+    g_launches++;
     sum_strands_kernel<<<grid, 256, 0, st>>>(d_per_query, n_windows, d_out);
     return cudaGetLastError();
 }

@@ -158,24 +158,7 @@ __global__ void __launch_bounds__(256) fin_lines_kernel(const uint64_t *__restri
     }
 }
 
-struct Scratch {
-    std::vector<void *> ptrs;
-    ~Scratch() { for (void *p : ptrs) cudaFree(p); }
-    template <class T> cudaError_t alloc(T **p, size_t count) {
-        cudaError_t e = cudaMalloc((void **)p, (count ? count : 1) * sizeof(T));
-        if (e == cudaSuccess) ptrs.push_back(*p);
-        return e;
-    }
-};
-
-#define F_TRY(expr)                                                                          \
-    do {                                                                                     \
-        cudaError_t e_ = (expr);                                                             \
-        if (e_ != cudaSuccess) {                                                             \
-            why = std::string("final-step image: ") + #expr + ": " + cudaGetErrorString(e_); \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;             \
-        }                                                                                    \
-    } while (0)
+#define F_TRY(e) CU_TRY_IN("final-step image: ", e)
 
 }  // namespace
 
@@ -191,10 +174,9 @@ static void fin_trace(const char *what) {
 }
 
 // Stage 1 (needs the quad image and the one-step blocks): code20 of every position, 8 bytes each
-int build_fin_codes_on_device(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20_out,
-                              std::string &why, int *launches) {
+int build_fin_codes_on_device(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20_out) {
     *d_codes20_out = nullptr;
-    if (!ix.quad || !d_codes10 || index_is_wide(ix)) { why = "final-step image: needs the quad image, the 10-symbol codes and 32-bit positions"; return MSBWT_EINVAL; }
+    if (!ix.quad || !d_codes10 || index_is_wide(ix)) return fail(MSBWT_EINVAL, "final-step image: needs the quad image, the 10-symbol codes and 32-bit positions");
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((ix.total + 255) / 256, (uint64_t)sms * 32));
@@ -202,13 +184,12 @@ int build_fin_codes_on_device(int device, const IndexView &ix, const uint32_t *d
     F_TRY(cudaMalloc((void **)&d_codes20, std::max<uint64_t>(1, ix.total) * sizeof(uint64_t)));
     fin_trace("codes");
     fin_code20_kernel<<<grid, 256>>>(ix, d_codes10, d_codes20);
-    if (launches) (*launches)++;
+    g_launches++;
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         cudaFree(d_codes20);
-        why = std::string("final-step image: code kernel: ") + cudaGetErrorString(e);
-        return MSBWT_ECUDA;
+        return fail(MSBWT_ECUDA, std::string("final-step image: code kernel: ") + cudaGetErrorString(e));
     }
     *d_codes20_out = d_codes20;
     return MSBWT_OK;
@@ -216,10 +197,9 @@ int build_fin_codes_on_device(int device, const IndexView &ix, const uint32_t *d
 
 // Stage 1 without a quad image (any index; the only way for one of 2^32 positions and more): `ix` needs only the one-step
 // blocks
-int build_fin_codes_by_walk(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20_out,
-                            std::string &why, int *launches) {
+int build_fin_codes_by_walk(int device, const IndexView &ix, const uint32_t *d_codes10, uint64_t **d_codes20_out) {
     *d_codes20_out = nullptr;
-    if (!d_codes10) { why = "final-step image: needs the 10-symbol codes"; return MSBWT_EINVAL; }
+    if (!d_codes10) return fail(MSBWT_EINVAL, "final-step image: needs the 10-symbol codes");
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((ix.total + 255) / 256, (uint64_t)sms * 32));
@@ -228,37 +208,35 @@ int build_fin_codes_by_walk(int device, const IndexView &ix, const uint32_t *d_c
     fin_trace("codes (walk)");
     if (index_is_wide(ix)) fin_code_walk_kernel<true><<<grid, 256>>>(ix, d_codes10, d_codes20);
     else fin_code_walk_kernel<false><<<grid, 256>>>(ix, d_codes10, d_codes20);
-    if (launches) (*launches)++;
+    g_launches++;
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         cudaFree(d_codes20);
-        why = std::string("final-step image: code walk kernel: ") + cudaGetErrorString(e);
-        return MSBWT_ECUDA;
+        return fail(MSBWT_ECUDA, std::string("final-step image: code walk kernel: ") + cudaGetErrorString(e));
     }
     *d_codes20_out = d_codes20;
     return MSBWT_OK;
 }
 
 // Stage 2 (needs nothing but the codes, which it OWNS and frees as soon as the run records exist): the lines
-int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20_in, int shift, int lb, FinImage &img,
-                              std::string &why, int *launches) {
+int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20_in, int shift, int lb, FinImage &img) {
     DevicePtr<uint64_t> codes20(d_codes20_in);
-    if (!d_codes20_in) { why = "final-step image: no position codes"; return MSBWT_EINVAL; }
-    if (shift < 8 || shift > 16 || lb < kFinCodeBits - kFinTagBits || lb > 20) { why = "final-step image: bucket shift 8..16, lines per bucket 2^12..2^20"; return MSBWT_EINVAL; }
-    if (((((total >> shift) + 1) << lb) >> (64 - kFinTagBits)) != 0) { why = "final-step image: line index and tag do not fit one 64-bit sort key"; return MSBWT_EINVAL; }
+    if (!d_codes20_in) return fail(MSBWT_EINVAL, "final-step image: no position codes");
+    if (shift < 8 || shift > 16 || lb < kFinCodeBits - kFinTagBits || lb > 20) return fail(MSBWT_EINVAL, "final-step image: bucket shift 8..16, lines per bucket 2^12..2^20");
+    if (((((total >> shift) + 1) << lb) >> (64 - kFinTagBits)) != 0) return fail(MSBWT_EINVAL, "final-step image: line index and tag do not fit one 64-bit sort key");
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((total + 255) / 256, (uint64_t)sms * 32));
     const uint64_t *d_codes20 = codes20.get();
 
-    Scratch tmp;
+    DeviceScratch tmp;
     unsigned long long *d_stat = nullptr;  // [0] records, [1] emit cursor, [2] overflowed lines
     F_TRY(tmp.alloc(&d_stat, 3));
     F_TRY(cudaMemsetAsync(d_stat, 0, 3 * sizeof(unsigned long long)));
     fin_count_runs_kernel<<<grid, 256>>>(d_codes20, total, (uint32_t)shift, d_stat);
     F_TRY(cudaGetLastError());
-    if (launches) (*launches)++;
+    g_launches++;
     unsigned long long n_runs = 0;
     F_TRY(cudaMemcpy(&n_runs, d_stat, sizeof(n_runs), cudaMemcpyDeviceToHost));
 
@@ -276,7 +254,7 @@ int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20_in
         fin_emit_kernel<<<grid, 256>>>(d_codes20, total, (uint32_t)shift, (uint32_t)lb, k0, v0, d_stat + 1);
         F_TRY(cudaGetLastError());
         F_TRY(cudaDeviceSynchronize());
-        if (launches) (*launches)++;
+        g_launches++;
     }
     codes20.reset();  // the records carry everything from here on
     F_TRY(cudaMalloc((void **)&img.lines, nlines * kFinLineBytes));
@@ -298,7 +276,7 @@ int build_fin_lines_on_device(int device, uint64_t total, uint64_t *d_codes20_in
         fin_trace("lines");
         fin_lines_kernel<<<grid, 256>>>(keys.Current(), vals.Current(), n_runs, reinterpret_cast<uint32_t *>(img.lines), d_stat + 2);
         F_TRY(cudaGetLastError());
-        if (launches) (*launches) += 2;
+        g_launches += 2;
     }
     unsigned long long over = 0;
     F_TRY(cudaMemcpy(&over, d_stat + 2, sizeof(over), cudaMemcpyDeviceToHost));

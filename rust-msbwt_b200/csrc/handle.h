@@ -1,9 +1,8 @@
-// handle.h -- what an `msbwt_index` handle owns (per-device replicas, staging lanes, scratch) and the error /
-// launch-count plumbing shared by the translation units that implement the C ABI: capi.cu (construction, accessors,
-// device-buffer entry points, inspection) and hostpath.cu (host-buffer entry points: the chunk pipelines and the
-// multi-GPU batch split).
+// handle.h -- what an `msbwt_index` handle owns (per-device replicas, staging lanes, scratch), shared by the
+// translation units that implement the C ABI: capi.cu (construction, accessors, device-buffer entry points,
+// inspection) and hostpath.cu (host-buffer entry points: the chunk pipelines and the multi-GPU batch split).  Errors
+// and launch counts are reported through engine.h, by the function that meets them.
 #pragma once
-#include <atomic>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -14,28 +13,6 @@
 #include "hostpack.h"
 
 namespace msbwt {
-
-extern thread_local std::string g_last_error;
-extern thread_local int g_call_launches;
-extern std::atomic<uint64_t> g_launches;
-
-inline void flush_launches() {
-    g_launches += (uint64_t)g_call_launches;
-    g_call_launches = 0;
-}
-
-inline int fail(int code, const std::string &msg) {
-    g_last_error = msg;
-    return code;
-}
-
-#define CU_TRY(expr)                                                                              \
-    do {                                                                                          \
-        cudaError_t e_ = (expr);                                                                  \
-        if (e_ != cudaSuccess)                                                                    \
-            return fail(e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA,             \
-                        std::string(#expr) + ": " + cudaGetErrorString(e_));                      \
-    } while (0)
 
 // grow-only device buffer
 struct DevBuf {

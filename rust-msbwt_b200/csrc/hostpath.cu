@@ -61,7 +61,6 @@ int run_on_replicas(const msbwt_index *idx, uint64_t n, F &&fn) {
         }
         res[d].rc = rc;
         if (rc != MSBWT_OK) res[d].err = g_last_error;
-        flush_launches();
     };
     if (ndev == 1) {
         body(0);
@@ -202,12 +201,10 @@ int stage_input(Lane &ln, HostStage &hs, const void *src, size_t bytes, const vo
 // search the lane's packed scratch and send the counts of queries [b, b + m) home
 int search_and_copy_out(Replica &rep, Lane &ln, uint32_t k, uint64_t b, uint64_t m, HostStage &hs, bool with_b, Xfer &x) {
     CU_TRY(launch_count_packed(rep.device, rep.view, rep.lanes, ln.packed.as<uint64_t>(), k, m, ln.out_a.as<uint64_t>(),
-                               ln.stream, &g_call_launches, with_b));
-    flush_launches();
+                               ln.stream, with_b));
     const void *d_res = ln.out_a.p;
     if (hs.dst.o32) {
         CU_TRY(launch_narrow_counts(rep.device, ln.out_a.as<uint64_t>(), m, ln.out_b.as<uint32_t>(), ln.stream));
-        g_launches++;
         d_res = ln.out_b.p;
     }
     void *h_res = hs.dst.o32 ? (void *)(hs.dst.o32 + b) : (void *)(hs.dst.o64 + b);
@@ -258,7 +255,6 @@ int bytes_route(Replica &rep, size_t ndev, const uint8_t *syms, uint32_t k, Slic
         }
         CU_TRY(launch_pack_seed(rep.view, ln.in_a.as<uint8_t>(), k, m, ln.packed.as<uint64_t>(), ln.out_a.as<uint64_t>(),
                                 rep.d_status + li, ln.stream));
-        g_launches++;
         x.h2d += m * k;
         if (int rc = search_and_copy_out(rep, ln, k, b, m, hs, true, x); rc != MSBWT_OK) return rc;
     }
@@ -325,7 +321,6 @@ int packed_route(Replica &rep, size_t ndev, const uint8_t *syms, uint32_t k, uin
             CU_TRY(cudaEventRecord(ln.h2d_done, ln.stream));
             CU_TRY(launch_pack_seed(rep.view, ln.in_a.as<uint8_t>(), k, m, ln.packed.as<uint64_t>(), ln.out_a.as<uint64_t>(),
                                     rep.d_status + raw_lane, ln.stream));
-            g_launches++;
             x.h2d += m * k;
             if (int rc = search_and_copy_out(rep, ln, k, b, m, hs, true, x); rc != MSBWT_OK) return rc;
             continue;
@@ -341,7 +336,6 @@ int packed_route(Replica &rep, size_t ndev, const uint8_t *syms, uint32_t k, uin
         CU_TRY(cudaMemcpyAsync(ln.in_b.p, stage, m * nw * sizeof(uint64_t), cudaMemcpyHostToDevice, ln.stream));
         CU_TRY(cudaEventRecord(ln.h2d_done, ln.stream));
         CU_TRY(launch_seed_packed(rep.view, ln.in_b.as<uint64_t>(), k, m, ln.packed.as<uint64_t>(), ln.out_a.as<uint64_t>(), ln.stream));
-        g_launches++;
         x.h2d += m * nw * sizeof(uint64_t);
         if (int rc = search_and_copy_out(rep, ln, k, b, m, hs, with_b, x); rc != MSBWT_OK) return rc;
     }
@@ -414,7 +408,6 @@ int u64_route(Replica &rep, size_t ndev, const uint64_t *kmers, uint32_t k, Slic
         if (hs.in) CU_TRY(cudaEventRecord(ln.h2d_done, ln.stream));
         if (trace) cudaEventRecord(mk.e[1], ln.stream);
         CU_TRY(launch_seed_u64(rep.view, ln.in_b.as<uint64_t>(), k, m, ln.packed.as<uint64_t>(), ln.out_a.as<uint64_t>(), ln.stream));
-        g_launches++;
         x.h2d += m * sizeof(uint64_t);
         if (int rc = search_and_copy_out(rep, ln, k, b, m, hs, with_b, x); rc != MSBWT_OK) return rc;
         if (trace) {
@@ -553,8 +546,7 @@ extern "C" int msbwt_count_kmers(const msbwt_index *idx, const uint8_t *syms, co
             // the kernel indexes syms with absolute offsets: bias the base pointer instead of rewriting them
             const uint8_t *biased = ln.in_a.as<uint8_t>() - offsets[b];
             CU_TRY(launch_count_bytes(rep.device, rep.view, biased, ln.in_b.as<uint64_t>(), m, ln.out_a.as<uint64_t>(),
-                                      rep.d_status + (round & 1), ln.stream, &g_call_launches));
-            flush_launches();
+                                      rep.d_status + (round & 1), ln.stream));
             CU_TRY(cudaMemcpyAsync(out + b, ln.out_a.p, m * sizeof(uint64_t), cudaMemcpyDeviceToHost, ln.stream));
             x.h2d += nbytes + (m + 1) * sizeof(uint64_t);
             x.d2h += m * sizeof(uint64_t);
@@ -595,8 +587,7 @@ extern "C" int msbwt_constrain_ranges(const msbwt_index *idx, const uint8_t *sym
             CU_TRY(cudaMemcpyAsync(ln.in_b.p, l + b, m * sizeof(uint64_t), cudaMemcpyHostToDevice, ln.stream));
             CU_TRY(cudaMemcpyAsync(ln.in_c.p, h + b, m * sizeof(uint64_t), cudaMemcpyHostToDevice, ln.stream));
             CU_TRY(launch_constrain_ranges(rep.device, rep.view, ln.in_a.as<uint8_t>(), ln.in_b.as<uint64_t>(), ln.in_c.as<uint64_t>(), m,
-                                           ln.out_a.as<uint64_t>(), ln.out_b.as<uint64_t>(), ln.stream, &g_call_launches));
-            flush_launches();
+                                           ln.out_a.as<uint64_t>(), ln.out_b.as<uint64_t>(), ln.stream));
             CU_TRY(cudaMemcpyAsync(out_l + b, ln.out_a.p, m * sizeof(uint64_t), cudaMemcpyDeviceToHost, ln.stream));
             CU_TRY(cudaMemcpyAsync(out_h + b, ln.out_b.p, m * sizeof(uint64_t), cudaMemcpyDeviceToHost, ln.stream));
         }
@@ -633,8 +624,7 @@ extern "C" int msbwt_constrain_ranges_fanout(const msbwt_index *idx, const uint6
             CU_TRY(cudaMemcpyAsync(ln.in_b.p, l + b, m * sizeof(uint64_t), cudaMemcpyHostToDevice, ln.stream));
             CU_TRY(cudaMemcpyAsync(ln.in_c.p, h + b, m * sizeof(uint64_t), cudaMemcpyHostToDevice, ln.stream));
             CU_TRY(launch_constrain_fanout(rep.device, rep.view, ln.in_b.as<uint64_t>(), ln.in_c.as<uint64_t>(), m,
-                                           ln.out_a.as<uint64_t>(), ln.out_b.as<uint64_t>(), ln.stream, &g_call_launches));
-            flush_launches();
+                                           ln.out_a.as<uint64_t>(), ln.out_b.as<uint64_t>(), ln.stream));
             CU_TRY(cudaMemcpyAsync(out_l + 4 * b, ln.out_a.p, 4 * m * sizeof(uint64_t), cudaMemcpyDeviceToHost, ln.stream));
             CU_TRY(cudaMemcpyAsync(out_h + 4 * b, ln.out_b.p, 4 * m * sizeof(uint64_t), cudaMemcpyDeviceToHost, ln.stream));
         }
@@ -674,16 +664,12 @@ extern "C" int msbwt_count_read_kmers(const msbwt_index *idx, const uint8_t *rea
             uint32_t *flag = rep.d_status + (c & 1);
             CU_TRY(cudaMemcpyAsync(ln.in_a.p, reads + b * read_len, m * read_len, cudaMemcpyHostToDevice, ln.stream));
             CU_TRY(launch_expand_read_kmers(rep.device, ln.in_a.as<uint8_t>(), read_len, m, k, strands, ln.in_b.as<uint8_t>(), ln.stream));
-            g_launches++;
             CU_TRY(launch_pack_seed(rep.view, ln.in_b.as<uint8_t>(), k, nq, ln.packed.as<uint64_t>(), ln.out_a.as<uint64_t>(), flag, ln.stream));
-            g_launches++;
             CU_TRY(launch_count_packed(rep.device, rep.view, rep.lanes, ln.packed.as<uint64_t>(), k, nq, ln.out_a.as<uint64_t>(),
-                                       ln.stream, &g_call_launches));
-            flush_launches();
+                                       ln.stream));
             const uint64_t *res = ln.out_a.as<uint64_t>();
             if (strands == 2) {
                 CU_TRY(launch_sum_strands(rep.device, ln.out_a.as<uint64_t>(), m * windows, ln.out_b.as<uint64_t>(), ln.stream));
-                g_launches++;
                 res = ln.out_b.as<uint64_t>();
             }
             CU_TRY(cudaMemcpyAsync(out + b * windows, res, m * windows * sizeof(uint64_t), cudaMemcpyDeviceToHost, ln.stream));

@@ -560,6 +560,7 @@ static int current_device() {
 cudaError_t launch_pack_seed(const IndexView &ix, const uint8_t *d_syms, uint32_t k, uint64_t n, uint64_t *d_packed,
                              uint64_t *d_out, uint32_t *d_status, cudaStream_t st) {
     if (!n) return cudaSuccess;
+    g_launches++;  // one kernel, whichever route
     // a suffix-table entry + exactly kFinSyms symbols (k = 31, 32): pack, seed and answer in one regular kernel
     if (final_fast_path_applies(ix, k, d_syms, 0))
         return launch_pack_seed_final(current_device(), ix, d_syms, 0, k, n, d_packed, d_out, d_status, st);
@@ -613,7 +614,7 @@ static cudaError_t launch_count_pair_t(int device, const IndexView &ix, const ui
 // one-step kernel on 2-bit words;
 // list B: the one-step kernel on 3-bit words (`with_b` false: the caller knows list B is empty).
 cudaError_t launch_count_packed(int device, const IndexView &ix, int lanes, const uint64_t *d_packed, uint32_t k,
-                                uint64_t n, uint64_t *d_out, cudaStream_t st, int *launches, bool with_b) {
+                                uint64_t n, uint64_t *d_out, cudaStream_t st, bool with_b) {
     if (!n) return cudaSuccess;
     if (n > kMaxPerLaunch) return cudaErrorInvalidValue;
     const PackedLayout lay = packed_layout(ix, k, n);
@@ -625,16 +626,17 @@ cudaError_t launch_count_packed(int device, const IndexView &ix, int lanes, cons
                         : launch_count_pair_t<false>(device, ix, d_packed, lay, k, d_out, st);
     else
         e = launch_one_step<2>(device, ix, lanes, d_packed, lay, k, d_out, st);
-    if (launches) (*launches)++;
+    g_launches++;
     if (e != cudaSuccess || !with_b) return e;
     e = launch_one_step<3>(device, ix, lanes, d_packed, lay, k, d_out, st);
-    if (launches) (*launches)++;
+    g_launches++;
     return e;
 }
 
 cudaError_t launch_seed_packed(const IndexView &ix, const uint64_t *d_words, uint32_t k, uint64_t n,
                                uint64_t *d_packed, uint64_t *d_out, cudaStream_t st) {
     if (!n) return cudaSuccess;
+    g_launches++;  // one kernel, whichever route
     if (k <= 32u && final_fast_path_applies(ix, k, d_words, 2))  // one word per k-mer: word 0 is the whole k-mer
         return launch_pack_seed_final(current_device(), ix, d_words, 2, k, n, d_packed, d_out, nullptr, st);
     const PackedLayout lay = packed_layout(ix, k, n);
@@ -651,6 +653,7 @@ cudaError_t launch_seed_u64(const IndexView &ix, const uint64_t *d_kmers, uint32
                             uint64_t *d_packed, uint64_t *d_out, cudaStream_t st) {
     if (!n) return cudaSuccess;
     if (!k || k > 32u) return cudaErrorInvalidValue;
+    g_launches++;  // one kernel, whichever route
     if (final_fast_path_applies(ix, k, d_kmers, 1))
         return launch_pack_seed_final(current_device(), ix, d_kmers, 1, k, n, d_packed, d_out, nullptr, st);
     const PackedLayout lay = packed_layout(ix, k, n);
@@ -672,6 +675,7 @@ bool packed_batch_needs_list_b(const IndexView &ix, uint32_t k) {
 
 cudaError_t launch_table_extend(int device, const IndexView &ix, const void *d_parent, void *d_child,
                                 uint32_t n_child, cudaStream_t st) {
+    g_launches++;
     if (is_wide(ix)) {
         const unsigned grid = persistent_grid(device, (const void *)table_extend_kernel<true>, kCountThreads, n_child, kCountThreads);
         table_extend_kernel<true><<<grid, kCountThreads, 0, st>>>(ix, d_parent, d_child, n_child);
@@ -686,7 +690,7 @@ bool index_is_wide(const IndexView &ix) { return is_wide(ix); }
 
 cudaError_t launch_count_bytes(int device, const IndexView &ix, const uint8_t *d_syms,
                                const uint64_t *d_offsets, uint64_t n, uint64_t *d_out, uint32_t *d_status,
-                               cudaStream_t st, int *launches) {
+                               cudaStream_t st) {
     for (uint64_t q0 = 0; q0 < n; q0 += kMaxPerLaunch) {
         const uint32_t m = (uint32_t)((n - q0) < kMaxPerLaunch ? (n - q0) : kMaxPerLaunch);
         if (is_wide(ix)) {
@@ -696,7 +700,7 @@ cudaError_t launch_count_bytes(int device, const IndexView &ix, const uint8_t *d
             const unsigned grid = persistent_grid(device, (const void *)count_kmers_bytes_kernel<false>, kCountThreads, m, kCountThreads);
             count_kmers_bytes_kernel<false><<<grid, kCountThreads, 0, st>>>(ix, d_syms, d_offsets + q0, m, d_out + q0, d_status);
         }
-        if (launches) (*launches)++;
+        g_launches++;
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }
@@ -705,7 +709,7 @@ cudaError_t launch_count_bytes(int device, const IndexView &ix, const uint8_t *d
 
 cudaError_t launch_constrain_ranges(int device, const IndexView &ix, const uint8_t *d_sym, const uint64_t *d_l,
                                     const uint64_t *d_h, uint64_t n, uint64_t *d_out_l, uint64_t *d_out_h,
-                                    cudaStream_t st, int *launches) {
+                                    cudaStream_t st) {
     for (uint64_t q0 = 0; q0 < n; q0 += kMaxPerLaunch) {
         const uint32_t m = (uint32_t)((n - q0) < kMaxPerLaunch ? (n - q0) : kMaxPerLaunch);
         if (is_wide(ix)) {
@@ -715,7 +719,7 @@ cudaError_t launch_constrain_ranges(int device, const IndexView &ix, const uint8
             const unsigned grid = persistent_grid(device, (const void *)constrain_ranges_kernel<false>, kCountThreads, m, kCountThreads);
             constrain_ranges_kernel<false><<<grid, kCountThreads, 0, st>>>(ix, d_sym + q0, d_l + q0, d_h + q0, m, d_out_l + q0, d_out_h + q0);
         }
-        if (launches) (*launches)++;
+        g_launches++;
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return e;
     }
@@ -731,6 +735,7 @@ cudaError_t launch_gather(int device, const void *d_buf, uint64_t buf_bytes, uin
     const uint32_t mask = (uint32_t)(n_granules - 1);
     const unsigned grid = (unsigned)sm_count(device) * 8u;
     const uint4 *buf = (const uint4 *)d_buf;
+    g_launches++;
     switch (granule) {
         case 32: gather_kernel<2><<<grid, 256, 0, st>>>(buf, mask, (uint32_t)n_gathers, (uint32_t)seed, d_sink); break;
         case 64: gather_kernel<4><<<grid, 256, 0, st>>>(buf, mask, (uint32_t)n_gathers, (uint32_t)seed, d_sink); break;

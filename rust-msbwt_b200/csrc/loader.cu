@@ -81,30 +81,28 @@ struct ImageWriter {
 // Format check shared by both builders, done on the host before any device is touched so that a
 // malformed stream is MSBWT_EFORMAT regardless of the machine: symbol >= 6 (the reference panics
 // indexing symbol_counts, src/rle_bwt.rs:371) or a single run of 13+ bytes (>= 2^60 symbols).
-int validate_rle(const uint8_t *rle, uint64_t len, std::string &why) {
-    if (len && !rle) { why = "rle is NULL"; return MSBWT_EINVAL; }
+int validate_rle(const uint8_t *rle, uint64_t len) {
+    if (len && !rle) return fail(MSBWT_EINVAL, "rle is NULL");
     uint8_t prev = 255;
     int digits = 0;
     uint64_t total = 0;  // every addend is below 2^60 and the sum is checked after each: it cannot wrap unnoticed
     for (uint64_t i = 0; i < len; i++) {
         const uint8_t c = rle[i] & 7u;
-        if (c >= kAlphabet) {
-            why = "RLE byte " + std::to_string(i) + " has symbol " + std::to_string(c) + " (>= 6)";
-            return MSBWT_EFORMAT;
-        }
+        if (c >= kAlphabet)
+            return fail(MSBWT_EFORMAT, "RLE byte " + std::to_string(i) + " has symbol " + std::to_string(c) + " (>= 6)");
         digits = (c == prev) ? digits + 1 : 0;
         prev = c;
-        if (digits >= 12) { why = "run longer than 2^60 symbols"; return MSBWT_EFORMAT; }
+        if (digits >= 12) return fail(MSBWT_EFORMAT, "run longer than 2^60 symbols");
         total += (uint64_t)(rle[i] >> 3) << (5 * digits);
-        if (total >> 62) { why = "BWT longer than 2^62 symbols"; return MSBWT_EFORMAT; }  // (the device builder's u64 prefix sums stay exact)
+        if (total >> 62) return fail(MSBWT_EFORMAT, "BWT longer than 2^62 symbols");  // (the device builder's u64 prefix sums stay exact)
     }
     return MSBWT_OK;
 }
 
-int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, HostImage &img, std::string &why) {
-    if (len && !rle) { why = "rle is NULL"; return MSBWT_EINVAL; }
+int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, HostImage &img) {
+    if (len && !rle) return fail(MSBWT_EINVAL, "rle is NULL");
     if (sb_shift == 0) sb_shift = kDefaultSuperShift;
-    if (sb_shift > (uint32_t)kDefaultSuperShift) { why = "superblock_shift > 25 would overflow the u32 block counters"; return MSBWT_EINVAL; }
+    if (sb_shift > (uint32_t)kDefaultSuperShift) return fail(MSBWT_EINVAL, "superblock_shift > 25 would overflow the u32 block counters");
 
     // pass 1: symbol totals (the C array) -- src/rle_bwt.rs:352-384
     uint8_t prev = 255;
@@ -112,17 +110,15 @@ int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, Ho
     uint64_t total = 0;
     for (uint64_t i = 0; i < len; i++) {
         const uint8_t v = rle[i], c = v & 7u;
-        if (c >= kAlphabet) {
-            why = "RLE byte " + std::to_string(i) + " has symbol " + std::to_string(c) + " (>= 6)";
-            return MSBWT_EFORMAT;
-        }
+        if (c >= kAlphabet)
+            return fail(MSBWT_EFORMAT, "RLE byte " + std::to_string(i) + " has symbol " + std::to_string(c) + " (>= 6)");
         digits = (c == prev) ? digits + 1 : 0;
         prev = c;
-        if (digits >= 12) { why = "run longer than 2^60 symbols"; return MSBWT_EFORMAT; }
+        if (digits >= 12) return fail(MSBWT_EFORMAT, "run longer than 2^60 symbols");
         const uint64_t add = (uint64_t)(v >> 3) << (5 * digits);
         img.counts[c] += add;
         total += add;
-        if (total >> 62) { why = "BWT longer than 2^62 symbols"; return MSBWT_EFORMAT; }
+        if (total >> 62) return fail(MSBWT_EFORMAT, "BWT longer than 2^62 symbols");
     }
     uint64_t sum = 0;
     for (int s = 0; s < kAlphabet; s++) { img.start[s] = sum; sum += img.counts[s]; }
@@ -135,8 +131,7 @@ int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, Ho
         img.aux.assign(img.nblocks * 2, 0u);
         img.cbase.assign((size_t)img.n_super * 8, 0ull);
     } catch (const std::bad_alloc &) {
-        why = "out of host memory for the block image";
-        return MSBWT_ENOMEM;
+        return fail(MSBWT_ENOMEM, "out of host memory for the block image");
     }
 
     // pass 2: runs -> blocks
@@ -268,34 +263,31 @@ struct DictReader {
 
 }  // namespace
 
-int read_npy_payload(const char *path, std::vector<uint8_t> &payload, std::string &why) {
-    if (!path) { why = "path is NULL"; return MSBWT_EINVAL; }
+int read_npy_payload(const char *path, std::vector<uint8_t> &payload) {
+    if (!path) return fail(MSBWT_EINVAL, "path is NULL");
     FILE *f = fopen(path, "rb");
-    if (!f) { why = std::string("cannot open ") + path + ": " + strerror(errno); return MSBWT_EIO; }
+    if (!f) return fail(MSBWT_EIO, std::string("cannot open ") + path + ": " + strerror(errno));
     struct Closer { FILE *f; ~Closer() { fclose(f); } } closer{f};
-    if (fseek(f, 0, SEEK_END) != 0) { why = "cannot seek"; return MSBWT_EIO; }
+    if (fseek(f, 0, SEEK_END) != 0) return fail(MSBWT_EIO, "cannot seek");
     const long long full = ftell(f);
     rewind(f);
     uint8_t fixed[10];
-    if (fread(fixed, 1, 10, f) != 10) { why = "file shorter than the 10-byte npy preamble"; return MSBWT_EFORMAT; }
+    if (fread(fixed, 1, 10, f) != 10) return fail(MSBWT_EFORMAT, "file shorter than the 10-byte npy preamble");
     // magic and version deliberately unchecked (src/rle_bwt.rs:96)
     const size_t header_len = (size_t)fixed[8] + 256u * (size_t)fixed[9];
     size_t skip = 10 + header_len;
     if (skip % 16) skip = (skip / 16 + 1) * 16;
     std::vector<char> hdr(skip - 10);
-    if (fread(hdr.data(), 1, hdr.size(), f) != hdr.size()) {
-        why = "could not read bytes 10-" + std::to_string(skip) + " of the header";
-        return MSBWT_EIO;
-    }
+    if (fread(hdr.data(), 1, hdr.size(), f) != hdr.size())
+        return fail(MSBWT_EIO, "could not read bytes 10-" + std::to_string(skip) + " of the header");
     DictReader rd{hdr.data(), hdr.data() + hdr.size()};
-    if (!rd.parse()) { why = "could not parse the npy header dict / shape"; return MSBWT_EFORMAT; }
+    if (!rd.parse()) return fail(MSBWT_EFORMAT, "could not parse the npy header dict / shape");
     const uint64_t disk = (uint64_t)full - skip;
-    if (rd.shape0 != disk) {
-        why = "header indicates shape of " + std::to_string(rd.shape0) + ", but remaining file size is " + std::to_string(disk);
-        return MSBWT_EIO;
-    }
-    try { payload.resize(disk); } catch (const std::bad_alloc &) { why = "out of host memory"; return MSBWT_ENOMEM; }
-    if (disk && fread(payload.data(), 1, disk, f) != disk) { why = "short read of the BWT body"; return MSBWT_EIO; }
+    if (rd.shape0 != disk)
+        return fail(MSBWT_EIO, "header indicates shape of " + std::to_string(rd.shape0) + ", but remaining file size is " +
+                                   std::to_string(disk));
+    try { payload.resize(disk); } catch (const std::bad_alloc &) { return fail(MSBWT_ENOMEM, "out of host memory"); }
+    if (disk && fread(payload.data(), 1, disk, f) != disk) return fail(MSBWT_EIO, "short read of the BWT body");
     return MSBWT_OK;
 }
 

@@ -156,24 +156,7 @@ __global__ void __launch_bounds__(256) oct_stamp_kernel(const uint64_t *__restri
     }
 }
 
-struct Scratch {
-    std::vector<void *> ptrs;
-    ~Scratch() { for (void *p : ptrs) cudaFree(p); }
-    template <class T> cudaError_t alloc(T **p, size_t count) {
-        cudaError_t e = cudaMalloc((void **)p, (count ? count : 1) * sizeof(T));
-        if (e == cudaSuccess) ptrs.push_back(*p);
-        return e;
-    }
-};
-
-#define O_TRY(expr)                                                                        \
-    do {                                                                                   \
-        cudaError_t e_ = (expr);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            why = std::string("oct image: ") + #expr + ": " + cudaGetErrorString(e_);      \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;           \
-        }                                                                                  \
-    } while (0)
+#define O_TRY(e) CU_TRY_IN("oct image: ", e)
 
 }  // namespace
 
@@ -185,24 +168,23 @@ uint64_t oct_image_bytes(uint64_t total, int shift) {
 // one-step blocks and the quad image; `d_codes4` (the quad builder's keep_codes) is OWNED by this call and freed as
 // soon as the codes exist; `d_codes2` (the pair builder's keep_codes) is borrowed.
 int build_oct_codes_on_device(int device, const IndexView &ix, uint16_t *d_codes4, const uint8_t *d_codes2,
-                              uint32_t **d_codes10, std::string &why, int *launches) {
+                              uint32_t **d_codes10) {
     DevicePtr<uint16_t> codes4(d_codes4);
     *d_codes10 = nullptr;
-    if (!ix.quad || !d_codes4 || !d_codes2) { why = "oct image: needs the quad image, its codes and the pair codes"; return MSBWT_EINVAL; }
-    if (index_is_wide(ix)) { why = "oct image: only for indexes with 32-bit positions (N < 2^32, one superblock)"; return MSBWT_EINVAL; }
+    if (!ix.quad || !d_codes4 || !d_codes2) return fail(MSBWT_EINVAL, "oct image: needs the quad image, its codes and the pair codes");
+    if (index_is_wide(ix)) return fail(MSBWT_EINVAL, "oct image: only for indexes with 32-bit positions (N < 2^32, one superblock)");
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((ix.total + 255) / 256, (uint64_t)sms * 32));
     uint32_t *d_codes8 = nullptr;
     O_TRY(cudaMalloc((void **)&d_codes8, std::max<uint64_t>(1, ix.total) * sizeof(uint32_t)));
     oct_code8_kernel<<<grid, 256>>>(ix, d_codes4, d_codes2, d_codes8);
-    if (launches) (*launches)++;
+    g_launches++;
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         cudaFree(d_codes8);
-        why = std::string("oct image: code kernel: ") + cudaGetErrorString(e);
-        return MSBWT_ECUDA;
+        return fail(MSBWT_ECUDA, std::string("oct image: code kernel: ") + cudaGetErrorString(e));
     }
     *d_codes10 = d_codes8;
     return MSBWT_OK;
@@ -210,7 +192,7 @@ int build_oct_codes_on_device(int device, const IndexView &ix, uint16_t *d_codes
 
 // Stage 1 without a quad image (any index; the only way for one of 2^32 positions and more): the codes by walking LF
 // through the one-step blocks -- `ix` needs nothing else.
-int build_oct_codes_by_walk(int device, const IndexView &ix, uint32_t **d_codes10, std::string &why, int *launches) {
+int build_oct_codes_by_walk(int device, const IndexView &ix, uint32_t **d_codes10) {
     *d_codes10 = nullptr;
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
@@ -219,13 +201,12 @@ int build_oct_codes_by_walk(int device, const IndexView &ix, uint32_t **d_codes1
     O_TRY(cudaMalloc((void **)&d_codes, std::max<uint64_t>(1, ix.total) * sizeof(uint32_t)));
     if (index_is_wide(ix)) oct_code_walk_kernel<true><<<grid, 256>>>(ix, d_codes);
     else oct_code_walk_kernel<false><<<grid, 256>>>(ix, d_codes);
-    if (launches) (*launches)++;
+    g_launches++;
     cudaError_t e = cudaGetLastError();
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         cudaFree(d_codes);
-        why = std::string("oct image: code walk kernel: ") + cudaGetErrorString(e);
-        return MSBWT_ECUDA;
+        return fail(MSBWT_ECUDA, std::string("oct image: code walk kernel: ") + cudaGetErrorString(e));
     }
     *d_codes10 = d_codes;
     return MSBWT_OK;
@@ -235,18 +216,17 @@ int build_oct_codes_by_walk(int device, const IndexView &ix, uint32_t **d_codes1
 // the caller may already have dropped it.  `requested_shift` 0 = automatic (layout.h).  When even the coarsest
 // buckets exceed `max_bytes` nothing is built (img.lines stays null) and MSBWT_OK is returned.
 int build_oct_lines_on_device(int device, const IndexView &ix, const uint32_t *d_codes8, int requested_shift,
-                              uint64_t max_bytes, OctImage &img, std::string &why, int *launches) {
-    if (!d_codes8) { why = "oct image: needs the position codes"; return MSBWT_EINVAL; }
-    if ((ix.total >> 40) != 0) { why = "oct image: a line's checkpoint holds 40 bits (N < 2^40)"; return MSBWT_EINVAL; }
+                              uint64_t max_bytes, OctImage &img) {
+    if (!d_codes8) return fail(MSBWT_EINVAL, "oct image: needs the position codes");
+    if ((ix.total >> 40) != 0) return fail(MSBWT_EINVAL, "oct image: a line's checkpoint holds 40 bits (N < 2^40)");
     const bool wide = index_is_wide(ix);
-    if (requested_shift && (requested_shift < kOctMinShift || requested_shift > kOctMaxShift)) {
-        why = "oct image: bucket shift out of range"; return MSBWT_EINVAL;
-    }
+    if (requested_shift && (requested_shift < kOctMinShift || requested_shift > kOctMaxShift))
+        return fail(MSBWT_EINVAL, "oct image: bucket shift out of range");
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((ix.total + 255) / 256, (uint64_t)sms * 32));
 
-    Scratch tmp;
+    DeviceScratch tmp;
     uint8_t *d_sym = nullptr;
     uint64_t *d_pos = nullptr;
     unsigned long long *d_stat = nullptr;  // [0] runs, [1] overflowed lines, [2] their occurrences
@@ -254,7 +234,7 @@ int build_oct_lines_on_device(int device, const IndexView &ix, const uint32_t *d
     O_TRY(cudaMemsetAsync(d_stat, 0, 3 * sizeof(unsigned long long)));
     oct_count_runs_kernel<<<grid, 256>>>(d_codes8, ix.total, d_stat);
     O_TRY(cudaGetLastError());
-    if (launches) (*launches)++;
+    g_launches++;
     unsigned long long runs = 0;
     O_TRY(cudaMemcpy(&runs, d_stat, sizeof(runs), cudaMemcpyDeviceToHost));
     img.runs = runs;
@@ -287,7 +267,7 @@ int build_oct_lines_on_device(int device, const IndexView &ix, const uint32_t *d
     for (int r = 0; r < kOctSyms; r++) {
         for (int c = 0; c < kOctCodes; c++) h_sym[(size_t)c] = acgt[(c >> (2 * (kOctSyms - 1 - r))) & 3];
         O_TRY(cudaMemcpy(d_sym, h_sym.data(), h_sym.size(), cudaMemcpyHostToDevice));
-        O_TRY(launch_constrain_ranges(device, ix, d_sym, cur, cur, kOctCodes, nxt, spare, nullptr, launches));
+        O_TRY(launch_constrain_ranges(device, ix, d_sym, cur, cur, kOctCodes, nxt, spare, nullptr));
         std::swap(cur, nxt);
     }
 
@@ -295,13 +275,13 @@ int build_oct_lines_on_device(int device, const IndexView &ix, const uint32_t *d
     if (ix.total) {
         oct_emit_kernel<<<grid, 256>>>(d_codes8, ix.total, (uint32_t)shift, nbuck8, reinterpret_cast<uint32_t *>(img.lines));
         O_TRY(cudaGetLastError());
-        if (launches) (*launches)++;
+        g_launches++;
     }
     // stamp
     if (wide) oct_stamp_kernel<true><<<kOctCodes / 8, 256>>>(cur, nbuck8, reinterpret_cast<uint32_t *>(img.lines), d_stat + 1);
     else oct_stamp_kernel<false><<<kOctCodes / 8, 256>>>(cur, nbuck8, reinterpret_cast<uint32_t *>(img.lines), d_stat + 1);
     O_TRY(cudaGetLastError());
-    if (launches) (*launches)++;
+    g_launches++;
     unsigned long long over[2] = {0, 0};
     O_TRY(cudaMemcpy(over, d_stat + 1, sizeof(over), cudaMemcpyDeviceToHost));
     img.overflow_lines = over[0];

@@ -112,29 +112,12 @@ __global__ void pair_stamp_kernel(const uint64_t *__restrict__ before, uint64_t 
     lines[line * kPairWords + (code >> 2) * 8 + (code & 3u)] = v;
 }
 
-struct Scratch {
-    std::vector<void *> ptrs;
-    ~Scratch() { for (void *p : ptrs) cudaFree(p); }
-    template <class T> cudaError_t alloc(T **p, size_t count) {
-        cudaError_t e = cudaMalloc((void **)p, (count ? count : 1) * sizeof(T));
-        if (e == cudaSuccess) ptrs.push_back(*p);
-        return e;
-    }
-};
-
-#define P_TRY(expr)                                                                        \
-    do {                                                                                   \
-        cudaError_t e_ = (expr);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            why = std::string("pair image: ") + #expr + ": " + cudaGetErrorString(e_);     \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;           \
-        }                                                                                  \
-    } while (0)
+#define P_TRY(e) CU_TRY_IN("pair image: ", e)
 
 }  // namespace
 
 int build_pair_image_on_device(int device, const IndexView &ix, const uint64_t start[kAlphabet], PairImage &img,
-                               std::string &why, int *launches, uint8_t **keep_codes) {
+                               uint8_t **keep_codes) {
     const bool wide = index_is_wide(ix);
     const uint64_t npair = ix.total / kPairSyms + 1;
     const uint32_t sb_shift = ix.sb_shift;
@@ -143,7 +126,7 @@ int build_pair_image_on_device(int device, const IndexView &ix, const uint64_t s
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
 
-    Scratch tmp;
+    DeviceScratch tmp;
     uint8_t *d_codes = nullptr, *d_counts = nullptr, *d_sym = nullptr;
     uint64_t *d_before = nullptr, *d_q = nullptr;
     P_TRY(cudaMalloc((void **)&img.lines, npair * kPairBytes));
@@ -165,7 +148,7 @@ int build_pair_image_on_device(int device, const IndexView &ix, const uint64_t s
     }
     P_TRY(cudaMemcpy(d_sym, h_sym, sizeof(h_sym), cudaMemcpyHostToDevice));
     P_TRY(cudaMemcpy(d_q, h_pos, sizeof(h_pos), cudaMemcpyHostToDevice));
-    P_TRY(launch_constrain_ranges(device, ix, d_sym, d_q, d_q, 16, d_q + 16, d_q + 32, nullptr, launches));
+    P_TRY(launch_constrain_ranges(device, ix, d_sym, d_q, d_q, 16, d_q + 16, d_q + 32, nullptr));
     P_TRY(cudaMemcpy(h_c2, d_q + 16, sizeof(h_c2), cudaMemcpyDeviceToHost));
 
     // 1. codes
@@ -175,12 +158,12 @@ int build_pair_image_on_device(int device, const IndexView &ix, const uint64_t s
         if (wide) pair_codes_kernel<true><<<grid, kCountThreads>>>(ix, d_codes);
         else pair_codes_kernel<false><<<grid, kCountThreads>>>(ix, d_codes);
         P_TRY(cudaGetLastError());
-        if (launches) (*launches)++;
+        g_launches++;
     }
     // 2. planes + per-line counts
     pair_fill_kernel<<<(unsigned)((npair + 127) / 128), 128>>>(d_codes, npair, reinterpret_cast<uint32_t *>(img.lines), d_counts);
     P_TRY(cudaGetLastError());
-    if (launches) (*launches)++;
+    g_launches++;
     // 3 + 4. per-code prefix sums over lines, stamped as they are produced
     {
         cub::TransformInputIterator<uint64_t, WidenU8, const uint8_t *> in(d_counts, WidenU8{});
@@ -197,14 +180,11 @@ int build_pair_image_on_device(int device, const IndexView &ix, const uint64_t s
             else pair_stamp_kernel<false><<<sgrid, 256>>>(d_before, npair, sb_shift, c, h_c2[c],
                                                           reinterpret_cast<uint32_t *>(img.lines), img.c2base);
             P_TRY(cudaGetLastError());
-            if (launches) (*launches)++;
+            g_launches++;
         }
     }
     P_TRY(cudaDeviceSynchronize());
-    if (keep_codes) {  // hand the code bytes to the caller instead of freeing them with the scratch
-        *keep_codes = d_codes;
-        tmp.ptrs.erase(std::find(tmp.ptrs.begin(), tmp.ptrs.end(), (void *)d_codes));
-    }
+    if (keep_codes) *keep_codes = tmp.take(d_codes);  // handed to the caller instead of freed with the scratch
     return MSBWT_OK;
 }
 

@@ -126,24 +126,7 @@ __global__ void quad_stamp_kernel(const uint64_t *__restrict__ before, uint64_t 
     code_sectors[s * kQuadWords] = v;
 }
 
-struct Scratch {
-    std::vector<void *> ptrs;
-    ~Scratch() { for (void *p : ptrs) cudaFree(p); }
-    template <class T> cudaError_t alloc(T **p, size_t count) {
-        cudaError_t e = cudaMalloc((void **)p, (count ? count : 1) * sizeof(T));
-        if (e == cudaSuccess) ptrs.push_back(*p);
-        return e;
-    }
-};
-
-#define Q_TRY(expr)                                                                        \
-    do {                                                                                   \
-        cudaError_t e_ = (expr);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            why = std::string("quad image: ") + #expr + ": " + cudaGetErrorString(e_);     \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;           \
-        }                                                                                  \
-    } while (0)
+#define Q_TRY(e) CU_TRY_IN("quad image: ", e)
 
 }  // namespace
 
@@ -152,8 +135,8 @@ uint64_t quad_image_bytes(uint64_t total) {
 }
 
 int build_quad_image_on_device(int device, const IndexView &ix, const uint8_t *d_codes2, QuadImage &img,
-                               std::string &why, int *launches, uint16_t **keep_codes) {
-    if (!ix.pair || !d_codes2) { why = "quad image: needs the pair image and its code bytes"; return MSBWT_EINVAL; }
+                               uint16_t **keep_codes) {
+    if (!ix.pair || !d_codes2) return fail(MSBWT_EINVAL, "quad image: needs the pair image and its code bytes");
     const bool wide = index_is_wide(ix);
     const uint64_t nsec_real = ix.total / kQuadSyms + 1;  // the last one holds position N
     const uint64_t nsec4 = nsec_real + 1;                 // + one all-zero sector per code: its checkpoint = the code's total
@@ -163,7 +146,7 @@ int build_quad_image_on_device(int device, const IndexView &ix, const uint8_t *d
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
 
-    Scratch tmp;
+    DeviceScratch tmp;
     uint16_t *d_codes4 = nullptr;
     uint8_t *d_sym = nullptr;
     uint64_t *d_before = nullptr, *d_pos = nullptr;
@@ -188,7 +171,7 @@ int build_quad_image_on_device(int device, const IndexView &ix, const uint8_t *d
         uint8_t h_sym[kQuadCodes];
         for (int c = 0; c < kQuadCodes; c++) h_sym[c] = acgt[(c >> (2 * (3 - r))) & 3];
         Q_TRY(cudaMemcpy(d_sym, h_sym, sizeof(h_sym), cudaMemcpyHostToDevice));
-        Q_TRY(launch_constrain_ranges(device, ix, d_sym, cur, cur, kQuadCodes, nxt, spare, nullptr, launches));
+        Q_TRY(launch_constrain_ranges(device, ix, d_sym, cur, cur, kQuadCodes, nxt, spare, nullptr));
         std::swap(cur, nxt);
     }
     Q_TRY(cudaMemcpy(h_c4, cur, sizeof(h_c4), cudaMemcpyDeviceToHost));
@@ -199,14 +182,14 @@ int build_quad_image_on_device(int device, const IndexView &ix, const uint8_t *d
         if (wide) quad_codes_kernel<true><<<grid, kCodeThreads>>>(ix, d_codes2, d_codes4);
         else quad_codes_kernel<false><<<grid, kCodeThreads>>>(ix, d_codes2, d_codes4);
         Q_TRY(cudaGetLastError());
-        if (launches) (*launches)++;
+        g_launches++;
     }
     // 2. occurrence bits
     {
         const unsigned grid = (unsigned)std::min<uint64_t>((nsec_real + 7) / 8, (uint64_t)sms * 64);
         quad_fill_kernel<<<grid, 256>>>(d_codes4, nsec_real, nsec4, reinterpret_cast<uint32_t *>(img.sectors));
         Q_TRY(cudaGetLastError());
-        if (launches) (*launches)++;
+        g_launches++;
     }
     // 3 + 4. per-code prefix sums over sectors, stamped as they are produced
     {
@@ -225,14 +208,11 @@ int build_quad_image_on_device(int device, const IndexView &ix, const uint8_t *d
             if (wide) quad_stamp_kernel<true><<<sgrid, 256>>>(d_before, nsec4, img.sb_shift4, c, h_c4[c], cs, img.c4base);
             else quad_stamp_kernel<false><<<sgrid, 256>>>(d_before, nsec4, img.sb_shift4, c, h_c4[c], cs, img.c4base);
             Q_TRY(cudaGetLastError());
-            if (launches) (*launches)++;
+            g_launches++;
         }
     }
     Q_TRY(cudaDeviceSynchronize());
-    if (keep_codes) {  // hand the quad codes to the caller instead of freeing them with the scratch
-        *keep_codes = d_codes4;
-        tmp.ptrs.erase(std::find(tmp.ptrs.begin(), tmp.ptrs.end(), (void *)d_codes4));
-    }
+    if (keep_codes) *keep_codes = tmp.take(d_codes4);  // handed to the caller instead of freed with the scratch
     return MSBWT_OK;
 }
 

@@ -195,14 +195,7 @@ canonical_resolve_kernel(const uint64_t *__restrict__ kmers, const uint64_t *__r
         if (bins[t]) atomicAdd(&hist[t], (unsigned long long)bins[t]);
 }
 
-#define S_TRY(expr)                                                                        \
-    do {                                                                                   \
-        cudaError_t e_ = (expr);                                                           \
-        if (e_ != cudaSuccess) {                                                           \
-            why = std::string("kmer spectrum: ") + #expr + ": " + cudaGetErrorString(e_);  \
-            return e_ == cudaErrorMemoryAllocation ? MSBWT_ENOMEM : MSBWT_ECUDA;           \
-        }                                                                                  \
-    } while (0)
+#define S_TRY(e) CU_TRY_IN("kmer spectrum: ", e)
 
 // the call's own stream: drained and destroyed on every way out, before the scratch it used is freed
 struct OwnStream {
@@ -244,8 +237,7 @@ uint64_t slice_parents() {
 // resolved into canonical pairs (canonical_resolve_kernel), which alone are binned, counted and, with `kmers`, listed
 template <bool WIDE, bool LIST>
 int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
-                 uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers,
-                 std::string &why, int *launches) {
+                 uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
     using P = typename Pos<WIDE>::type;
     using NodeT = Node<P, LIST>;
     const uint64_t B = slice_parents();
@@ -327,10 +319,8 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
     uint64_t staged = 0, listed = 0;
     auto flush = [&]() -> int {
         if (!staged) return MSBWT_OK;
-        if (!out_kmers.reserve(listed + staged) || !out_counts.reserve(listed + staged)) {
-            why = "kmer spectrum: host buffer for the k-mer list";
-            return MSBWT_ENOMEM;
-        }
+        if (!out_kmers.reserve(listed + staged) || !out_counts.reserve(listed + staged))
+            return fail(MSBWT_ENOMEM, "kmer spectrum: host buffer for the k-mer list");
         S_TRY(cudaMemcpyAsync(out_kmers.p + listed, d_stage_kmers, staged * sizeof(uint64_t), cudaMemcpyDeviceToHost, st.s));
         S_TRY(cudaMemcpyAsync(out_counts.p + listed, d_stage_counts, staged * sizeof(uint64_t), cudaMemcpyDeviceToHost, st.s));
         S_TRY(cudaStreamSynchronize(st.s));
@@ -348,18 +338,18 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
         canonical_revcomp_kernel<<<g, kCountThreads, 0, st.s>>>(d_stage_kmers, n, k, d_rc_kmers);
         S_TRY(cudaGetLastError());
         S_TRY(launch_seed_u64(ix, d_rc_kmers, k, n, d_packed, d_rc_counts, st.s));
-        S_TRY(launch_count_packed(device, ix, lanes, d_packed, k, n, d_rc_counts, st.s, launches, with_b));
+        S_TRY(launch_count_packed(device, ix, lanes, d_packed, k, n, d_rc_counts, st.s, with_b));
         canonical_resolve_kernel<<<g, kCountThreads, resolve_smem, st.s>>>(
             d_stage_kmers, d_stage_counts, n, k, walk_min, min_count, nbins, smem_bins, d_hist, d_count, d_rc_kmers,
             d_rc_counts, want_list ? d_resolved : nullptr);
         S_TRY(cudaGetLastError());
-        if (launches) *launches += 3;  // reverse complements, seed, resolve
+        g_launches += 2;  // reverse complements, resolve (the seed and search wrappers count theirs)
         if (!want_list) return MSBWT_OK;
         S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const uint64_t *)d_rc_kmers, (const uint8_t *)d_resolved,
                                          d_stage_kmers, d_count + 1, (int)n, st.s));
         S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const uint64_t *)d_rc_counts, (const uint8_t *)d_resolved,
                                          d_stage_counts, d_count + 1, (int)n, st.s));
-        if (launches) *launches += 4;
+        g_launches += 4;
         unsigned long long emitted = 0;
         S_TRY(cudaMemcpyAsync(&emitted, d_count + 1, sizeof(emitted), cudaMemcpyDeviceToHost, st.s));
         S_TRY(cudaStreamSynchronize(st.s));
@@ -382,7 +372,7 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
             S_TRY(cudaGetLastError());
             S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const NodeT *)children, (const uint8_t *)d_keep,
                                              level[d + 1], d_count + 1, (int)(4 * m), st.s));
-            if (launches) *launches += 3;  // the expansion + CUB's init and select kernels
+            g_launches += 3;  // the expansion + CUB's init and select kernels
             unsigned long long survivors = 0;
             S_TRY(cudaMemcpyAsync(&survivors, d_count + 1, sizeof(survivors), cudaMemcpyDeviceToHost, st.s));
             S_TRY(cudaStreamSynchronize(st.s));
@@ -395,7 +385,7 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
                 ix, slice, m, shift, walk_min, emit_bins, emit_smem_bins, d_hist, canonical ? d_count + 2 : d_count, ck, cc,
                 d_keep);
             S_TRY(cudaGetLastError());
-            if (launches) (*launches)++;
+            g_launches++;
             if (LIST) {
                 const uint64_t most = std::min<uint64_t>(4 * (uint64_t)m, cap);  // survivors this slice can have
                 if (staged + most > staging)
@@ -404,7 +394,7 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
                                                  d_stage_kmers + staged, d_count + 1, (int)(4 * m), st.s));
                 S_TRY(cub::DeviceSelect::Flagged(d_temp, temp_bytes, (const uint64_t *)cc, (const uint8_t *)d_keep,
                                                  d_stage_counts + staged, d_count + 1, (int)(4 * m), st.s));
-                if (launches) *launches += 4;
+                g_launches += 4;
                 unsigned long long survivors = 0;
                 S_TRY(cudaMemcpyAsync(&survivors, d_count + 1, sizeof(survivors), cudaMemcpyDeviceToHost, st.s));
                 S_TRY(cudaStreamSynchronize(st.s));
@@ -418,10 +408,7 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
     S_TRY(cudaMemcpyAsync(&total_kmers, d_count, sizeof(total_kmers), cudaMemcpyDeviceToHost, st.s));
     if (nbins) S_TRY(cudaMemcpyAsync(hist, d_hist, nbins * sizeof(uint64_t), cudaMemcpyDeviceToHost, st.s));
     S_TRY(cudaStreamSynchronize(st.s));
-    if (want_list && listed != total_kmers) {
-        why = "kmer spectrum: the list and the histogram disagree";
-        return MSBWT_ECUDA;
-    }
+    if (want_list && listed != total_kmers) return fail(MSBWT_ECUDA, "kmer spectrum: the list and the histogram disagree");
     *n_kmers = total_kmers;
     if (want_list) {
         *kmers = listed ? out_kmers.p : nullptr;
@@ -434,19 +421,14 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
 }  // namespace
 
 int kmer_spectrum_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
-                            uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers,
-                            std::string &why, int *launches) {
+                            uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
     // the canonical walk always carries the k-mer values: the pairs are resolved from them
     const bool list = canonical || kmers != nullptr;
     if (index_is_wide(ix))
-        return list ? spectrum_run<true, true>(device, ix, lanes, canonical, k, min_count, hist, nbins, kmers, counts,
-                                               n_kmers, why, launches)
-                    : spectrum_run<true, false>(device, ix, lanes, false, k, min_count, hist, nbins, kmers, counts,
-                                                n_kmers, why, launches);
-    return list ? spectrum_run<false, true>(device, ix, lanes, canonical, k, min_count, hist, nbins, kmers, counts,
-                                            n_kmers, why, launches)
-                : spectrum_run<false, false>(device, ix, lanes, false, k, min_count, hist, nbins, kmers, counts, n_kmers,
-                                             why, launches);
+        return list ? spectrum_run<true, true>(device, ix, lanes, canonical, k, min_count, hist, nbins, kmers, counts, n_kmers)
+                    : spectrum_run<true, false>(device, ix, lanes, false, k, min_count, hist, nbins, kmers, counts, n_kmers);
+    return list ? spectrum_run<false, true>(device, ix, lanes, canonical, k, min_count, hist, nbins, kmers, counts, n_kmers)
+                : spectrum_run<false, false>(device, ix, lanes, false, k, min_count, hist, nbins, kmers, counts, n_kmers);
 }
 
 }  // namespace msbwt

@@ -22,6 +22,7 @@ cudaError_t launch_count_oct_stats(int device, const IndexView &ix, const uint64
     if (cudaError_t e = cudaMemsetAsync(work, 0, sizeof(uint32_t), st); e != cudaSuccess) return e;
     if (cudaError_t e = cudaMemsetAsync(d_stats, 0, kOctStatWords * sizeof(unsigned long long), st); e != cudaSuccess) return e;
     const unsigned grid = oct_grid(device, (const void *)count_kmers_oct_kernel<true>, kOctSmemPacked, lay.n);
+    g_launches++;
     count_kmers_oct_kernel<true><<<grid, kCountThreads, kOctSmemPacked, st>>>(ix, d_packed, lay, k, d_out, work, d_stats);
     return cudaGetLastError();
 }

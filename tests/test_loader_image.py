@@ -111,6 +111,24 @@ def test_rle_whose_runs_add_up_past_2_pow_62_is_refused_before_any_device_work()
     assert e.value.code == 3
 
 
+def test_host_side_failures_keep_their_messages(tmp_path):
+    """msbwt_last_error() of failures found before any device work, verbatim, and "" after a call that succeeds"""
+    L = M.load_library()
+    b = M.RleBWT.new()
+    with pytest.raises(M.MsbwtError) as e:
+        b.load_vector(np.array([9, 14], dtype=np.uint8))  # 14 = symbol 6
+    assert e.value.code == 3 and L.msbwt_last_error() == b"RLE byte 1 has symbol 6 (>= 6)"
+    missing = str(tmp_path / "missing.npy")
+    with pytest.raises(OSError):
+        b.load_numpy_file(missing)
+    assert L.msbwt_last_error() == f"cannot open {missing}: No such file or directory".encode()
+    with pytest.raises(M.MsbwtError) as e:
+        M.debug_build_image(np.full(13, 1 | (31 << 3), dtype=np.uint8))  # a thirteenth digit: one run beyond 2^60
+    assert e.value.code == 3 and L.msbwt_last_error() == b"run longer than 2^60 symbols"
+    M.debug_build_image(np.array([9, 10], dtype=np.uint8))
+    assert L.msbwt_last_error() == b""
+
+
 def test_string_util_mirror():
     assert list(M.convert_stoi("ACGTN$acgtnx")) == [1, 2, 3, 5, 4, 0, 1, 2, 3, 5, 4, 4]
     assert M.convert_itos([0, 1, 2, 3, 4, 5]) == "$ACGNT"
