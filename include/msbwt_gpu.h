@@ -426,6 +426,38 @@ int msbwt_kmer_spectrum(const msbwt_index *idx, uint32_t k, uint64_t min_count, 
  * holds fewer than 2^22 * ceil(min_count / 2) symbols. */
 int msbwt_kmer_spectrum_canonical(const msbwt_index *idx, uint32_t k, uint64_t min_count, uint64_t *hist,
                                   uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers);
+/* The unitigs of the compacted de Bruijn graph of the solid k-mers (1 <= k <= 32), node-centric as in BCALM2 and
+ * cuttlefish.  Nodes V: canonical == 0, the k-mers msbwt_kmer_spectrum lists (count_kmer(X) >= min_count);
+ * canonical == 1, every X with C(X) >= min_count, C as in msbwt_kmer_spectrum_canonical, so both members of each pair
+ * are nodes and V is closed under rc.  X -> Y is an edge iff X[1..k) = Y[0..k-1) and both are in V (the (k+1)-mer need
+ * not occur; self-loops count toward the degrees), and it is compacted iff outdeg(X) = 1, indeg(Y) = 1 and X != Y.
+ * Plain mode: every node lies on exactly one maximal path of compacted edges, its unitig.  A linear path starts at its
+ * node with no compacted in-edge; a cycle of compacted edges is cut before its smallest node (by the integer value of
+ * msbwt_count_kmers_u64's encoding), starts there and has |C| + k - 1 symbols.  Canonical mode: the plain unitigs of
+ * that V, each unitig U kept iff first(U) <= first(U'), U' being the unitig holding rc(first(U)): one unitig per
+ * reverse-complement pair and a self-reverse-complementary unitig once (for a linear U: first(U) <= rc(last(U)); for
+ * a pair of cycles {C, rc C}: min(C) <= min(rc C)).  On an index that already holds both strands of its reads, plain
+ * mode returns every unitig together with its reverse complement; on an index of the reads as they are, canonical
+ * mode is what an assembler wants.
+ * Outputs: *n_unitigs unitigs, strictly ascending by the value of their first k-mer.  *syms: their sequences one after
+ * the other in the msbwt alphabet (A,C,G,T = 1,2,3,5, the bytes msbwt_count_kmers_fixed takes); *offsets: n + 1 u64,
+ * unitig i = (*syms)[offsets[i], offsets[i + 1]); *count_sums[i] = the sum of count_kmer (C in canonical mode) over
+ * its k-windows, so its mean abundance is count_sums[i] / (length - k + 1).  All three are owned by the caller
+ * (release each with msbwt_buffer_free) and NULL when n == 0.  Two calls return identical arrays.
+ * Runs on the handle's first replica with a stream and scratch of its own and takes no lock (it may run beside queries
+ * on the same handle).  It lists V with the spectrum walk twice (a histogram-only pass sizes the device arrays the
+ * second pass fills, so no k-mer crosses the link), radix-sorts it, links every node by one binary search, ranks the
+ * unitigs by pointer jumping and writes them out on the device.  Device memory: the spectrum's walk (see
+ * msbwt_kmer_spectrum) on top of V's 32 bytes per node while V is listed, then 53 bytes per node (53.1-53.3 measured
+ * at 58-727 M nodes on configs[2] on a B200, tools/unitig_bench.py) (keys, counts and the sort's alternates 32, links 8,
+ * offsets and numbers 12, a flag 1), 16 more while cycles of compacted edges are cut, then the outputs (16 bytes per
+ * unitig and its symbols) in place of the counts (8 per node).  Canonical mode doubles the node count against the
+ * canonical spectrum's list.
+ * EINVAL (nothing written): bad handle, k == 0 or k > 32, min_count == 0, canonical not 0 or 1, any output pointer
+ * NULL.  ENOMEM / ECUDA: nothing is leaked, nothing is left running, the outputs are NULL / 0; a V of 2^32 nodes or
+ * more (node ids are 32-bit) is ENOMEM. */
+int msbwt_unitigs(const msbwt_index *idx, uint32_t k, uint64_t min_count, int canonical, uint8_t **syms,
+                  uint64_t **offsets, uint64_t **count_sums, uint64_t *n_unitigs);
 
 /* ---- the data format either side of the path: src/bwt_converter.rs ----
  * convert_to_vec (:26-80): a text BWT over `$ACGNT` (newlines are skipped and do not end a run) -> msbwt RLE bytes

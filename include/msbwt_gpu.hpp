@@ -162,6 +162,27 @@ class RleBWT {
         msbwt_buffer_free(reinterpret_cast<uint8_t *>(cn));
         return out;
     }
+    // the unitigs of the compacted de Bruijn graph of the solid k-mers (msbwt_unitigs): sequences (msbwt alphabet)
+    // concatenated, n + 1 offsets, per-unitig sums of the k-window counts; ascending by first k-mer
+    struct Unitigs {
+        std::vector<uint8_t> syms;
+        std::vector<uint64_t> offsets{0}, count_sums;
+    };
+    Unitigs unitigs(uint32_t k, uint64_t min_count = 2, bool canonical = false) const {
+        Unitigs out;
+        uint8_t *s = nullptr;
+        uint64_t *o = nullptr, *c = nullptr, n = 0;
+        check(msbwt_unitigs(h_, k, min_count, canonical ? 1 : 0, &s, &o, &c, &n));
+        if (n) {
+            out.syms.assign(s, s + o[n]);
+            out.offsets.assign(o, o + n + 1);
+            out.count_sums.assign(c, c + n);
+        }
+        msbwt_buffer_free(s);
+        msbwt_buffer_free(reinterpret_cast<uint8_t *>(o));
+        msbwt_buffer_free(reinterpret_cast<uint8_t *>(c));
+        return out;
+    }
     const msbwt_index *handle() const { return h_; }
 
   private:

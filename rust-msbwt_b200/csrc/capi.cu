@@ -1074,6 +1074,24 @@ extern "C" int msbwt_kmer_spectrum_canonical(const msbwt_index *idx, uint32_t k,
     return kmer_spectrum_call(idx, true, k, min_count, hist, nbins, kmers, counts, n_kmers);
 }
 
+extern "C" int msbwt_unitigs(const msbwt_index *idx, uint32_t k, uint64_t min_count, int canonical, uint8_t **syms,
+                             uint64_t **offsets, uint64_t **count_sums, uint64_t *n_unitigs) {
+    g_last_error.clear();
+    if (!idx || idx->reps.empty()) return fail(MSBWT_EINVAL, "bad handle");
+    if (!k || k > 32) return fail(MSBWT_EINVAL, "unitigs: k must be in 1..32");
+    if (!min_count) return fail(MSBWT_EINVAL, "unitigs: min_count must be at least 1");
+    if (canonical != 0 && canonical != 1) return fail(MSBWT_EINVAL, "unitigs: canonical must be 0 or 1");
+    if (!syms || !offsets || !count_sums || !n_unitigs) return fail(MSBWT_EINVAL, "unitigs: NULL output pointer");
+    *syms = nullptr;
+    *offsets = *count_sums = nullptr;
+    *n_unitigs = 0;
+    // as the spectrum: replica 0's images are read-only after create and the call has its own stream and scratch
+    const Replica &rep = *idx->reps[0];
+    DeviceGuard guard(rep.device);
+    return unitigs_on_device(rep.device, rep.view, rep.lanes, canonical == 1, k, min_count, syms, offsets, count_sums,
+                             n_unitigs);
+}
+
 extern "C" void msbwt_buffer_free(uint8_t *p) { free(p); }
 
 // ================================================================ measurement aid

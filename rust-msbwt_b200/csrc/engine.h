@@ -198,6 +198,20 @@ int merge_rle_bwts_on_device(const uint8_t *h_rle_a, uint64_t len_a, const uint8
 int kmer_spectrum_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
                             uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers);
 
+// the same list (LIST mode, `canonical` as above) written to device arrays of `sink.cap` entries, which a first,
+// histogram-only call sized: *n_kmers entries of sink.kmers / sink.counts, in the order the host list would have
+struct DeviceKmerList {
+    uint64_t *kmers = nullptr, *counts = nullptr;
+    uint64_t cap = 0;
+};
+int kmer_spectrum_to_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
+                            const DeviceKmerList &sink, uint64_t *n_kmers);
+
+// ---- unitigs.cu: the unitigs of the compacted de Bruijn graph of the solid k-mers (msbwt_unitigs; one replica, on the
+// current device).  *syms, *offsets, *count_sums: malloc'd host arrays the caller frees, null when *n_unitigs == 0 ----
+int unitigs_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
+                      uint8_t **syms, uint64_t **offsets, uint64_t **count_sums, uint64_t *n_unitigs);
+
 // ---- loader.cu: RLE stream checks, the host builder (msbwt_debug_build_image) and the .npy reader ----
 int validate_rle(const uint8_t *rle, uint64_t len);
 int build_image_from_rle(const uint8_t *rle, uint64_t len, uint32_t sb_shift, HostImage &img);

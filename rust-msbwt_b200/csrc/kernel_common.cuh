@@ -97,6 +97,14 @@ inline int sm_count(int device) {
     return cached[device];
 }
 
+// rc(v) of a k-mer in msbwt_count_kmers_u64's encoding: every code c becomes 3 - c (= c ^ 3) and the k 2-bit groups
+// are reversed.  The bit reversal also swaps the two bits inside each group, so they are swapped back.
+__device__ __forceinline__ uint64_t revcomp_kmer(uint64_t v, uint32_t k) {
+    uint64_t r = __brevll(~v);
+    r = ((r >> 1) & 0x5555555555555555ull) | ((r & 0x5555555555555555ull) << 1);
+    return r >> (64 - 2 * k);  // the complemented zero bits above the k-mer end up below it
+}
+
 // one full wave of CTAs (a multiple of the SM count), fewer if there is less work
 inline unsigned persistent_grid(int device, const void *kernel, int threads, uint64_t work_groups,
                                 int groups_per_cta) {

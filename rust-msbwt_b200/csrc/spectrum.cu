@@ -136,14 +136,6 @@ spectrum_emit_kernel(IndexView ix, const Node<typename Pos<WIDE>::type, LIST> *_
         if (bins[t]) atomicAdd(&hist[t], (unsigned long long)bins[t]);
 }
 
-// rc(v) of a k-mer in msbwt_count_kmers_u64's encoding: every code c becomes 3 - c (= c ^ 3) and the k 2-bit groups
-// are reversed.  The bit reversal also swaps the two bits inside each group, so they are swapped back.
-__device__ __forceinline__ uint64_t revcomp_kmer(uint64_t v, uint32_t k) {
-    uint64_t r = __brevll(~v);
-    r = ((r >> 1) & 0x5555555555555555ull) | ((r & 0x5555555555555555ull) << 1);
-    return r >> (64 - 2 * k);  // the complemented zero bits above the k-mer end up below it
-}
-
 __global__ void __launch_bounds__(kCountThreads)
 canonical_revcomp_kernel(const uint64_t *__restrict__ kmers, uint32_t n, uint32_t k, uint64_t *__restrict__ rc) {
     for (uint32_t i = blockIdx.x * kCountThreads + threadIdx.x; i < n; i += gridDim.x * kCountThreads)
@@ -235,13 +227,15 @@ uint64_t slice_parents() {
 
 // `canonical` (LIST only): the walk lists every k-mer with count >= walk_min and stages it; each staged batch is then
 // resolved into canonical pairs (canonical_resolve_kernel), which alone are binned, counted and, with `kmers`, listed
+// `sink` (LIST only): the list goes to these device arrays instead of host buffers (kmers stays null)
 template <bool WIDE, bool LIST>
 int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
-                 uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {
+                 uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers,
+                 const DeviceKmerList *sink = nullptr) {
     using P = typename Pos<WIDE>::type;
     using NodeT = Node<P, LIST>;
     const uint64_t B = slice_parents();
-    const bool want_list = kmers != nullptr;
+    const bool want_list = kmers != nullptr || sink != nullptr;
     // A pair with C >= min_count has a member with count >= ceil(min_count / 2); a pair whose members both count less
     // has C <= min_count - 1.  So the canonical walk prunes at ceil(min_count / 2), exactly.
     const uint64_t walk_min = canonical ? min_count / 2 + (min_count & 1) : min_count;  // (min_count + 1) / 2 wraps at 2^64 - 1
@@ -319,6 +313,15 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
     uint64_t staged = 0, listed = 0;
     auto flush = [&]() -> int {
         if (!staged) return MSBWT_OK;
+        if (sink) {
+            if (listed + staged > sink->cap) return fail(MSBWT_ECUDA, "kmer spectrum: more k-mers than the sizing pass found");
+            S_TRY(cudaMemcpyAsync(sink->kmers + listed, d_stage_kmers, staged * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st.s));
+            S_TRY(cudaMemcpyAsync(sink->counts + listed, d_stage_counts, staged * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st.s));
+            S_TRY(cudaStreamSynchronize(st.s));  // the staging buffers are refilled next
+            listed += staged;
+            staged = 0;
+            return MSBWT_OK;
+        }
         if (!out_kmers.reserve(listed + staged) || !out_counts.reserve(listed + staged))
             return fail(MSBWT_ENOMEM, "kmer spectrum: host buffer for the k-mer list");
         S_TRY(cudaMemcpyAsync(out_kmers.p + listed, d_stage_kmers, staged * sizeof(uint64_t), cudaMemcpyDeviceToHost, st.s));
@@ -410,7 +413,7 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
     S_TRY(cudaStreamSynchronize(st.s));
     if (want_list && listed != total_kmers) return fail(MSBWT_ECUDA, "kmer spectrum: the list and the histogram disagree");
     *n_kmers = total_kmers;
-    if (want_list) {
+    if (kmers) {
         *kmers = listed ? out_kmers.p : nullptr;
         *counts = listed ? out_counts.p : nullptr;
         if (listed) out_kmers.p = out_counts.p = nullptr;
@@ -419,6 +422,13 @@ int spectrum_run(int device, const IndexView &ix, int lanes, bool canonical, uin
 }
 
 }  // namespace
+
+int kmer_spectrum_to_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
+                            const DeviceKmerList &sink, uint64_t *n_kmers) {
+    return index_is_wide(ix)
+               ? spectrum_run<true, true>(device, ix, lanes, canonical, k, min_count, nullptr, 0, nullptr, nullptr, n_kmers, &sink)
+               : spectrum_run<false, true>(device, ix, lanes, canonical, k, min_count, nullptr, 0, nullptr, nullptr, n_kmers, &sink);
+}
 
 int kmer_spectrum_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
                             uint64_t *hist, uint32_t nbins, uint64_t **kmers, uint64_t **counts, uint64_t *n_kmers) {

@@ -157,6 +157,7 @@ def load_library():
         "msbwt_merge_rle_bwts": (i32, [vp, u64, vp, u64, i32, C.POINTER(vp), C.POINTER(u64), C.POINTER(u64), C.POINTER(u32)]),
         "msbwt_kmer_spectrum": (i32, [vp, u32, u64, vp, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_kmer_spectrum_canonical": (i32, [vp, u32, u64, vp, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
+        "msbwt_unitigs": (i32, [vp, u32, u64, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_buffer_free": (None, [vp]),
         "msbwt_convert_to_rle": (i32, [vp, u64, C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_save_rle_npy": (i32, [vp, u64, C.c_char_p]),
@@ -186,7 +187,7 @@ EXPORTED_SYMBOLS = (
     "msbwt_count_kmers_fixed", "msbwt_constrain_ranges", "msbwt_count_kmers_fixed_device",
     "msbwt_constrain_ranges_device", "msbwt_packed_bytes", "msbwt_pack_kmers_device",
     "msbwt_count_kmers_packed_device", "msbwt_launch_count", "msbwt_gather_bench", "msbwt_l2_fetch_granularity", "msbwt_debug_build_image", "msbwt_debug_copy_image",
-    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_merge_rle_bwts", "msbwt_kmer_spectrum", "msbwt_kmer_spectrum_canonical", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
+    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_merge_rle_bwts", "msbwt_kmer_spectrum", "msbwt_kmer_spectrum_canonical", "msbwt_unitigs", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
     "msbwt_save_runs_npy",
     "msbwt_host_free", "msbwt_last_error", "msbwt_abi_version",
 )
@@ -457,6 +458,29 @@ class RleBWT:
         with that count, in a deterministic order and no other promised."""
         _, kmers, counts = self._kmer_spectrum(k, min_count, 0, True, canonical)
         return kmers, counts
+
+    def unitigs(self, k: int, min_count: int = 2, canonical: bool = False) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """(syms u8, offsets u64[n + 1], count_sums u64[n]): the unitigs of the compacted de Bruijn graph of the k-mers
+        with count_kmer >= min_count (k <= 32; node-centric, msbwt_unitigs), ascending by first k-mer.  Unitig i is
+        syms[offsets[i]:offsets[i + 1]] in the msbwt alphabet (convert_itos turns it into text); count_sums[i] sums the
+        counts of its k-windows.  canonical=True: nodes are both members of every pair whose canonical count (see
+        kmer_spectrum) is >= min_count, and each unitig is returned once per reverse-complement pair."""
+        if k < 0 or min_count < 0:
+            raise MsbwtError(EINVAL, "k and min_count must not be negative")
+        L = load_library()
+        s, o, c, n = C.c_void_p(0), C.c_void_p(0), C.c_void_p(0), C.c_uint64(0)
+        _check(L.msbwt_unitigs(self.handle, k, min_count, 1 if canonical else 0, C.byref(s), C.byref(o), C.byref(c),
+                               C.byref(n)), "unitigs")
+        try:
+            if not n.value:
+                return np.zeros(0, np.uint8), np.zeros(1, np.uint64), np.zeros(0, np.uint64)
+            offsets = np.ctypeslib.as_array(C.cast(o, C.POINTER(C.c_uint64)), shape=(n.value + 1,)).copy()
+            sums = np.ctypeslib.as_array(C.cast(c, C.POINTER(C.c_uint64)), shape=(n.value,)).copy()
+            syms = np.ctypeslib.as_array(C.cast(s, C.POINTER(C.c_uint8)), shape=(int(offsets[-1]),)).copy()
+            return syms, offsets, sums
+        finally:
+            for p in (s, o, c):
+                L.msbwt_buffer_free(p)
 
     # -- device-buffer entry points (raw pointers: torch `.data_ptr()` / stream handles)
     def count_kmers_fixed_device(self, d_syms: int, k: int, n: int, d_out: int, d_status: int = 0,

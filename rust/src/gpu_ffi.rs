@@ -72,6 +72,7 @@ extern "C" {
     pub fn msbwt_build_rle_bwt_ragged(syms: *const u8, offsets: *const u64, n_reads: u64, device: c_int, rle: *mut *mut u8, rle_len: *mut u64, total: *mut u64) -> c_int;
     pub fn msbwt_merge_rle_bwts(rle_a: *const u8, len_a: u64, rle_b: *const u8, len_b: u64, device: c_int, rle: *mut *mut u8, rle_len: *mut u64, total: *mut u64, iterations: *mut u32) -> c_int;
     pub fn msbwt_kmer_spectrum(idx: *const msbwt_index, k: u32, min_count: u64, hist: *mut u64, nbins: u32, kmers: *mut *mut u64, counts: *mut *mut u64, n_kmers: *mut u64) -> c_int;
+    pub fn msbwt_unitigs(idx: *const msbwt_index, k: u32, min_count: u64, canonical: c_int, syms: *mut *mut u8, offsets: *mut *mut u64, count_sums: *mut *mut u64, n_unitigs: *mut u64) -> c_int;
     pub fn msbwt_kmer_spectrum_canonical(idx: *const msbwt_index, k: u32, min_count: u64, hist: *mut u64, nbins: u32, kmers: *mut *mut u64, counts: *mut *mut u64, n_kmers: *mut u64) -> c_int;
     pub fn msbwt_buffer_free(p: *mut u8);
     pub fn msbwt_convert_to_rle(text: *const u8, n: u64, rle: *mut *mut u8, rle_len: *mut u64) -> c_int;
