@@ -326,8 +326,10 @@ int msbwt_constrain_ranges_fanout_device(const msbwt_index *idx, int slot, const
  * strands == 1, and count_kmer(window) + count_kmer(reverse_complement_i(window)) (src/string_util.rs:45-50)
  * when strands == 2.  Only the reads cross PCIe (read_len bytes per read instead of k per window); the
  * windows are laid out on the device and go through the same pack / search kernels as msbwt_count_kmers_fixed.
- * EINVAL when k == 0, k > read_len, strands not in {1,2} (nothing written) or a symbol is >= 6 (found by the
- * pack kernel, as for msbwt_count_kmers_fixed: `out` is then unspecified). */
+ * A read is never split across launches, so one read's (read_len-k+1) * strands * k window bytes must fit the
+ * device; they may pass 2^32.
+ * EINVAL when k == 0, k > read_len, strands not in {1,2}, (read_len-k+1) * strands >= 2^32 (nothing written) or a
+ * symbol is >= 6 (found by the pack kernel, as for msbwt_count_kmers_fixed: `out` is then unspecified). */
 int msbwt_count_read_kmers(const msbwt_index *idx, const uint8_t *reads, uint32_t read_len, uint64_t n_reads,
                            uint32_t k, uint32_t strands, uint64_t *out /* n_reads * (read_len-k+1) */);
 

@@ -50,8 +50,16 @@ expand_read_kmers_kernel(const uint8_t *__restrict__ reads, uint32_t read_len, u
     const uint64_t step = (uint64_t)gridDim.x * blockDim.x * 16u;
     for (uint64_t o = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) * 16u; o < total; o += step) {
         uint64_t r = o / per_read;
-        const uint32_t p = (uint32_t)(o - r * per_read);
-        uint32_t qq = p / k, i = p - qq * k;                  // query within the read, symbol within the query
+        uint32_t qq, i;                                       // query within the read, symbol within the query
+        if (per_read >> 32) {  // one read's windows pass 2^32 bytes (e.g. a 22 Mbp read at k = 100, both strands)
+            const uint64_t p = o - r * per_read;
+            qq = (uint32_t)(p / k);
+            i = (uint32_t)(p - (uint64_t)qq * k);
+        } else {               // the usual case keeps the cheaper 32-bit division
+            const uint32_t p = (uint32_t)(o - r * per_read);
+            qq = p / k;
+            i = p - qq * k;
+        }
         const uint8_t *rd = reads + r * read_len;
         uint32_t word[4] = {0u, 0u, 0u, 0u};
         const uint32_t nb = (uint32_t)(total - o < 16u ? total - o : 16u);

@@ -642,6 +642,8 @@ extern "C" int msbwt_count_read_kmers(const msbwt_index *idx, const uint8_t *rea
     if (!n_reads) return MSBWT_OK;
     if (!reads || !out) return fail(MSBWT_EINVAL, "NULL host buffer");
     const uint64_t windows = (uint64_t)read_len - k + 1, per_read_q = windows * strands;
+    // the expand kernel numbers a read's queries in 32 bits
+    if (per_read_q >> 32) return fail(MSBWT_EINVAL, "count_read_kmers: a read has 2^32 or more queries (windows x strands)");
     AllLocks locks(idx);
     // symbols are validated where they are packed (count_kmer's own check, src/msbwt_core.rs:127): the pack
     // kernel flags any symbol >= 6 and the call then returns EINVAL
