@@ -460,6 +460,55 @@ int msbwt_kmer_spectrum_canonical(const msbwt_index *idx, uint32_t k, uint64_t m
  * more (node ids are 32-bit) is ENOMEM. */
 int msbwt_unitigs(const msbwt_index *idx, uint32_t k, uint64_t min_count, int canonical, uint8_t **syms,
                   uint64_t **offsets, uint64_t **count_sums, uint64_t *n_unitigs);
+/* Read correction against the index in the manner of fmlrc (not bit-compatible with fmlrc2): weak runs of a read's
+ * k-mer windows are bridged through the de Bruijn graph of the solid k-mers, breadth-first.  Read r is
+ * syms[offsets[r] .. offsets[r+1]) over A,C,G,N,T = 1,2,3,4,5, reads of any lengths.  Parameters: k in 1..32,
+ * min_count >= 1, frac_permille in 0..1000 (fmlrc's frac 0.1 is 100), branch_limit >= 1 (fmlrc's branch-limit factor,
+ * 4 there).  Each read is corrected on its own, from the counts of the read as given:
+ *  1. Window counts.  Windows w = 0 .. nwin-1, nwin = len - k + 1, window w = read[w .. w+k).  A window holding N has
+ *     count2 = 0; otherwise count2(X) = count_kmer(X) + count_kmer(rc X), what msbwt_count_read_kmers(strands = 2)
+ *     gives (a palindrome counts twice).  Reads shorter than k + 2 are returned unchanged.
+ *  2. Threshold.  v = the ascending list of the read's non-zero count2 values, m its length.  m = 0: the read is
+ *     unchanged.  Otherwise T = max(min_count, floor(v[floor(m/2)] * frac_permille / 1000)), in integers.
+ *  3. Weak runs.  A window is weak when count2 < T; a weak run is a maximal run [a, b) of weak windows.  It is
+ *     eligible when 1 <= a, b <= nwin - 1 and b - a >= k - 1: then X = window a-1 is its solid seed, Y = window b its
+ *     solid target, and P = read[a-1+k .. b) the bases between them, of length L0 = b - a + 1 - k >= 0 (a substitution
+ *     gives L0 = 1, a deletion 0, an insertion 1).  Runs that touch either end of the read, or are shorter than k - 1
+ *     windows, are left as they are.
+ *  4. Bridges.  Emax = floor(13 L0 / 10) + 2.  A walk is a string over ACGT that starts with X and whose every
+ *     k-window Z has count2(Z) >= T; walks grow breadth-first, one symbol per round, for rounds t = 1 .. k + Emax.  At
+ *     round t >= k a walk whose newest window is Y is a bridge S = X E Y with |E| = t - k and is not extended; every
+ *     other walk is extended at the next round (also one that meets Y before round k).  The gap's work is the number
+ *     of walks created over all rounds (bridges included, X not); when it exceeds branch_limit * (k + Emax) the gap is
+ *     abandoned and left unchanged, even if bridges were found.
+ *  5. Choice.  Among the bridges, the E with the smallest Levenshtein distance to P (unit costs over symbol codes; an
+ *     N in P matches nothing); ties go to the shorter E, then to the lexicographically smaller (A < C < G < T).  No
+ *     bridge: unchanged.  Otherwise P is replaced by E (E != P, since X P Y holds a weak window).  All gaps of a read
+ *     are decided from the read as given and applied together (their P's are disjoint).
+ * Outputs: *out_syms and *out_offsets (n_reads + 1 u64, from 0) hold the corrected reads in input order in the same
+ * ragged form; release both with msbwt_buffer_free.  stats (u64[5], may be NULL), summed over the call: [0] weak runs,
+ * [1] eligible runs, [2] bridged (replaced), [3] abandoned over the budget, [4] eligible runs with no bridge.
+ * The result depends only on the index's counts and the reads: not on chunking, the number of replicas or which
+ * images the index carries.
+ * Not covered: runs at either end of a read (they need an open-ended extension rule), k > 32 (fmlrc's second pass at
+ * K = 59), fmlrc2's depth-first order and choice rules.  fmlrc's two passes are two calls.
+ * The reads are split into one contiguous slice per replica; each replica corrects its slice on its own stream and
+ * scratch in chunks of whole reads of about 2^22 symbols, and takes no lock (the call may run beside queries on the
+ * same handle).  Per chunk everything runs on the device: window counts through the query path, per-read medians by a
+ * segmented sort, weak runs, one breadth-first search over every gap of the chunk (each round's 4 children x 2 strands
+ * counted in one batch, one small read-back per round), Levenshtein scoring per bridge and the assembly of the new
+ * reads.  Device memory per replica follows the chunk, not the batch: the buffers hold about 130 bytes per chunk
+ * symbol (the query path's scratch for two queries per symbol included) and about 500 per walk of the widest round,
+ * and grow by half again when a chunk needs more.  Measured peaks (tools/correct_bench.py, configs[2]'s index on a
+ * B200): 0.27-0.36 GB for one chunk of 2 M symbols of 10 kbp reads, 0.94-1.10 GB for chunks of 2^22 symbols of
+ * 150 bp reads.  A read longer than 2^22 symbols is a chunk of its own.
+ * EINVAL (nothing written): bad handle, k outside 1..32, min_count == 0, frac_permille > 1000, branch_limit == 0,
+ * a NULL output pointer, NULL syms / offsets with n_reads > 0, decreasing offsets, a read of 2^31 symbols or more, or
+ * a symbol 0 ($) or >= 6.  ENOMEM / ECUDA: nothing is leaked and nothing is left running; one chunk whose walks need
+ * 2^32 node ids or more is ENOMEM. */
+int msbwt_correct_reads(const msbwt_index *idx, const uint8_t *syms, const uint64_t *offsets, uint64_t n_reads,
+                        uint32_t k, uint64_t min_count, uint32_t frac_permille, uint32_t branch_limit,
+                        uint8_t **out_syms, uint64_t **out_offsets, uint64_t *stats);
 
 /* ---- the data format either side of the path: src/bwt_converter.rs ----
  * convert_to_vec (:26-80): a text BWT over `$ACGNT` (newlines are skipped and do not end a run) -> msbwt RLE bytes

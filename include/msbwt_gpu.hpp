@@ -183,6 +183,27 @@ class RleBWT {
         msbwt_buffer_free(reinterpret_cast<uint8_t *>(c));
         return out;
     }
+    // reads corrected in the manner of fmlrc (msbwt_correct_reads): weak interior runs of k-mer windows bridged
+    // through the solid k-mers; `stats` (optional) receives the call's five counters
+    std::vector<std::vector<uint8_t>> correct_reads(const std::vector<std::vector<uint8_t>> &reads, uint32_t k,
+                                                    uint64_t min_count = 5, uint32_t frac_permille = 100,
+                                                    uint32_t branch_limit = 4, uint64_t *stats = nullptr) const {
+        std::vector<uint8_t> flat;
+        std::vector<uint64_t> offsets{0};
+        for (const auto &r : reads) {
+            flat.insert(flat.end(), r.begin(), r.end());
+            offsets.push_back(flat.size());
+        }
+        uint8_t *s = nullptr;
+        uint64_t *o = nullptr;
+        check(msbwt_correct_reads(h_, flat.data(), offsets.data(), reads.size(), k, min_count, frac_permille,
+                                  branch_limit, &s, &o, stats));
+        std::vector<std::vector<uint8_t>> out(reads.size());
+        for (size_t r = 0; r < reads.size(); r++) out[r].assign(s + o[r], s + o[r + 1]);
+        msbwt_buffer_free(s);
+        msbwt_buffer_free(reinterpret_cast<uint8_t *>(o));
+        return out;
+    }
     const msbwt_index *handle() const { return h_; }
 
   private:

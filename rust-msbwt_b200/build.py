@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmsbwt_b200.so")
-SOURCES = ["capi.cu", "hostpath.cu", "kernels.cu", "quad_kernels.cu", "stats_kernels.cu", "wide_kernels.cu", "final_kernels.cu", "ext_kernels.cu", "loader.cu", "builder.cu", "pair_builder.cu", "quad_builder.cu", "oct_builder.cu", "fin_builder.cu", "bwt_build.cu", "bwt_merge.cu", "spectrum.cu", "unitigs.cu"]
+SOURCES = ["capi.cu", "hostpath.cu", "kernels.cu", "quad_kernels.cu", "stats_kernels.cu", "wide_kernels.cu", "final_kernels.cu", "ext_kernels.cu", "loader.cu", "builder.cu", "pair_builder.cu", "quad_builder.cu", "oct_builder.cu", "fin_builder.cu", "bwt_build.cu", "bwt_merge.cu", "spectrum.cu", "unitigs.cu", "correct.cu"]
 HOST_SOURCES = ["hostpack.cpp", "codec.cpp"]  # plain g++ (AVX2 intrinsics behind a runtime check)
 HEADERS = ["engine.h", "handle.h", "layout.h", "device_rank.cuh", "kernel_common.cuh", "pack_common.cuh", "oct_kernel.cuh", "hostpack.h", os.path.join(ROOT, "include", "msbwt_gpu.h")]
 

@@ -72,6 +72,18 @@ struct DeviceScratch {
     }
 };
 
+// a call's own stream: drained and destroyed on every way out, before the scratch it used is freed (declare it after
+// that scratch)
+struct OwnStream {
+    cudaStream_t s = nullptr;
+    ~OwnStream() {
+        if (s) {
+            cudaStreamSynchronize(s);
+            cudaStreamDestroy(s);
+        }
+    }
+};
+
 constexpr int kCountThreads = 256;
 constexpr uint64_t kMaxPerLaunch = 1ull << 30;  // queries per pack/count launch (u32 indices inside the kernels)
 // resident CTAs per SM the kernels are compiled for (register budget = 65536 / (256 * min_ctas)):
@@ -211,6 +223,17 @@ int kmer_spectrum_to_device(int device, const IndexView &ix, int lanes, bool can
 // current device).  *syms, *offsets, *count_sums: malloc'd host arrays the caller frees, null when *n_unitigs == 0 ----
 int unitigs_on_device(int device, const IndexView &ix, int lanes, bool canonical, uint32_t k, uint64_t min_count,
                       uint8_t **syms, uint64_t **offsets, uint64_t **count_sums, uint64_t *n_unitigs);
+
+// ---- correct.cu: msbwt_correct_reads for reads [0, n_reads) of `offsets` (one replica, on the current device, with
+// its own stream and scratch).  Appends the corrected reads' symbols and lengths; stats[5] as in msbwt_gpu.h ----
+struct CorrectParams {
+    uint32_t k;
+    uint64_t min_count;
+    uint32_t frac_permille, branch_limit;
+};
+int correct_reads_on_device(int device, const IndexView &ix, int lanes, const uint8_t *syms, const uint64_t *offsets,
+                            uint64_t n_reads, const CorrectParams &prm, std::vector<uint8_t> &out_syms,
+                            std::vector<uint64_t> &out_lens, uint64_t stats[5]);
 
 // ---- loader.cu: RLE stream checks, the host builder (msbwt_debug_build_image) and the .npy reader ----
 int validate_rle(const uint8_t *rle, uint64_t len);

@@ -43,7 +43,7 @@ struct CountsOut {
 // that replica's device current, and joins.  Whatever a route does -- including returning early on a CUDA error --
 // every lane stream of the replica is drained before its thread leaves, so no copy of this call is still reading
 // or writing the caller's buffers when the call returns.  The first failure (by device order) is reported.
-// Caller holds the replica locks.
+// Caller holds the replica locks when fn uses the lanes.
 template <class F>
 int run_on_replicas(const msbwt_index *idx, uint64_t n, F &&fn) {
     const size_t ndev = idx->reps.size();
@@ -681,4 +681,74 @@ extern "C" int msbwt_count_read_kmers(const msbwt_index *idx, const uint8_t *rea
         if (int rc = drain(rep); rc != MSBWT_OK) return rc;
         return check_status(rep, "count_read_kmers");
     });
+}
+
+extern "C" int msbwt_correct_reads(const msbwt_index *idx, const uint8_t *syms, const uint64_t *offsets, uint64_t n_reads,
+                                   uint32_t k, uint64_t min_count, uint32_t frac_permille, uint32_t branch_limit,
+                                   uint8_t **out_syms, uint64_t **out_offsets, uint64_t *stats) {
+    g_last_error.clear();
+    g_last_h2d = g_last_d2h = 0;
+    if (!idx || idx->reps.empty()) return fail(MSBWT_EINVAL, "bad handle");
+    if (!k || k > 32) return fail(MSBWT_EINVAL, "correct_reads: k must be in 1..32");
+    if (!min_count) return fail(MSBWT_EINVAL, "correct_reads: min_count must be at least 1");
+    if (frac_permille > 1000) return fail(MSBWT_EINVAL, "correct_reads: frac_permille must be in 0..1000");
+    if (!branch_limit) return fail(MSBWT_EINVAL, "correct_reads: branch_limit must be at least 1");
+    if (!out_syms || !out_offsets) return fail(MSBWT_EINVAL, "correct_reads: NULL output pointer");
+    if (n_reads && (!syms || !offsets)) return fail(MSBWT_EINVAL, "NULL host buffer");
+    for (uint64_t r = 0; r < n_reads; r++) {
+        if (offsets[r + 1] < offsets[r]) return fail(MSBWT_EINVAL, "correct_reads: offsets decrease at read " + std::to_string(r));
+        // a read is sorted as one CUB segment, whose sizes are int
+        if (offsets[r + 1] - offsets[r] >= (1ull << 31)) return fail(MSBWT_EINVAL, "correct_reads: a read of 2^31 symbols or more");
+    }
+    if (n_reads)
+        for (uint64_t i = offsets[0]; i < offsets[n_reads]; i++)
+            if (syms[i] == 0 || syms[i] >= 6)
+                return fail(MSBWT_EINVAL, "correct_reads: symbol " + std::to_string(syms[i]) + " at " + std::to_string(i) +
+                                              " (reads hold A, C, G, N, T = 1..5)");
+    // each replica corrects one contiguous slice of the reads with its own stream and scratch (no lane: no lock)
+    const CorrectParams prm{k, min_count, frac_permille, branch_limit};
+    struct Part {
+        std::vector<uint8_t> syms;
+        std::vector<uint64_t> lens;
+        uint64_t stats[5] = {0, 0, 0, 0, 0};
+    };
+    std::vector<Part> parts(idx->reps.size());
+    int rc = run_on_replicas(idx, n_reads, [&](Replica &rep, Slice sl, Xfer &x) {
+        size_t d = 0;
+        while (idx->reps[d].get() != &rep) d++;
+        Part &pt = parts[d];
+        const int r = correct_reads_on_device(rep.device, rep.view, rep.lanes, syms, offsets + sl.begin, sl.len(), prm,
+                                              pt.syms, pt.lens, pt.stats);
+        x.h2d += offsets[sl.end] - offsets[sl.begin] + (sl.len() + 1) * sizeof(uint64_t);
+        x.d2h += pt.syms.size() + pt.lens.size() * sizeof(uint64_t);
+        return r;
+    });
+    if (rc != MSBWT_OK) return rc;
+    uint64_t total = 0;
+    for (const Part &pt : parts) total += pt.syms.size();
+    uint8_t *os = (uint8_t *)malloc(std::max<uint64_t>(total, 1));
+    uint64_t *oo = (uint64_t *)malloc((n_reads + 1) * sizeof(uint64_t));
+    if (!os || !oo) {
+        free(os);
+        free(oo);
+        return fail(MSBWT_ENOMEM, "correct_reads: host buffers for the result");
+    }
+    uint64_t at = 0, r = 0;
+    oo[0] = 0;
+    for (const Part &pt : parts) {
+        if (!pt.syms.empty()) memcpy(os + at, pt.syms.data(), pt.syms.size());
+        at += pt.syms.size();
+        for (uint64_t len : pt.lens) {
+            oo[r + 1] = oo[r] + len;
+            r++;
+        }
+    }
+    if (stats)
+        for (int i = 0; i < 5; i++) {
+            stats[i] = 0;
+            for (const Part &pt : parts) stats[i] += pt.stats[i];
+        }
+    *out_syms = os;
+    *out_offsets = oo;
+    return MSBWT_OK;
 }

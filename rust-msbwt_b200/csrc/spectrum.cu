@@ -189,17 +189,6 @@ canonical_resolve_kernel(const uint64_t *__restrict__ kmers, const uint64_t *__r
 
 #define S_TRY(e) CU_TRY_IN("kmer spectrum: ", e)
 
-// the call's own stream: drained and destroyed on every way out, before the scratch it used is freed
-struct OwnStream {
-    cudaStream_t s = nullptr;
-    ~OwnStream() {
-        if (s) {
-            cudaStreamSynchronize(s);
-            cudaStreamDestroy(s);
-        }
-    }
-};
-
 // a malloc'd host array that grows by doubling; released unless handed to the caller
 struct HostU64 {
     uint64_t *p = nullptr;

@@ -242,16 +242,6 @@ unitig_emit_kernel(uint32_t n, uint32_t k, const uint64_t *__restrict__ keys, co
 
 #define U_TRY(e) CU_TRY_IN("unitigs: ", e)
 
-struct OwnStream {
-    cudaStream_t s = nullptr;
-    ~OwnStream() {
-        if (s) {
-            cudaStreamSynchronize(s);
-            cudaStreamDestroy(s);
-        }
-    }
-};
-
 // malloc'd host outputs, released unless handed to the caller
 struct HostOut {
     uint8_t *syms = nullptr;

@@ -158,6 +158,7 @@ def load_library():
         "msbwt_kmer_spectrum": (i32, [vp, u32, u64, vp, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_kmer_spectrum_canonical": (i32, [vp, u32, u64, vp, u32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_unitigs": (i32, [vp, u32, u64, i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(u64)]),
+        "msbwt_correct_reads": (i32, [vp, vp, vp, u64, u32, u64, u32, u32, C.POINTER(vp), C.POINTER(vp), vp]),
         "msbwt_buffer_free": (None, [vp]),
         "msbwt_convert_to_rle": (i32, [vp, u64, C.POINTER(vp), C.POINTER(u64)]),
         "msbwt_save_rle_npy": (i32, [vp, u64, C.c_char_p]),
@@ -187,7 +188,7 @@ EXPORTED_SYMBOLS = (
     "msbwt_count_kmers_fixed", "msbwt_constrain_ranges", "msbwt_count_kmers_fixed_device",
     "msbwt_constrain_ranges_device", "msbwt_packed_bytes", "msbwt_pack_kmers_device",
     "msbwt_count_kmers_packed_device", "msbwt_launch_count", "msbwt_gather_bench", "msbwt_l2_fetch_granularity", "msbwt_debug_build_image", "msbwt_debug_copy_image",
-    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_merge_rle_bwts", "msbwt_kmer_spectrum", "msbwt_kmer_spectrum_canonical", "msbwt_unitigs", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
+    "msbwt_host_alloc", "msbwt_build_rle_bwt", "msbwt_build_rle_bwt_ragged", "msbwt_merge_rle_bwts", "msbwt_kmer_spectrum", "msbwt_kmer_spectrum_canonical", "msbwt_unitigs", "msbwt_correct_reads", "msbwt_buffer_free", "msbwt_convert_to_rle", "msbwt_save_rle_npy",
     "msbwt_save_runs_npy",
     "msbwt_host_free", "msbwt_last_error", "msbwt_abi_version",
 )
@@ -481,6 +482,35 @@ class RleBWT:
         finally:
             for p in (s, o, c):
                 L.msbwt_buffer_free(p)
+
+    def correct_reads(self, reads, k: int, min_count: int = 5, frac_permille: int = 100,
+                      branch_limit: int = 4) -> tuple[list[np.ndarray], np.ndarray]:
+        """Reads corrected against the index in the manner of fmlrc (msbwt_correct_reads; include/msbwt_gpu.h holds
+        the definition): every weak run of k-mer windows inside a read is bridged through the k-mers whose
+        both-strand count reaches the read's threshold, breadth-first, and replaced by the bridge closest to it in
+        edit distance.  `reads`: a sequence of uint8 symbol arrays / strings over ACGNT, as build_rle_bwt_ragged takes.
+        Returns (the corrected reads as uint8 arrays, stats u64[5]: weak runs, eligible runs, bridged, abandoned over
+        the budget, eligible with no bridge)."""
+        if k < 0 or min_count < 0 or frac_permille < 0 or branch_limit < 0:
+            raise MsbwtError(EINVAL, "k, min_count, frac_permille and branch_limit must not be negative")
+        L = load_library()
+        arrs = [convert_stoi(r) if isinstance(r, (str, bytes)) else _u8(r).reshape(-1) for r in reads]
+        offs = np.zeros(len(arrs) + 1, dtype=np.uint64)
+        if arrs:
+            np.cumsum([a.size for a in arrs], out=offs[1:])
+        flat = _u8(np.concatenate(arrs)) if arrs and offs[-1] else np.zeros(1, np.uint8)
+        s, o, stats = C.c_void_p(0), C.c_void_p(0), np.zeros(5, np.uint64)
+        _check(L.msbwt_correct_reads(self.handle, _p(flat), _p(offs), len(arrs), k, min_count, frac_permille,
+                                     branch_limit, C.byref(s), C.byref(o), _p(stats)), "correct_reads")
+        try:
+            o_arr = np.ctypeslib.as_array(C.cast(o, C.POINTER(C.c_uint64)), shape=(len(arrs) + 1,)).copy()
+            total = int(o_arr[-1])
+            syms = (np.ctypeslib.as_array(C.cast(s, C.POINTER(C.c_uint8)), shape=(total,)).copy() if total
+                    else np.zeros(0, np.uint8))
+        finally:
+            L.msbwt_buffer_free(s)
+            L.msbwt_buffer_free(o)
+        return [syms[o_arr[r]:o_arr[r + 1]] for r in range(len(arrs))], stats
 
     # -- device-buffer entry points (raw pointers: torch `.data_ptr()` / stream handles)
     def count_kmers_fixed_device(self, d_syms: int, k: int, n: int, d_out: int, d_status: int = 0,

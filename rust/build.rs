@@ -10,7 +10,7 @@ fn main() {
     let mut objs = vec![];
     // the same list as rust-msbwt_b200/build.py SOURCES
     for f in ["capi.cu", "hostpath.cu", "kernels.cu", "quad_kernels.cu", "stats_kernels.cu", "wide_kernels.cu", "final_kernels.cu", "ext_kernels.cu",
-              "loader.cu", "builder.cu", "pair_builder.cu", "quad_builder.cu", "oct_builder.cu", "fin_builder.cu", "bwt_build.cu", "bwt_merge.cu", "spectrum.cu", "unitigs.cu"] {
+              "loader.cu", "builder.cu", "pair_builder.cu", "quad_builder.cu", "oct_builder.cu", "fin_builder.cu", "bwt_build.cu", "bwt_merge.cu", "spectrum.cu", "unitigs.cu", "correct.cu"] {
         let obj = out.join(f).with_extension("o");
         let ok = Command::new(&nvcc)
             .args(["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

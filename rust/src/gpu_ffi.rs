@@ -74,6 +74,7 @@ extern "C" {
     pub fn msbwt_kmer_spectrum(idx: *const msbwt_index, k: u32, min_count: u64, hist: *mut u64, nbins: u32, kmers: *mut *mut u64, counts: *mut *mut u64, n_kmers: *mut u64) -> c_int;
     pub fn msbwt_unitigs(idx: *const msbwt_index, k: u32, min_count: u64, canonical: c_int, syms: *mut *mut u8, offsets: *mut *mut u64, count_sums: *mut *mut u64, n_unitigs: *mut u64) -> c_int;
     pub fn msbwt_kmer_spectrum_canonical(idx: *const msbwt_index, k: u32, min_count: u64, hist: *mut u64, nbins: u32, kmers: *mut *mut u64, counts: *mut *mut u64, n_kmers: *mut u64) -> c_int;
+    pub fn msbwt_correct_reads(idx: *const msbwt_index, syms: *const u8, offsets: *const u64, n_reads: u64, k: u32, min_count: u64, frac_permille: u32, branch_limit: u32, out_syms: *mut *mut u8, out_offsets: *mut *mut u64, stats: *mut u64) -> c_int;
     pub fn msbwt_buffer_free(p: *mut u8);
     pub fn msbwt_convert_to_rle(text: *const u8, n: u64, rle: *mut *mut u8, rle_len: *mut u64) -> c_int;
     pub fn msbwt_save_rle_npy(rle: *const u8, len: u64, path: *const c_char) -> c_int;

@@ -80,6 +80,33 @@ impl GpuRleBWT {
         assert!(rc == ffi::MSBWT_OK, "count_kmers_u64_u32 failed: {}", last_error());
         out
     }
+
+    /// Reads corrected against the index in the manner of fmlrc (msbwt_correct_reads, include/msbwt_gpu.h): weak
+    /// interior runs of k-mer windows bridged through the solid k-mers, and the five counters of the call.
+    pub fn correct_reads(&self, reads: &[Vec<u8>], k: u32, min_count: u64, frac_permille: u32, branch_limit: u32) -> (Vec<Vec<u8>>, [u64; 5]) {
+        let mut offsets = Vec::with_capacity(reads.len() + 1);
+        offsets.push(0u64);
+        let mut flat = Vec::new();
+        for r in reads {
+            flat.extend_from_slice(r);
+            offsets.push(flat.len() as u64);
+        }
+        let (mut s, mut o, mut stats) = (ptr::null_mut(), ptr::null_mut(), [0u64; 5]);
+        let rc = unsafe {
+            ffi::msbwt_correct_reads(self.handle, flat.as_ptr(), offsets.as_ptr(), reads.len() as u64, k, min_count, frac_permille, branch_limit, &mut s, &mut o, stats.as_mut_ptr())
+        };
+        assert!(rc == ffi::MSBWT_OK, "correct_reads failed: {}", last_error());
+        let out = unsafe {
+            let o = std::slice::from_raw_parts(o, reads.len() + 1);
+            let v = (0..reads.len()).map(|r| std::slice::from_raw_parts(s.add(o[r] as usize), (o[r + 1] - o[r]) as usize).to_vec()).collect();
+            v
+        };
+        unsafe {
+            ffi::msbwt_buffer_free(s);
+            ffi::msbwt_buffer_free(o as *mut u8);
+        }
+        (out, stats)
+    }
 }
 
 impl Default for GpuRleBWT {
